@@ -2,6 +2,7 @@
 """bench.py -- BPR training throughput on the BASELINE.json workloads (driver contract).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--batch B] [--shape ml-20m] [--configs LIST]
+                    [--dump-outputs DIR]
 
 One "step" = one synchronous BPR-MF training step over one batch of ``--batch`` triples (u,i,j) per GPU
 (the reference's zero_grad + calc_loss + backward + optimizer.step, AbstractRecommender.py:119-128).
@@ -170,6 +171,26 @@ def timed_ms(fn, warm, reps):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / reps
+
+
+DUMP_BYTES = 64 << 20
+
+
+def timed_outputs(tensors, seed=0):
+    """Host copies of what the timed path returned, for --dump-outputs (float32 / float64 as computed).  When they exceed
+    DUMP_BYTES in all, every 2-D table keeps the same fraction of its rows, drawn with a fixed seed: the same rows in every
+    run with the same arguments."""
+    total = sum(t.numel() * t.element_size() for t in tensors.values())
+    tables = sum(t.numel() * t.element_size() for t in tensors.values() if t.dim() == 2)
+    keep = 1.0 if total <= DUMP_BYTES else (DUMP_BYTES - (total - tables)) / tables
+    rng = np.random.default_rng(seed)
+    out = {}
+    for name, t in tensors.items():
+        if t.dim() == 2 and keep < 1.0:
+            rows = np.sort(rng.choice(t.shape[0], max(1, int(t.shape[0] * keep)), replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        out[name] = t.detach().cpu().numpy()
+    return out
 
 
 def mf_config(U, I, F, **kw):
@@ -666,6 +687,8 @@ def run_own(args):
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs writes the single-GPU path's outputs; run it with one process")
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
         return run_sharded(args, rank, local, world, dev)
@@ -693,30 +716,33 @@ def run_own(args):
     P, Q, ws, hp = model.embed_user.weight, model.embed_item.weight, model._ws, model._hp
 
     def run_steps(first, k, timed):
-        """k steps starting at global step `first`, walking the epoch cyclically; one launch per epoch segment."""
-        evs, launches, s = [], 0, first
+        """k steps starting at global step `first`, walking the epoch cyclically; one launch per epoch segment.
+        -> (events, launches, per-step losses of the last launch)."""
+        evs, launches, s, losses = [], 0, first, None
         while k > 0:
             pos = s % spe
             seg = min(k, spe - pos)
             if timed:
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-            ops.mf_bpr_train_steps(P, Q, ws, bu, bi, bj, B, pos, seg, hp, check=False)
+            losses = ops.mf_bpr_train_steps(P, Q, ws, bu, bi, bj, B, pos, seg, hp, check=False)
             if timed:
                 e1.record()
                 evs.append((e0, e1, seg, pos))
             launches += 1
             s += seg
             k -= seg
-        return evs, launches
+        return evs, launches, losses
 
     clocks = ClockSampler(local)
     run_steps(0, args.warmup, False)
     torch.cuda.synchronize()
     t_region0 = time.time()
-    evs, launches = run_steps(args.warmup, args.steps, True)
+    evs, launches, losses = run_steps(args.warmup, args.steps, True)
     torch.cuda.synchronize()
     t_region1 = time.time()
+    # snapshot now: fit_host_batches below trains the same tables further
+    outputs = timed_outputs({"embed_user.weight": P, "embed_item.weight": Q, "loss": losses[-1:]}) if args.dump_outputs else None
     ms = sum(e0.elapsed_time(e1) for e0, e1, _, _ in evs)
     done_triples = 0
     for _, _, seg, pos in evs:
@@ -820,6 +846,10 @@ def run_own(args):
                          "kernel": sk["instantiation"], "avg_launch_ms": avg_launch_ms},
             "cpu_baseline": cpu,
             "configs": cfgs}
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     return 0
 
@@ -1060,7 +1090,14 @@ def main():
     ap.add_argument("--ref-workers", dest="ref_workers", type=int, default=4, help="DataLoader workers of the reference (test.py:94)")
     ap.add_argument("--rows-file", dest="rows_file", default=None, help="reference arm: .npy of sampler triples to train on")
     ap.add_argument("--quick", action="store_true", help="reference arm: main measurement only")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="own arm, one GPU: after the timed steps write DIR/<name>.npy of what the last timed step returned "
+                         "(embed_user.weight, embed_item.weight, loss); above 64 MB a fixed seeded sample of table rows")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the own arm's outputs")
     if args.impl == "reference":
         args.steps = 8 if args.steps is None else args.steps
         args.warmup = 2 if args.warmup is None else args.warmup

@@ -145,7 +145,7 @@ def test_edge_cases_small_inputs():
 def test_deterministic_mode_is_bitwise_reproducible(orc):
     """deterministic=True: every cross-thread sum of a step is taken in fixed point (integer atomics are associative), so two
     fits from the same state give bitwise identical tables and epoch losses; the default mode (float RED in arrival order)
-    agrees with it to fp32 noise; and because the oracle accumulates the same sums in fp64, GPU == oracle almost everywhere."""
+    agrees with it to fp32 noise; and the oracle, which accumulates the same sums in fp64, stays within 1e-6 of it."""
     from daisyrec_b200.model.MFRecommender import MF
     from daisyrec_b200.utils.dataset import BasicDataset, get_dataloader
     rng = np.random.default_rng(12)
@@ -167,6 +167,9 @@ def test_deterministic_mode_is_bitwise_reproducible(orc):
     Po, Qo = P0.copy(), Q0.copy()
     for _ in range(2):
         orc.mf_bpr_epoch(Po, Qo, np.ascontiguousarray(data), None, B, orc.hyper(0.01, 0.001, 0.001))
-    for got, want in ((runs[0][0], Po), (runs[0][1], Qo)):
-        # (measured 0.70: the rest differ by one fp32 ulp where the oracle's fp64 sum and the 2^-40 fixed-point sum round apart)
-        assert (got == want).mean() > 0.6 and np.abs(got - want).max() < 1e-4, float((got == want).mean())
+    for got, want, equal in ((runs[0][0], Po, 0.6), (runs[0][1], Qo, 0.15)):
+        # Measured on a B200 (1000 W limit): 0.70 of P and 0.18 of Q bit-equal, largest differences 3e-7 and 1.1e-8.  A single step leaves
+        # some entries one fp32 ulp apart (the default mode the same ones), and later steps carry them on; an item row takes
+        # few contributions per step, so a larger share of Q carries one.
+        assert (got == want).mean() > equal and np.abs(got - want).max() < 1e-6, \
+            (float((got == want).mean()), float(np.abs(got - want).max()))

@@ -50,6 +50,11 @@ def test_nfm_steps_match_reference_fixture(orc):
                 for _l in range(L):
                     noisy[o + F * F:o + F * F + F] = True                 # Linear bias
                     o += F * F + F + 2 * F
+            if optn == "adam":
+                # The same holds batch by batch: the bias of a unit that is active for both items of every triple shifts both
+                # scores alike, so its gradient is zero.  The reference's sums cancel to exactly 0 there and its Adam leaves
+                # the slot where it was; any other summation order leaves noise.
+                noisy |= Ns[s + 1] == Ns[s]
             for got, want, nm in ((P, Ps[s + 1], "P"), (Q, Qs[s + 1], "Q"), (bias, Bs[s + 1], "bias"), (N, Ns[s + 1], "N")):
                 err = np.abs(got.cpu().numpy() - want)
                 tol = (1e-5 if optn == "sgd" else 1e-4) * max(1.0, np.abs(want).max())
