@@ -93,25 +93,17 @@ SIGNATURES = {
     "drb_ngcf_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, c_i32p, C.c_int32, C.c_int32]),
     "drb_ngcf_workspace_init": (C.c_int, [vp, C.c_int32, C.c_int32, c_i32p, C.c_int32, C.c_int32, vp]),
     "drb_ngcf_forward": (C.c_int, [vp, vp, vp, C.c_int32, C.c_int32, c_i32p, C.c_int32, vp, vp, vp, vp, vp, C.c_int64, C.c_int32,
-                                   vp, vp]),
+                                   vp, C.c_float, vp, vp]),
     "drb_ngcf_bpr_train_steps": (C.c_int, [vp, vp, vp, C.c_int32, C.c_int32, c_i32p, C.c_int32, vp, vp, vp, vp, vp, C.c_int64,
                                            vp, vp, vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.POINTER(Hyper), C.c_int64,
-                                           C.c_int32, C.c_int32, vp, C.c_int32, c_i64p, vp]),
-    "drb_ngcf_forward_dropout": (C.c_int, [vp, vp, vp, C.c_int32, C.c_int32, c_i32p, C.c_int32, vp, vp, vp, vp, vp, C.c_int64,
-                                           C.c_int32, vp, C.c_float, vp, vp]),
-    "drb_ngcf_bpr_train_steps_dropout": (C.c_int, [vp, vp, vp, C.c_int32, C.c_int32, c_i32p, C.c_int32, vp, vp, vp, vp, vp, C.c_int64,
-                                                   vp, vp, vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.POINTER(Hyper),
-                                                   C.c_int64, C.c_int32, C.c_int32, vp, C.c_float, vp, C.c_int32, c_i64p, vp]),
+                                           C.c_int32, C.c_int32, vp, C.c_float, vp, C.c_int32, c_i64p, vp]),
     "drb_nfm_param_count": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),
     "drb_nfm_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int64]),
     "drb_nfm_workspace_init": (C.c_int, [vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int64, vp]),
     "drb_nfm_bpr_train_steps": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                           C.c_int32, C.c_int64, vp, vp, vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
-                                          C.POINTER(Hyper), C.c_int64, C.c_int32, C.c_int32, vp, C.c_int32, c_i64p, vp]),
-    "drb_nfm_bpr_train_steps_dropout": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
-                                                  C.c_int32, C.c_int64, vp, vp, vp, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
-                                                  C.POINTER(Hyper), C.c_int64, C.c_int32, C.c_int32, vp, C.c_float, vp, C.c_int32,
-                                                  c_i64p, vp]),
+                                          C.POINTER(Hyper), C.c_int64, C.c_int32, C.c_int32, vp, C.c_float, vp, C.c_int32, c_i64p,
+                                          vp]),
     "drb_nfm_scores": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                  C.c_int32, C.c_int64, vp, vp, C.c_int64, C.c_int32, vp, vp]),
     "drb_comm_unique_id": (C.c_int, [vp]),

@@ -28,6 +28,14 @@ int cuda_fail(cudaError_t e, const char *what, const char *file, int line);
 
 int sm_count();
 
+// blocks of a grid-stride loop over n items: one per `block` items, at most per_sm per SM, at least one
+inline int grid_size(long long n, int block, int per_sm = 16)
+{
+    long long b = (n + block - 1) / block, cap = (long long)sm_count() * per_sm;
+    if (b > cap) b = cap;
+    return (int)(b < 1 ? 1 : b);
+}
+
 // ---------------------------------------------------------------- row geometry
 // A factor row of F floats is processed by a group of W lanes (W a power of two <= 32);
 // lane l owns the chunks c = l, l+W, ... of VEC consecutive floats (NCH chunks per lane at most).

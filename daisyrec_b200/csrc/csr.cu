@@ -172,13 +172,6 @@ __global__ void lgcn_adj_kernel(const int64_t *__restrict__ ui_ptr, const int32_
     }
 }
 
-static int grid1(long long n, int block)
-{
-    long long b = (n + block - 1) / block, cap = (long long)sm_count() * 16;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
-}
-
 struct CsrWs {
     unsigned *deg, *cursor, *uniq;
     int64_t *raw_ptr;
@@ -227,9 +220,9 @@ extern "C" int drb_csr_build(const int32_t *d_row, const int32_t *d_col, int64_t
     carve_csr(d_ws, n_rows, nnz, &w);
     // bad flag, deg, cursor are contiguous at the start of the workspace: one memset
     DRB_CUDA(cudaMemsetAsync(d_ws, 0, (size_t)((char *)w.uniq - (char *)d_ws), st));
-    if (nnz) csr_count_kernel<<<grid1(nnz, 256), 256, 0, st>>>(d_row, nnz, n_rows, w.deg, w.bad);
+    if (nnz) csr_count_kernel<<<grid_size(nnz, 256), 256, 0, st>>>(d_row, nnz, n_rows, w.deg, w.bad);
     csr_exscan_kernel<<<1, 1024, 0, st>>>(w.deg, w.raw_ptr, n_rows);
-    if (nnz) csr_scatter_kernel<<<grid1(nnz, 256), 256, 0, st>>>(d_row, d_col, nnz, n_rows, n_cols, w.raw_ptr, w.cursor, w.tmp, w.bad);
+    if (nnz) csr_scatter_kernel<<<grid_size(nnz, 256), 256, 0, st>>>(d_row, d_col, nnz, n_rows, n_cols, w.raw_ptr, w.cursor, w.tmp, w.bad);
     const size_t smem = sizeof(uint32_t) * (size_t)((n_cols + 31) / 32);
     if (smem > 48 * 1024) {
         DRB_CUDA(cudaFuncSetAttribute(csr_rows_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -257,8 +250,8 @@ extern "C" int drb_lgcn_build_adj(const int64_t *d_ui_ptr, const int32_t *d_ui_c
 {
     DRB_REQUIRE(d_ui_ptr && d_iu_ptr && d_adj_ptr && U > 0 && I > 0 && nnz >= 0, "lgcn_build_adj: bad arguments");
     DRB_REQUIRE(nnz == 0 || (d_ui_col && d_iu_col && d_adj_col && d_adj_val), "lgcn_build_adj: null arrays");
-    lgcn_adj_kernel<<<grid1(2 * nnz + U + I + 1, 256), 256, 0, (cudaStream_t)stream>>>(d_ui_ptr, d_ui_col, d_iu_ptr, d_iu_col, U, I,
-                                                                                       nnz, d_adj_ptr, d_adj_col, d_adj_val);
+    lgcn_adj_kernel<<<grid_size(2 * nnz + U + I + 1, 256), 256, 0, (cudaStream_t)stream>>>(d_ui_ptr, d_ui_col, d_iu_ptr, d_iu_col, U, I,
+                                                                                           nnz, d_adj_ptr, d_adj_col, d_adj_val);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }

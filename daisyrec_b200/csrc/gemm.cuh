@@ -1,4 +1,5 @@
-// gemm.cuh -- plain entry points of the dense-layer GEMM dispatcher in neumf.cu (dtype 0: fp32 CUDA cores, 1: bf16 tcgen05).
+// gemm.cuh -- plain entry points of the dense-layer GEMM dispatcher in neumf.cu (dtype 0: fp32 CUDA cores, 1: bf16 tcgen05),
+// and the dense optimiser step the tower / layer blocks of NeuMF, NGCF and NFM share.
 #pragma once
 #include "common.cuh"
 
@@ -15,5 +16,11 @@ int gemm_tn_acc_t(int dtype, long long M, int N, int K, const float *A, long lon
                   long long ldc, cudaStream_t st);
 // gb[n] += sum_m dZ[m, n]          (bias gradient, N <= 256)
 int colsum_acc(const float *dZ, long long M, int N, float *gb, cudaStream_t st);
+
+struct WsHeader;
+// W -= step number adam_step + 1 of SGD or torch.optim.Adam's single-tensor rule (m, v: Adam's state) on a flat block of n
+// floats, and g = 0; no-op once hdr->status is set (a NaN loss earlier in the step)
+int dense_update(float *W, float *g, float *m, float *v, long long n, const drb_hyper *h, long long adam_step, const WsHeader *hdr,
+                 cudaStream_t st);
 
 }  // namespace drb

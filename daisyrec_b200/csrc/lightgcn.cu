@@ -192,19 +192,10 @@ static int propagate_sum(const Adj &a, const float *X0, float *S, float *Xa, flo
 static int scale_table(float *x, long long n, float s, cudaStream_t st)
 {
     long long n4 = n / 4;
-    if (n4 > 0) {
-        long long blocks = (n4 + 255) / 256, cap = (long long)sm_count() * 16;
-        scale_kernel<<<(int)(blocks > cap ? cap : blocks), 256, 0, st>>>(x, n4, s);
-    }
+    if (n4 > 0) scale_kernel<<<grid_size(n4, 256), 256, 0, st>>>(x, n4, s);
     if (n4 * 4 < n) scale_tail_kernel<<<1, 32, 0, st>>>(x, n4 * 4, n, s);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
-}
-
-static void fill_adj(Adj &a, const int64_t *row_ptr, const int32_t *col, const float *val, const int32_t *seg_row,
-                     const int64_t *seg_ptr, int64_t nseg, int64_t n)
-{
-    a.row_ptr = row_ptr; a.col = col; a.val = val; a.seg_row = seg_row; a.seg_ptr = seg_ptr; a.nseg = nseg; a.n = n;
 }
 
 }  // namespace drb
@@ -255,8 +246,7 @@ extern "C" int drb_lgcn_propagate(const float *d_E0, void *d_ws, int32_t U, int3
     cudaStream_t st = (cudaStream_t)stream;
     LgcnWs w;
     carve_lgcn(d_ws, U, I, F, DRB_OPT_SGD, &w);
-    Adj a;
-    fill_adj(a, d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, (int64_t)U + I);
+    const Adj a{d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, (long long)U + I};
     int rc = propagate_sum(a, d_E0, d_Em, w.Xa, w.Xb, F, L, st);
     if (rc != DRB_OK) return rc;
     return scale_table(d_Em, ((long long)U + I) * F, 1.f / (float)(L + 1), st);
@@ -280,9 +270,8 @@ extern "C" int drb_lgcn_bpr_train_steps(float *d_E0, void *d_ws, int32_t U, int3
     cudaStream_t st = (cudaStream_t)stream;
     LgcnWs w;
     carve_lgcn(d_ws, U, I, F, h->opt, &w);
-    Adj a;
     const long long nn = (long long)U + I;
-    fill_adj(a, d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, nn);
+    const Adj a{d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, nn};
     const size_t tab = sizeof(float) * (size_t)nn * F;
     const float inv = 1.f / (float)(L + 1);
     DRB_CUDA(cudaMemsetAsync(w.hdr, 0, sizeof(WsHeader), st));   // clear a stale NaN flag; sticky within the call
@@ -293,27 +282,16 @@ extern "C" int drb_lgcn_bpr_train_steps(float *d_E0, void *d_ws, int32_t U, int3
         if (rc == DRB_OK) rc = scale_table(w.Em, nn * F, inv, st);
         if (rc != DRB_OK) return rc;
         // phase 1 on the propagated tables (scores) + ego tables (norms): G = dL/dE_mean
-        StepParams p;
-        p.P = w.Em; p.Q = w.Em + (size_t)U * F;
+        StepParams p = split_step(h, U, I, d_bu + base, d_bi + base, d_bj + base, nb, adam_step0 + s, d_step_loss + s);
+        p.P = w.Em; p.Q = w.Em + (size_t)U * F; p.F = F;
         p.ws.hdr = w.hdr; p.ws.gP = w.G; p.ws.gQ = w.G + (size_t)U * F; p.ws.cntU = w.cntU; p.ws.cntI = w.cntI;
         p.ws.mP = w.m; p.ws.vP = w.v; p.ws.mQ = w.m ? w.m + (size_t)U * F : nullptr; p.ws.vQ = w.v ? w.v + (size_t)U * F : nullptr;
-        p.bu = d_bu + base; p.bi = d_bi + base; p.bj = d_bj + base;
-        p.n = nb; p.batch = nb; p.first_step = 0; p.n_steps = 1;
-        p.U = U; p.I = I; p.F = F; p.tile = 512;
-        p.lr = h->lr; p.reg1 = h->reg_1; p.reg2 = h->reg_2; p.opt = h->opt;
-        p.beta1 = h->beta1; p.beta2 = h->beta2; p.eps = h->eps; p.adam_step0 = adam_step0 + s;
-        p.step_loss = d_step_loss + s;
-        p.apply = apply ? 1 : 0;
-        p.dense_hint = 1;
         p.Pn = d_E0; p.Qn = d_E0 + (size_t)U * F;
-        p.gscale = 1.f; p.dense_grad = 1; p.neg_mult = 1.f; p.keep_counts = 0;
-        p.neg_row_ptr = nullptr; p.neg_col = nullptr; p.neg_out = nullptr; p.neg_seed = 0ull; p.loss = DRB_LOSS_BPR;
-        if (!apply) {
-            p.phases = 3;                                        // loss only: both phases in one launch, no update
-            return launch_steps(p, st, /*keep_status=*/true);
-        }
+        p.dense_grad = 1;
+        p.apply = apply ? 1 : 0;
+        p.phases = apply ? 1 : 3;                                // loss only: both phases in one launch, no update
+        if (!apply) return launch_steps(p, st, /*keep_status=*/true);
         DRB_CUDA(cudaMemsetAsync(w.G, 0, tab, st));
-        p.phases = 1;
         rc = launch_steps(p, st, true);
         if (rc != DRB_OK) return rc;
         // backward propagation of the gradient: Gs = sum_l A^l G

@@ -500,27 +500,13 @@ int fill_params(StepParams &p, float *P, float *Q, void *d_ws, int U, int I, int
     p.det = det;
     p.bu = bu; p.bi = bi; p.bj = bj;
     p.n = n; p.batch = batch; p.first_step = first; p.n_steps = nsteps;
-    p.U = U; p.I = I; p.F = F; p.tile = kTileMax;
-    p.lr = h->lr; p.reg1 = h->reg_1; p.reg2 = h->reg_2; p.opt = h->opt;
-    p.beta1 = h->beta1; p.beta2 = h->beta2; p.eps = h->eps;
+    p.U = U; p.I = I; p.F = F;
+    copy_hyper(p, h);
+    p.loss = h->loss;
     p.adam_step0 = adam_step0;
     p.step_loss = d_step_loss;
     p.apply = apply;
-    p.phases = 3;
-    p.dense_hint = -1;
-    p.Pn = nullptr;
-    p.Qn = nullptr;
-    p.gscale = 1.f;
-    p.dense_grad = 0;
-    p.neg_mult = 1.f;
-    p.keep_counts = 0;
-    p.neg_row_ptr = nullptr;
-    p.neg_col = nullptr;
-    p.neg_out = nullptr;
-    p.neg_seed = 0ull;
-    p.loss = h->loss;
     p.bias = d_bias;
-    p.step_offsets = nullptr;
     return DRB_OK;
 }
 }  // namespace drb
@@ -723,10 +709,7 @@ extern "C" int drb_gather_triples(const int32_t *d_triples, const int64_t *d_per
 {
     DRB_REQUIRE(d_triples && d_bu && d_bi && d_bj && n >= 0, "gather_triples: bad arguments");
     if (n == 0) return DRB_OK;
-    long long blocks = (n + 255) / 256;
-    long long cap = (long long)sm_count() * 16;
-    if (blocks > cap) blocks = cap;
-    gather_triples_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(d_triples, d_perm, n, d_bu, d_bi, d_bj);
+    gather_triples_kernel<<<grid_size(n, 256), 256, 0, (cudaStream_t)stream>>>(d_triples, d_perm, n, d_bu, d_bi, d_bj);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }

@@ -499,28 +499,6 @@ __global__ void neumf_finalize_kernel(const double *__restrict__ red, float reg1
     }
 }
 
-// dense optimiser step on the tower block (SGD, or torch.optim.Adam's single-tensor rule)
-__global__ void neumf_update_w_kernel(float *__restrict__ W, float *__restrict__ g, float *__restrict__ m,
-                                      float *__restrict__ v, long long n, float lr, int opt, float beta1, float beta2,
-                                      float eps, float step_size, float bc2_sqrt, const WsHeader *hdr)
-{
-    if (hdr->status != 0) return;
-    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (long long)gridDim.x * blockDim.x) {
-        float gk = g[k];
-        g[k] = 0.f;
-        if (opt == DRB_OPT_SGD) {
-            W[k] = W[k] - lr * gk;
-        } else {
-            float mm = m[k], vv = v[k];
-            mm = mm + (gk - mm) * (1.f - beta1);
-            vv = vv * beta2 + (1.f - beta2) * gk * gk;
-            float denom = sqrtf(vv) / bc2_sqrt + eps;
-            W[k] = W[k] - step_size * (mm / denom);
-            m[k] = mm; v[k] = vv;
-        }
-    }
-}
-
 // scores[r] = wp . cat(UG[u]*IG[item], A_L[r]) + bp      (inference head)
 __global__ void neumf_score_kernel(const float *__restrict__ UG, const float *__restrict__ IG, const float *__restrict__ wp,
                                    const float *__restrict__ AL, const int64_t *__restrict__ users,
@@ -570,11 +548,36 @@ int colsum_acc(const float *dZ, long long M, int N, float *gb, cudaStream_t st)
     return DRB_OK;
 }
 
-static int grid1d(long long n, int block, int per_sm = 16)
+// dense optimiser step on a flat block (SGD, or torch.optim.Adam's single-tensor rule); clears the gradient
+__global__ void dense_update_kernel(float *__restrict__ W, float *__restrict__ g, float *__restrict__ m, float *__restrict__ v,
+                                    long long n, float lr, int opt, float beta1, float beta2, float eps, float step_size,
+                                    float bc2_sqrt, const WsHeader *hdr)
 {
-    long long b = (n + block - 1) / block, cap = (long long)sm_count() * per_sm;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
+    if (hdr->status != 0) return;
+    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (long long)gridDim.x * blockDim.x) {
+        const float gk = g[k];
+        g[k] = 0.f;
+        if (opt == DRB_OPT_SGD) {
+            W[k] = W[k] - lr * gk;
+        } else {
+            float mm = m[k], vv = v[k];
+            mm = mm + (gk - mm) * (1.f - beta1);
+            vv = vv * beta2 + (1.f - beta2) * gk * gk;
+            W[k] = W[k] - step_size * (mm / (sqrtf(vv) / bc2_sqrt + eps));
+            m[k] = mm; v[k] = vv;
+        }
+    }
+}
+int dense_update(float *W, float *g, float *m, float *v, long long n, const drb_hyper *h, long long adam_step, const WsHeader *hdr,
+                 cudaStream_t st)
+{
+    const double t = (double)(adam_step + 1);
+    const float step_size = (float)((double)h->lr / (1.0 - pow((double)h->beta1, t)));
+    const float bc2_sqrt = (float)sqrt(1.0 - pow((double)h->beta2, t));
+    dense_update_kernel<<<grid_size(n, 256), 256, 0, st>>>(W, g, m, v, n, h->lr, h->opt, h->beta1, h->beta2, h->eps, step_size,
+                                                           bc2_sqrt, hdr);
+    DRB_CUDA(cudaGetLastError());
+    return DRB_OK;
 }
 
 // tower forward on `rows` rows already gathered into acts' A_0 block
@@ -589,7 +592,7 @@ static int tower_forward(const NeumfDims &d, const float *W, float *acts, long l
         if (rc != DRB_OK) return rc;
         if (drop.p > 0.f && l + 1 < d.L) {   // the next Linear sees dropout(relu(z_l)); the tower output is not dropped
             long long n4 = rows * d.n[l + 1] / 4;
-            neumf_dropout_kernel<<<grid1d(n4, 256), 256, 0, st>>>(out, n4, drop, (uint32_t)(l + 1));
+            neumf_dropout_kernel<<<grid_size(n4, 256), 256, 0, st>>>(out, n4, drop, (uint32_t)(l + 1));
             DRB_CUDA(cudaGetLastError());
         }
     }
@@ -703,7 +706,7 @@ extern "C" int drb_neumf_bpr_train_steps(float *d_UG, float *d_IG, float *d_UM, 
         }
         // forward
         if (use_tower && !fused) {
-            neumf_gather_kernel<<<grid1d(R * 2 * (d.D / 4), 256), 256, 0, st>>>(d_UM, d_IM, bu, bi, bj, B, d.D, w.acts, drop);
+            neumf_gather_kernel<<<grid_size(R * 2 * (d.D / 4), 256), 256, 0, st>>>(d_UM, d_IM, bu, bi, bj, B, d.D, w.acts, drop);
             DRB_CUDA(cudaGetLastError());
             rc = tower_forward(d, d_W, w.acts, R, R, tower_dtype, drop, st);
             if (rc != DRB_OK) return rc;
@@ -713,7 +716,7 @@ extern "C" int drb_neumf_bpr_train_steps(float *d_UG, float *d_IG, float *d_UM, 
         if (!fused) {
             int hw = 1;
             while (hw < F / 4 && hw < 32) hw <<= 1;              // lanes per triple in the head kernel
-            neumf_head_kernel<<<grid1d(B, 8 * (32 / hw), 8), 256, sizeof(float) * (2 * F + 1), st>>>(
+            neumf_head_kernel<<<grid_size(B, 8 * (32 / hw), 8), 256, sizeof(float) * (2 * F + 1), st>>>(
                 d_UG, d_IG, d_UM, d_IM, d_W + d.wp_off, AL, bu, bi, bj, B, F, d.D, has_reg, apply ? 1 : 0, hw, mode, w.gUG, w.gIG,
                 w.gW + d.wp_off, dZ, w.cntU, w.cntI, w.red);
             DRB_CUDA(cudaGetLastError());
@@ -744,18 +747,12 @@ extern "C" int drb_neumf_bpr_train_steps(float *d_UG, float *d_IG, float *d_UM, 
             float *t = cur; cur = nxt; nxt = t;
         }
         if (use_tower && !fused) {
-            neumf_scatter_kernel<<<grid1d(B * (d.D / 4), 256), 256, 0, st>>>(cur, bu, bi, bj, B, d.D, w.gUM, w.gIM, drop);
+            neumf_scatter_kernel<<<grid_size(B * (d.D / 4), 256), 256, 0, st>>>(cur, bu, bi, bj, B, d.D, w.gUM, w.gIM, drop);
             DRB_CUDA(cudaGetLastError());
         }
         // apply: table pairs through the MF dense sweep, tower block through the small dense kernel
-        StepParams p;
-        p.bu = bu; p.bi = bi; p.bj = bj; p.n = B; p.batch = B; p.first_step = 0; p.n_steps = 1;
-        p.U = U; p.I = I; p.tile = 512;
-        p.lr = h->lr; p.reg1 = h->reg_1; p.reg2 = h->reg_2; p.opt = h->opt;
-        p.beta1 = h->beta1; p.beta2 = h->beta2; p.eps = h->eps; p.adam_step0 = adam_step0 + s;
-        p.step_loss = w.red + 12;                                // scratch: the real loss was written by finalize
-        p.apply = 1; p.phases = 2; p.dense_hint = 1; p.Pn = nullptr; p.Qn = nullptr; p.gscale = 1.f; p.dense_grad = 0;
-        p.neg_row_ptr = nullptr; p.neg_col = nullptr; p.neg_out = nullptr; p.neg_seed = 0ull; p.loss = DRB_LOSS_BPR;
+        StepParams p = split_step(h, U, I, bu, bi, bj, B, adam_step0 + s, w.red + 12);   // scratch: finalize wrote the loss
+        p.phases = 2;
         p.ws.cntU = w.cntU; p.ws.cntI = w.cntI;
         // (UG, IG): negative occurrences weigh 2x (lines :157 and :158 both add |IG_j|)
         p.P = d_UG; p.Q = d_IG; p.F = F; p.ws.hdr = w.hdrG; p.ws.gP = w.gUG; p.ws.gQ = w.gIG;
@@ -766,13 +763,8 @@ extern "C" int drb_neumf_bpr_train_steps(float *d_UG, float *d_IG, float *d_UM, 
         p.P = d_UM; p.Q = d_IM; p.F = d.D; p.ws.hdr = w.hdrM; p.ws.gP = w.gUM; p.ws.gQ = w.gIM;
         p.ws.mP = w.mUM; p.ws.vP = w.vUM; p.ws.mQ = w.mIM; p.ws.vQ = w.vIM; p.neg_mult = 0.f; p.keep_counts = 0;
         rc = launch_steps(p, st, true);
+        if (rc == DRB_OK) rc = dense_update(d_W, w.gW, w.mW, w.vW, d.nW, h, adam_step0 + s, w.hdrG, st);
         if (rc != DRB_OK) return rc;
-        double tt = (double)(adam_step0 + s + 1);
-        float step_size = (float)((double)h->lr / (1.0 - pow((double)h->beta1, tt)));
-        float bc2_sqrt = (float)sqrt(1.0 - pow((double)h->beta2, tt));
-        neumf_update_w_kernel<<<grid1d(d.nW, 256), 256, 0, st>>>(d_W, w.gW, w.mW, w.vW, d.nW, h->lr, h->opt, h->beta1, h->beta2,
-                                                                 h->eps, step_size, bc2_sqrt, w.hdrG);
-        DRB_CUDA(cudaGetLastError());
     }
     if (sync_and_check) return check_nan(w.hdrG, st, nan_step);
     return DRB_OK;
@@ -795,8 +787,8 @@ extern "C" int drb_neumf_scores(const float *d_UG, const float *d_IG, const floa
     for (long long row0 = 0; row0 < total; row0 += max_rows) {
         long long rows = total - row0 < max_rows ? total - row0 : max_rows;
         if (mode != 1) {
-            neumf_gather_pairs_kernel<<<grid1d(rows * 2 * (d.D / 4), 256), 256, 0, st>>>(d_UM, d_IM, d_users, d_items, row0, rows,
-                                                                                       per_user, d.D, w.dA);
+            neumf_gather_pairs_kernel<<<grid_size(rows * 2 * (d.D / 4), 256), 256, 0, st>>>(d_UM, d_IM, d_users, d_items, row0, rows,
+                                                                                            per_user, d.D, w.dA);
             DRB_CUDA(cudaGetLastError());
         }
         // use dA as A_0 and dB as ping-pong for the hidden layers (independent of the optimiser layout)
@@ -809,8 +801,8 @@ extern "C" int drb_neumf_scores(const float *d_UG, const float *d_IG, const floa
             if (rc != DRB_OK) return rc;
             in = out;
         }
-        neumf_score_kernel<<<grid1d(rows * 32, 256), 256, 0, st>>>(d_UG, d_IG, d_W + d.wp_off, in, d_users, d_items, row0, rows,
-                                                                  per_user, F, mode, d_scores);
+        neumf_score_kernel<<<grid_size(rows * 32, 256), 256, 0, st>>>(d_UG, d_IG, d_W + d.wp_off, in, d_users, d_items, row0, rows,
+                                                                      per_user, F, mode, d_scores);
         DRB_CUDA(cudaGetLastError());
     }
     return DRB_OK;

@@ -108,13 +108,6 @@ static size_t nfm_head_bytes(const NfmDims &d, int opt)
     return (size_t)((uintptr_t)w.pred - 256);
 }
 
-static int nfm_grid(long long items, int block)
-{
-    long long b = (items + block - 1) / block, cap = (long long)sm_count() * 16;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
-}
-
 __device__ __forceinline__ float nfm_act(int act, float z)
 {
     if (act == 0) return z > 0.f ? z : 0.f;
@@ -454,27 +447,6 @@ __global__ void nfm_scatter_kernel(const float *__restrict__ dh, const float *__
     }
 }
 
-// dense optimiser step on a flat block (SGD, or torch.optim.Adam's single-tensor rule); clears the gradient
-__global__ void nfm_update_kernel(float *__restrict__ W, float *__restrict__ g, float *__restrict__ m, float *__restrict__ v,
-                                  long long n, float lr, int opt, float beta1, float beta2, float eps, float step_size,
-                                  float bc2_sqrt, const WsHeader *hdr)
-{
-    if (hdr->status != 0) return;
-    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (long long)gridDim.x * blockDim.x) {
-        const float gk = g[k];
-        g[k] = 0.f;
-        if (opt == DRB_OPT_SGD) {
-            W[k] = W[k] - lr * gk;
-        } else {
-            float mm = m[k], vv = v[k];
-            mm = mm + (gk - mm) * (1.f - beta1);
-            vv = vv * beta2 + (1.f - beta2) * gk * gk;
-            W[k] = W[k] - step_size * (mm / (sqrtf(vv) / bc2_sqrt + eps));
-            m[k] = mm; v[k] = vv;
-        }
-    }
-}
-
 // BatchNorm over the rows of x (two halves of B rows); statistics into w.bnm[slot], running statistics updated
 static int nfm_bn_train(const NfmDims &d, const NfmWs &w, int slot, const float *x, long long B, const float *gamma,
                         const float *beta, float *rm, float *rv, float *xhat, float *y, cudaStream_t st)
@@ -491,7 +463,7 @@ static int nfm_bn_train(const NfmDims &d, const NfmWs &w, int slot, const float 
     nfm_bn_finish_kernel<<<(F + 63) / 64, 64, 0, st>>>(w.stats, B, F, 0, bnm, rm, rv);
     nfm_colstat_kernel<<<grid, 256, 0, st>>>(x, nullptr, B, F, bnm, 1, w.stats);
     nfm_bn_finish_kernel<<<(F + 63) / 64, 64, 0, st>>>(w.stats, B, F, 1, bnm, rm, rv);
-    nfm_bn_apply_kernel<<<nfm_grid(2 * B * F, 256), 256, 0, st>>>(x, B, 2 * B, F, bnm, rm, rv, gamma, beta, 1, xhat, y);
+    nfm_bn_apply_kernel<<<grid_size(2 * B * F, 256), 256, 0, st>>>(x, B, 2 * B, F, bnm, rm, rv, gamma, beta, 1, xhat, y);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }
@@ -509,7 +481,7 @@ static int nfm_bn_backward(const NfmDims &d, const NfmWs &w, int slot, const flo
     dim3 grid((unsigned)blocks, 2);
     nfm_colstat_kernel<<<grid, 256, 0, st>>>(dy, xhat, B, F, nullptr, 2, w.stats);
     nfm_bn_param_grad_kernel<<<(F + 63) / 64, 64, 0, st>>>(w.stats, F, ggamma, gbeta);
-    nfm_bn_bwd_kernel<<<nfm_grid(2 * B * F, 256), 256, 0, st>>>(dy, xhat, w.stats, bnm, gamma, B, 2 * B, F, dx);
+    nfm_bn_bwd_kernel<<<grid_size(2 * B * F, 256), 256, 0, st>>>(dy, xhat, w.stats, bnm, gamma, B, 2 * B, F, dx);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }
@@ -544,29 +516,16 @@ extern "C" int drb_nfm_workspace_init(void *d_ws, int32_t U, int32_t I, int32_t 
 
 // n_steps synchronous NFM + BPR steps (apply != 0) or the loss of one batch (apply == 0: like calc_loss under train(), the
 // BatchNorm running statistics still move).  act: 0 relu, 1 sigmoid, 2 tanh.
+// With d_keep != NULL nn.Dropout is active (dropout = config['dropout'] > 0, the reference default 0.5).  d_keep: the masks
+// torch's Dropout modules draw, as bytes (0 / 1), for the n_steps steps in order: per step [forward call: pos, neg][site:
+// FM_layers' Dropout, then the one behind each activation][batch][F] (the caller draws them on torch's CPU generator in exactly
+// that order; a ragged last batch uses its own row count).  Every step must hold `batch` triples when n_steps > 1.
 extern "C" int drb_nfm_bpr_train_steps(float *d_P, float *d_Q, float *d_bias, float *d_N, float *d_Rs, void *d_ws, int32_t U,
                                        int32_t I, int32_t F, int32_t L, int32_t batch_norm, int32_t act, int64_t max_rows,
                                        const int32_t *d_bu, const int32_t *d_bi, const int32_t *d_bj, int64_t n, int64_t batch,
                                        int64_t first_step, int64_t n_steps, const drb_hyper *h, int64_t adam_step0, int32_t apply,
-                                       int32_t tower_dtype, double *d_step_loss, int32_t sync_and_check, int64_t *nan_step,
-                                       void *stream)
-{
-    return drb_nfm_bpr_train_steps_dropout(d_P, d_Q, d_bias, d_N, d_Rs, d_ws, U, I, F, L, batch_norm, act, max_rows, d_bu, d_bi, d_bj,
-                                           n, batch, first_step, n_steps, h, adam_step0, apply, tower_dtype, nullptr, 0.f,
-                                           d_step_loss, sync_and_check, nan_step, stream);
-}
-
-// The same with nn.Dropout active (dropout = config['dropout'] > 0, the reference default 0.5).  d_keep: the masks torch's Dropout
-// modules draw, as bytes (0 / 1), for the n_steps steps in order: per step [forward call: pos, neg][site: FM_layers' Dropout, then
-// the one behind each activation][batch][F] (the caller draws them on torch's CPU generator in exactly that order; a ragged
-// last batch uses its own row count).  Every step must hold `batch` triples when n_steps > 1.
-extern "C" int drb_nfm_bpr_train_steps_dropout(float *d_P, float *d_Q, float *d_bias, float *d_N, float *d_Rs, void *d_ws, int32_t U,
-                                               int32_t I, int32_t F, int32_t L, int32_t batch_norm, int32_t act, int64_t max_rows,
-                                               const int32_t *d_bu, const int32_t *d_bi, const int32_t *d_bj, int64_t n,
-                                               int64_t batch, int64_t first_step, int64_t n_steps, const drb_hyper *h,
-                                               int64_t adam_step0, int32_t apply, int32_t tower_dtype, const uint8_t *d_keep,
-                                               float dropout, double *d_step_loss, int32_t sync_and_check, int64_t *nan_step,
-                                               void *stream)
+                                       int32_t tower_dtype, const uint8_t *d_keep, float dropout, double *d_step_loss,
+                                       int32_t sync_and_check, int64_t *nan_step, void *stream)
 {
     NfmDims d;
     DRB_REQUIRE(d_keep == nullptr || (dropout > 0.f && dropout < 1.f), "nfm: dropout masks need 0 < dropout < 1");
@@ -595,7 +554,7 @@ extern "C" int drb_nfm_bpr_train_steps_dropout(float *d_P, float *d_Q, float *d_
         const uint8_t *keep = d_keep ? d_keep + (size_t)s * 2 * nsites * (size_t)batch * F : nullptr;   // this step's masks
         int rc = DRB_OK;
         // ---- forward (both calls at once; BatchNorm statistics per half)
-        nfm_product_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(d_P, d_Q, bu, bi, bj, B, R, F, w.e);
+        nfm_product_kernel<<<grid_size(tot, 256), 256, 0, st>>>(d_P, d_Q, bu, bi, bj, B, R, F, w.e);
         DRB_CUDA(cudaGetLastError());
         float *h_fm = w.e;                                                // output of FM_layers
         if (d.bn) {
@@ -604,7 +563,7 @@ extern "C" int drb_nfm_bpr_train_steps_dropout(float *d_P, float *d_Q, float *d_
             h_fm = w.h0;
         }
         if (keep) {
-            nfm_dropout_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(h_fm, keep, B, tot, F, 0, nsites, drop_scale);
+            nfm_dropout_kernel<<<grid_size(tot, 256), 256, 0, st>>>(h_fm, keep, B, tot, F, 0, nsites, drop_scale);
             DRB_CUDA(cudaGetLastError());
         }
         const float *hin = h_fm;
@@ -612,42 +571,42 @@ extern "C" int drb_nfm_bpr_train_steps_dropout(float *d_P, float *d_Q, float *d_
             const float *W = d_N + d.oW[l], *b = W + (size_t)F * F;
             rc = gemm_nt(tower_dtype, R, F, F, hin, F, W, F, w.zpre[l], F, st);
             if (rc != DRB_OK) return rc;
-            nfm_bias_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.zpre[l], b, tot, F, d.bn ? nullptr : w.z[l]);
+            nfm_bias_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.zpre[l], b, tot, F, d.bn ? nullptr : w.z[l]);
             DRB_CUDA(cudaGetLastError());
             if (d.bn) {
                 rc = nfm_bn_train(d, w, 1 + l, w.zpre[l], B, d_N + d.oBN[l], d_N + d.oBN[l] + F, d_Rs + (size_t)(1 + l) * 2 * F,
                                   d_Rs + (size_t)(1 + l) * 2 * F + F, w.xh[l], w.z[l], st);
                 if (rc != DRB_OK) return rc;
             }
-            nfm_act_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.z[l], tot, d.act, w.h[l]);
+            nfm_act_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.z[l], tot, d.act, w.h[l]);
             DRB_CUDA(cudaGetLastError());
             if (keep) {
-                nfm_dropout_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.h[l], keep, B, tot, F, 1 + l, nsites, drop_scale);
+                nfm_dropout_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.h[l], keep, B, tot, F, 1 + l, nsites, drop_scale);
                 DRB_CUDA(cudaGetLastError());
             }
             hin = w.h[l];
         }
-        nfm_head_kernel<<<nfm_grid(R * 32, 256), 256, 0, st>>>(hin, d_bias, U, I, bu, bi, bj, B, R, F, wp, w.fm, w.pred);
+        nfm_head_kernel<<<grid_size(R * 32, 256), 256, 0, st>>>(hin, d_bias, U, I, bu, bi, bj, B, R, F, wp, w.fm, w.pred);
         DRB_CUDA(cudaMemsetAsync(w.hdr, 0, kHdrResetBytes, st));
-        nfm_pair_kernel<<<nfm_grid(B * 32, 256), 256, 0, st>>>(w.pred, d_P, d_Q, bu, bi, bj, B, F, has_reg, apply ? 1 : 0, w.coef,
-                                                             w.cntU, w.cntI, w.hdr->acc[0]);
+        nfm_pair_kernel<<<grid_size(B * 32, 256), 256, 0, st>>>(w.pred, d_P, d_Q, bu, bi, bj, B, F, has_reg, apply ? 1 : 0, w.coef,
+                                                                w.cntU, w.cntI, w.hdr->acc[0]);
         nfm_finalize_kernel<<<1, 1, 0, st>>>(w.hdr, h->reg_1, h->reg_2, d_step_loss + s, first_step + s);
         DRB_CUDA(cudaGetLastError());
         if (!apply) break;
         // ---- backward
-        nfm_head_bwd_kernel<<<nfm_grid(B * 32, 256), 256, sizeof(float) * F, st>>>(w.coef, w.fm, wp, U, I, bu, bi, bj, B, R, F, w.dh,
-                                                                                 w.gN + d.o_wp, w.gB);
+        nfm_head_bwd_kernel<<<grid_size(B * 32, 256), 256, sizeof(float) * F, st>>>(w.coef, w.fm, wp, U, I, bu, bi, bj, B, R, F, w.dh,
+                                                                                    w.gN + d.o_wp, w.gB);
         DRB_CUDA(cudaGetLastError());
         for (int l = L - 1; l >= 0; --l) {
             const float *W = d_N + d.oW[l];
             const float *hprev = l == 0 ? (d.bn ? w.h0 : w.e) : w.h[l - 1];
             float *gW = w.gN + d.oW[l], *gb = gW + (size_t)F * F;
             if (keep)
-                nfm_act_bwd_drop_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.dh, w.z[l], keep, B, tot, F, 1 + l, nsites, drop_scale,
-                                                                          d.act, w.tmp);
+                nfm_act_bwd_drop_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.dh, w.z[l], keep, B, tot, F, 1 + l, nsites, drop_scale,
+                                                                             d.act, w.tmp);
             else
-                nfm_act_bwd_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.dh, w.z[l], w.h[l], tot, d.act, w.tmp);   // d act input
-            DRB_CUDA(cudaGetLastError());
+                nfm_act_bwd_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.dh, w.z[l], w.h[l], tot, d.act, w.tmp);   // d act input
+                                                                        DRB_CUDA(cudaGetLastError());
             float *dz = w.tmp;                                            // d Linear output
             if (d.bn) {
                 rc = nfm_bn_backward(d, w, 1 + l, w.tmp, w.xh[l], B, d_N + d.oBN[l], w.gN + d.oBN[l], w.gN + d.oBN[l] + F, w.dh, st);
@@ -662,7 +621,7 @@ extern "C" int drb_nfm_bpr_train_steps_dropout(float *d_P, float *d_Q, float *d_
             if (dprev != w.dh) DRB_CUDA(cudaMemcpyAsync(w.dh, dprev, sizeof(float) * (size_t)tot, cudaMemcpyDeviceToDevice, st));
         }
         if (keep) {                                                       // backward of FM_layers' Dropout
-            nfm_dropout_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.dh, keep, B, tot, F, 0, nsites, drop_scale);
+            nfm_dropout_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.dh, keep, B, tot, F, 0, nsites, drop_scale);
             DRB_CUDA(cudaGetLastError());
         }
         if (d.bn) {
@@ -670,32 +629,18 @@ extern "C" int drb_nfm_bpr_train_steps_dropout(float *d_P, float *d_Q, float *d_
             if (rc != DRB_OK) return rc;
             DRB_CUDA(cudaMemcpyAsync(w.dh, w.tmp, sizeof(float) * (size_t)tot, cudaMemcpyDeviceToDevice, st));
         }
-        nfm_scatter_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.dh, d_P, d_Q, bu, bi, bj, B, R, F, w.gP, w.gQ);
+        nfm_scatter_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.dh, d_P, d_Q, bu, bi, bj, B, R, F, w.gP, w.gQ);
         DRB_CUDA(cudaGetLastError());
         // ---- update: factor tables through the MF dense sweep (counter-weighted regulariser), the rest densely
-        StepParams p;
-        p.P = d_P; p.Q = d_Q;
+        StepParams p = split_step(h, U, I, bu, bi, bj, B, adam_step0 + s, w.scratch);
+        p.P = d_P; p.Q = d_Q; p.F = F;
         p.ws.hdr = w.hdr; p.ws.gP = w.gP; p.ws.gQ = w.gQ; p.ws.cntU = w.cntU; p.ws.cntI = w.cntI;
-        p.ws.mP = w.mP; p.ws.vP = w.vP; p.ws.mQ = w.mQ; p.ws.vQ = w.vQ; p.ws.gB = p.ws.mB = p.ws.vB = nullptr;
-        p.bu = bu; p.bi = bi; p.bj = bj; p.n = B; p.batch = B; p.first_step = 0; p.n_steps = 1;
-        p.U = U; p.I = I; p.F = F; p.tile = 512;
-        p.lr = h->lr; p.reg1 = h->reg_1; p.reg2 = h->reg_2; p.opt = h->opt;
-        p.beta1 = h->beta1; p.beta2 = h->beta2; p.eps = h->eps; p.adam_step0 = adam_step0 + s;
-        p.step_loss = w.scratch;
-        p.apply = 1; p.phases = 2; p.dense_hint = 1; p.Pn = nullptr; p.Qn = nullptr; p.gscale = 1.f; p.dense_grad = 0;
-        p.neg_mult = 1.f; p.keep_counts = 0;
-        p.neg_row_ptr = nullptr; p.neg_col = nullptr; p.neg_out = nullptr; p.neg_seed = 0ull; p.loss = DRB_LOSS_BPR;
+        p.ws.mP = w.mP; p.ws.vP = w.vP; p.ws.mQ = w.mQ; p.ws.vQ = w.vQ;
+        p.phases = 2;
         rc = launch_steps(p, st, true);
+        if (rc == DRB_OK) rc = dense_update(d_bias, w.gB, w.mB, w.vB, (long long)U + I + 1, h, adam_step0 + s, w.hdr, st);
+        if (rc == DRB_OK) rc = dense_update(d_N, w.gN, w.mN, w.vN, d.nN, h, adam_step0 + s, w.hdr, st);
         if (rc != DRB_OK) return rc;
-        const double tt = (double)(adam_step0 + s + 1);
-        const float step_size = (float)((double)h->lr / (1.0 - pow((double)h->beta1, tt)));
-        const float bc2_sqrt = (float)sqrt(1.0 - pow((double)h->beta2, tt));
-        const long long nb = (long long)U + I + 1;
-        nfm_update_kernel<<<nfm_grid(nb, 256), 256, 0, st>>>(d_bias, w.gB, w.mB, w.vB, nb, h->lr, h->opt, h->beta1, h->beta2, h->eps,
-                                                           step_size, bc2_sqrt, w.hdr);
-        nfm_update_kernel<<<nfm_grid(d.nN, 256), 256, 0, st>>>(d_N, w.gN, w.mN, w.vN, d.nN, h->lr, h->opt, h->beta1, h->beta2,
-                                                             h->eps, step_size, bc2_sqrt, w.hdr);
-        DRB_CUDA(cudaGetLastError());
     }
     if (sync_and_check) return check_nan(d_ws, st, nan_step);
     return DRB_OK;
@@ -719,27 +664,27 @@ extern "C" int drb_nfm_scores(const float *d_P, const float *d_Q, const float *d
         const long long rows = n - row0 < max_rows ? n - row0 : max_rows, tot = rows * F;
         const int32_t *uu = d_u + row0, *ii = d_i + row0;
         // "B = rows": every row is a 'pos' row of the product / head kernels
-        nfm_product_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(d_P, d_Q, uu, ii, ii, rows, rows, F, w.e);
+        nfm_product_kernel<<<grid_size(tot, 256), 256, 0, st>>>(d_P, d_Q, uu, ii, ii, rows, rows, F, w.e);
         const float *hin = w.e;
         if (d.bn) {
-            nfm_bn_apply_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.e, rows, rows, F, nullptr, d_Rs, d_Rs + F, d_N + d.o_bn0,
-                                                                  d_N + d.o_bn0 + F, 0, nullptr, w.h0);
+            nfm_bn_apply_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.e, rows, rows, F, nullptr, d_Rs, d_Rs + F, d_N + d.o_bn0,
+                                                                     d_N + d.o_bn0 + F, 0, nullptr, w.h0);
             hin = w.h0;
         }
         for (int l = 0; l < L; ++l) {
             const float *W = d_N + d.oW[l], *b = W + (size_t)F * F;
             int rc = gemm_nt(tower_dtype, rows, F, F, hin, F, W, F, w.zpre[l], F, st);
             if (rc != DRB_OK) return rc;
-            nfm_bias_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.zpre[l], b, tot, F, d.bn ? nullptr : w.z[l]);
+            nfm_bias_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.zpre[l], b, tot, F, d.bn ? nullptr : w.z[l]);
             if (d.bn)
-                nfm_bn_apply_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.zpre[l], rows, rows, F, nullptr,
-                                                                      d_Rs + (size_t)(1 + l) * 2 * F, d_Rs + (size_t)(1 + l) * 2 * F + F,
-                                                                      d_N + d.oBN[l], d_N + d.oBN[l] + F, 0, nullptr, w.z[l]);
-            nfm_act_kernel<<<nfm_grid(tot, 256), 256, 0, st>>>(w.z[l], tot, d.act, w.h[l]);
+                nfm_bn_apply_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.zpre[l], rows, rows, F, nullptr,
+                                                                         d_Rs + (size_t)(1 + l) * 2 * F, d_Rs + (size_t)(1 + l) * 2 * F + F,
+                                                                         d_N + d.oBN[l], d_N + d.oBN[l] + F, 0, nullptr, w.z[l]);
+            nfm_act_kernel<<<grid_size(tot, 256), 256, 0, st>>>(w.z[l], tot, d.act, w.h[l]);
             hin = w.h[l];
         }
-        nfm_head_kernel<<<nfm_grid(rows * 32, 256), 256, 0, st>>>(hin, d_bias, U, I, uu, ii, ii, rows, rows, F, wp, nullptr,
-                                                                d_scores + row0);
+        nfm_head_kernel<<<grid_size(rows * 32, 256), 256, 0, st>>>(hin, d_bias, U, I, uu, ii, ii, rows, rows, F, wp, nullptr,
+                                                                   d_scores + row0);
         DRB_CUDA(cudaGetLastError());
     }
     return DRB_OK;

@@ -15,7 +15,7 @@
 //   per layer, backwards   ngcf_act_bwd_kernel (normalize + LeakyReLU backward) -> bias column sums, two weight-gradient
 //               GEMMs, two input-gradient GEMMs -> ngcf_mix_bwd_kernel (dE, dX) -> spmm (A_hat symmetric) -> add
 //   update      phase 2 of the MF kernel on the ego table (dense gradient + counter-weighted regulariser, SGD / Adam),
-//               drb_dense_update on the flat layer block.
+//               dense_update (neumf.cu) on the flat layer block.
 // Parameter block W (flat fp32, module registration order :106-108 / :46-47): per layer W1 [out, in], b1 [out], W2 [out, in],
 // b2 [out].  HBM-bound like LightGCN: every step streams the [n, width] activations of every layer a handful of times.
 #include "gemm.cuh"
@@ -106,13 +106,6 @@ static size_t carve_ngcf(void *base, const NgcfDims &q, int opt, NgcfWs *w)
     }
     if (w) *w = t;
     return off;
-}
-
-static int ngcf_grid(long long items, int block)
-{
-    long long b = (items + block - 1) / block, cap = (long long)sm_count() * 16;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
 }
 
 // scalar forms of the two mix kernels for layer widths that are not multiples of 4
@@ -293,33 +286,12 @@ __global__ void ngcf_finalize_kernel(WsHeader *hdr, float reg1, float reg2, doub
     if (isnan(loss)) { hdr->status = DRB_ERR_NAN_LOSS; hdr->nan_step = step; }
 }
 
-// dense optimiser step on the flat layer block (SGD, or torch.optim.Adam's single-tensor rule); clears the gradient
-__global__ void ngcf_update_w_kernel(float *__restrict__ W, float *__restrict__ g, float *__restrict__ m, float *__restrict__ v,
-                                     long long n, float lr, int opt, float beta1, float beta2, float eps, float step_size,
-                                     float bc2_sqrt, const WsHeader *hdr)
-{
-    if (hdr->status != 0) return;
-    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (long long)gridDim.x * blockDim.x) {
-        const float gk = g[k];
-        g[k] = 0.f;
-        if (opt == DRB_OPT_SGD) {
-            W[k] = W[k] - lr * gk;
-        } else {
-            float mm = m[k], vv = v[k];
-            mm = mm + (gk - mm) * (1.f - beta1);
-            vv = vv * beta2 + (1.f - beta2) * gk * gk;
-            W[k] = W[k] - step_size * (mm / (sqrtf(vv) / bc2_sqrt + eps));
-            m[k] = mm; v[k] = vv;
-        }
-    }
-}
-
 // keep: masks of the L layers concatenated ([n, d[1]], [n, d[2]], ...), or nullptr
 static int ngcf_forward(const NgcfDims &q, const NgcfWs &w, const Adj &adj, const float *E0, const float *W, int dtype,
                         cudaStream_t st, const uint8_t *keep = nullptr, float scale = 1.f)
 {
     const long long n = q.n;
-    ngcf_copy_block_kernel<<<ngcf_grid(n * q.d[0], 256), 256, 0, st>>>(E0, n, q.d[0], w.ALL, q.C, 0);
+    ngcf_copy_block_kernel<<<grid_size(n * q.d[0], 256), 256, 0, st>>>(E0, n, q.d[0], w.ALL, q.C, 0);
     DRB_CUDA(cudaGetLastError());
     const float *E = E0;
     for (int l = 0; l < q.L; ++l) {
@@ -327,14 +299,14 @@ static int ngcf_forward(const NgcfDims &q, const NgcfWs &w, const Adj &adj, cons
         const float *W1 = W + q.w_off[l], *b1 = W1 + (size_t)in * out, *W2 = b1 + out, *b2 = W2 + (size_t)in * out;
         int rc = launch_spmm(adj, E, w.X[l], nullptr, in, st);
         if (rc != DRB_OK) return rc;
-        if (in % 4 == 0) ngcf_mix_kernel<<<ngcf_grid(n * (in / 4), 256), 256, 0, st>>>(E, w.X[l], n, in, w.ST);
-        else ngcf_mix_scalar_kernel<<<ngcf_grid(n * in, 256), 256, 0, st>>>(E, w.X[l], n, in, w.ST);
+        if (in % 4 == 0) ngcf_mix_kernel<<<grid_size(n * (in / 4), 256), 256, 0, st>>>(E, w.X[l], n, in, w.ST);
+        else ngcf_mix_scalar_kernel<<<grid_size(n * in, 256), 256, 0, st>>>(E, w.X[l], n, in, w.ST);
         DRB_CUDA(cudaGetLastError());
         rc = gemm_nt(dtype, n, out, in, w.ST, 2 * in, W1, in, w.Y1, out, st);
         if (rc == DRB_OK) rc = gemm_nt(dtype, n, out, in, w.ST + in, 2 * in, W2, in, w.Y2, out, st);
         if (rc != DRB_OK) return rc;
-        ngcf_act_kernel<<<ngcf_grid(n * 32, 256), 256, 0, st>>>(w.Y1, w.Y2, b1, b2, n, out, w.Y[l], w.rn[l], w.E[l + 1], w.ALL,
-                                                              q.C, q.off[l + 1], keep, scale);
+        ngcf_act_kernel<<<grid_size(n * 32, 256), 256, 0, st>>>(w.Y1, w.Y2, b1, b2, n, out, w.Y[l], w.rn[l], w.E[l + 1], w.ALL,
+                                                                q.C, q.off[l + 1], keep, scale);
         DRB_CUDA(cudaGetLastError());
         if (keep) keep += (size_t)n * out;
         E = w.E[l + 1];
@@ -368,22 +340,13 @@ extern "C" int drb_ngcf_workspace_init(void *d_ws, int32_t U, int32_t I, const i
     return DRB_OK;
 }
 
-// NGCF.forward: d_out [n, C] = cat(E_0 .. E_L, dim=1)
+// NGCF.forward: d_out [n, C] = cat(E_0 .. E_L, dim=1), with nn.Dropout(mess_dropout) active when d_keep != NULL (:164; the
+// reference's module is always in training mode, rank() included).  d_keep: the masks torch draws, one per layer over its
+// [n, width] output, as bytes, layers concatenated.
 extern "C" int drb_ngcf_forward(const float *d_E0, const float *d_W, void *d_ws, int32_t U, int32_t I, const int32_t *dims,
                                 int32_t L, const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val,
                                 const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg, int32_t tower_dtype,
-                                float *d_out, void *stream)
-{
-    return drb_ngcf_forward_dropout(d_E0, d_W, d_ws, U, I, dims, L, d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, tower_dtype,
-                                    nullptr, 0.f, d_out, stream);
-}
-
-// forward() with nn.Dropout(mess_dropout) active (:164; the reference's module is always in training mode, rank() included).
-// d_keep: the masks torch draws, one per layer over its [n, width] output, as bytes, layers concatenated; NULL = no dropout.
-extern "C" int drb_ngcf_forward_dropout(const float *d_E0, const float *d_W, void *d_ws, int32_t U, int32_t I, const int32_t *dims,
-                                        int32_t L, const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val,
-                                        const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg, int32_t tower_dtype,
-                                        const uint8_t *d_keep, float dropout, float *d_out, void *stream)
+                                const uint8_t *d_keep, float dropout, float *d_out, void *stream)
 {
     NgcfDims q;
     DRB_REQUIRE(d_keep == nullptr || (dropout > 0.f && dropout < 1.f), "ngcf: dropout masks need 0 < mess_dropout < 1");
@@ -391,39 +354,23 @@ extern "C" int drb_ngcf_forward_dropout(const float *d_E0, const float *d_W, voi
     cudaStream_t st = (cudaStream_t)stream;
     NgcfWs w;
     carve_ngcf(d_ws, q, DRB_OPT_SGD, &w);
-    Adj adj;
-    adj.row_ptr = d_row_ptr; adj.col = d_col; adj.val = d_val; adj.seg_row = d_seg_row; adj.seg_ptr = d_seg_ptr; adj.nseg = nseg;
-    adj.n = q.n;
+    const Adj adj{d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, q.n};
     int rc = ngcf_forward(q, w, adj, d_E0, d_W, tower_dtype, st, d_keep, d_keep ? 1.0f / (float)(1.0 - (double)dropout) : 1.f);
     if (rc != DRB_OK) return rc;
     DRB_CUDA(cudaMemcpyAsync(d_out, w.ALL, sizeof(float) * (size_t)q.n * q.C, cudaMemcpyDeviceToDevice, st));
     return DRB_OK;
 }
 
-// n_steps synchronous NGCF + BPR steps (apply != 0) or the loss of one batch (apply == 0).
+// n_steps synchronous NGCF + BPR steps (apply != 0) or the loss of one batch (apply == 0), with the message dropout of :164
+// active when d_keep != NULL (reference default mess_dropout 0.1).  d_keep: per step the masks of the one forward() a step runs
+// (layers concatenated, bytes), steps concatenated.
 extern "C" int drb_ngcf_bpr_train_steps(float *d_E0, float *d_W, void *d_ws, int32_t U, int32_t I, const int32_t *dims, int32_t L,
                                         const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val,
                                         const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg, const int32_t *d_bu,
                                         const int32_t *d_bi, const int32_t *d_bj, int64_t n_triples, int64_t batch,
                                         int64_t first_step, int64_t n_steps, const drb_hyper *h, int64_t adam_step0,
-                                        int32_t apply, int32_t tower_dtype, double *d_step_loss, int32_t sync_and_check,
-                                        int64_t *nan_step, void *stream)
-{
-    return drb_ngcf_bpr_train_steps_dropout(d_E0, d_W, d_ws, U, I, dims, L, d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, d_bu,
-                                            d_bi, d_bj, n_triples, batch, first_step, n_steps, h, adam_step0, apply, tower_dtype,
-                                            nullptr, 0.f, d_step_loss, sync_and_check, nan_step, stream);
-}
-
-// The same with the message dropout of :164 active (reference default mess_dropout 0.1).  d_keep: per step the masks of the one
-// forward() a step runs (layers concatenated, bytes), steps concatenated.
-extern "C" int drb_ngcf_bpr_train_steps_dropout(float *d_E0, float *d_W, void *d_ws, int32_t U, int32_t I, const int32_t *dims,
-                                                int32_t L, const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val,
-                                                const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg,
-                                                const int32_t *d_bu, const int32_t *d_bi, const int32_t *d_bj, int64_t n_triples,
-                                                int64_t batch, int64_t first_step, int64_t n_steps, const drb_hyper *h,
-                                                int64_t adam_step0, int32_t apply, int32_t tower_dtype, const uint8_t *d_keep,
-                                                float dropout, double *d_step_loss, int32_t sync_and_check, int64_t *nan_step,
-                                                void *stream)
+                                        int32_t apply, int32_t tower_dtype, const uint8_t *d_keep, float dropout,
+                                        double *d_step_loss, int32_t sync_and_check, int64_t *nan_step, void *stream)
 {
     NgcfDims q;
     DRB_REQUIRE(d_keep == nullptr || (dropout > 0.f && dropout < 1.f), "ngcf: dropout masks need 0 < mess_dropout < 1");
@@ -438,9 +385,7 @@ extern "C" int drb_ngcf_bpr_train_steps_dropout(float *d_E0, float *d_W, void *d
     cudaStream_t st = (cudaStream_t)stream;
     NgcfWs w;
     carve_ngcf(d_ws, q, h->opt, &w);
-    Adj adj;
-    adj.row_ptr = d_row_ptr; adj.col = d_col; adj.val = d_val; adj.seg_row = d_seg_row; adj.seg_ptr = d_seg_ptr; adj.nseg = nseg;
-    adj.n = q.n;
+    const Adj adj{d_row_ptr, d_col, d_val, d_seg_row, d_seg_ptr, nseg, q.n};
     const long long n = q.n;
     const int F = q.d[0], C = q.C;
     DRB_CUDA(cudaMemsetAsync(w.hdr, 0, sizeof(WsHeader), st));
@@ -452,29 +397,18 @@ extern "C" int drb_ngcf_bpr_train_steps_dropout(float *d_E0, float *d_W, void *d
         int rc = ngcf_forward(q, w, adj, d_E0, d_W, tower_dtype, st, keep, drop_scale);
         if (rc != DRB_OK) return rc;
         // phase 1: scores on the concatenated representation, norms on the ego rows, G = dL / d(representation)
-        StepParams p;
-        p.P = w.ALL; p.Q = w.ALL + (size_t)U * C;
+        StepParams p = split_step(h, U, I, d_bu + base, d_bi + base, d_bj + base, nb, adam_step0 + s, d_step_loss + s);
+        p.P = w.ALL; p.Q = w.ALL + (size_t)U * C; p.F = C;
         p.ws.hdr = w.hdr; p.ws.gP = w.G; p.ws.gQ = w.G + (size_t)U * C; p.ws.cntU = w.cntU; p.ws.cntI = w.cntI;
-        p.ws.mP = p.ws.vP = p.ws.mQ = p.ws.vQ = nullptr;
-        p.ws.gB = p.ws.mB = p.ws.vB = nullptr;
-        p.bu = d_bu + base; p.bi = d_bi + base; p.bj = d_bj + base;
-        p.n = nb; p.batch = nb; p.first_step = 0; p.n_steps = 1;
-        p.U = U; p.I = I; p.F = C; p.tile = 512;
-        p.lr = h->lr; p.reg1 = h->reg_1; p.reg2 = h->reg_2; p.opt = h->opt;
-        p.beta1 = h->beta1; p.beta2 = h->beta2; p.eps = h->eps; p.adam_step0 = adam_step0 + s;
-        p.step_loss = d_step_loss + s;
-        p.apply = apply ? 1 : 0;
-        p.dense_hint = 1;
-        p.Pn = nullptr; p.Qn = nullptr;
         p.reg1 = 0.f; p.reg2 = 0.f;                      // the ego rows are F wide, the score rows C wide: norms come from ngcf_norms_kernel
-        p.gscale = 1.f; p.dense_grad = 1; p.neg_mult = 1.f; p.keep_counts = 0;
-        p.neg_row_ptr = nullptr; p.neg_col = nullptr; p.neg_out = nullptr; p.neg_seed = 0ull; p.loss = DRB_LOSS_BPR;
+        p.dense_grad = 1;
+        p.apply = apply ? 1 : 0;
         p.phases = 1;
         if (apply) DRB_CUDA(cudaMemsetAsync(w.G, 0, sizeof(float) * (size_t)n * C, st));
         rc = launch_steps(p, st, true);                  // resets the header accumulators, then accumulates the BPR sum
         if (rc != DRB_OK) return rc;
         if (h->reg_1 != 0.f || h->reg_2 != 0.f) {
-            ngcf_norms_kernel<<<ngcf_grid(nb * 32, 256), 256, 0, st>>>(d_E0, U, F, p.bu, p.bi, p.bj, nb, w.hdr->acc[0]);
+            ngcf_norms_kernel<<<grid_size(nb * 32, 256), 256, 0, st>>>(d_E0, U, F, p.bu, p.bi, p.bj, nb, w.hdr->acc[0]);
             DRB_CUDA(cudaGetLastError());
         }
         ngcf_finalize_kernel<<<1, 1, 0, st>>>(w.hdr, h->reg_1, h->reg_2, d_step_loss + s, first_step + s);
@@ -489,13 +423,13 @@ extern "C" int drb_ngcf_bpr_train_steps_dropout(float *d_E0, float *d_W, void *d
             float *gW1 = w.gW + q.w_off[l], *gb1 = gW1 + (size_t)in * out, *gW2 = gb1 + out, *gb2 = gW2 + (size_t)in * out;
             const uint8_t *keep_l = keep;
             if (keep_l) for (int k = 0; k < l; ++k) keep_l += (size_t)n * q.d[k + 1];
-            ngcf_act_bwd_kernel<<<ngcf_grid(n * 32, 256), 256, 0, st>>>(w.G, C, q.off[l + 1], dE, w.E[l + 1], w.Y[l], w.rn[l], n, out,
-                                                                      w.dY, keep_l, drop_scale);
+            ngcf_act_bwd_kernel<<<grid_size(n * 32, 256), 256, 0, st>>>(w.G, C, q.off[l + 1], dE, w.E[l + 1], w.Y[l], w.rn[l], n, out,
+                                                                        w.dY, keep_l, drop_scale);
             DRB_CUDA(cudaGetLastError());
             rc = colsum_acc(w.dY, n, out, gb1, st);
             if (rc == DRB_OK) rc = colsum_acc(w.dY, n, out, gb2, st);
-            if (in % 4 == 0) ngcf_mix_kernel<<<ngcf_grid(n * (in / 4), 256), 256, 0, st>>>(El, w.X[l], n, in, w.ST);   // [S | T] again
-            else ngcf_mix_scalar_kernel<<<ngcf_grid(n * in, 256), 256, 0, st>>>(El, w.X[l], n, in, w.ST);
+            if (in % 4 == 0) ngcf_mix_kernel<<<grid_size(n * (in / 4), 256), 256, 0, st>>>(El, w.X[l], n, in, w.ST);   // [S | T] again
+                                                                                           else ngcf_mix_scalar_kernel<<<grid_size(n * in, 256), 256, 0, st>>>(El, w.X[l], n, in, w.ST);
             DRB_CUDA(cudaGetLastError());
             // gW1 [out, in] += dY^T S,  gW2 += dY^T T
             if (rc == DRB_OK) rc = gemm_tn_acc_t(tower_dtype, in, out, (int)n, w.ST, 2 * in, w.dY, out, gW1, in, st);
@@ -506,16 +440,16 @@ extern "C" int drb_ngcf_bpr_train_steps_dropout(float *d_E0, float *d_W, void *d
             if (rc != DRB_OK) return rc;
             float *dEl = (dE == w.dEa) ? w.dEb : w.dEa;
             if (in % 4 == 0)
-                ngcf_mix_bwd_kernel<<<ngcf_grid(n * in / 4, 256), 256, 0, st>>>(w.dS, w.dT, El, w.X[l], n * in / 4, dEl, w.dX);
+                ngcf_mix_bwd_kernel<<<grid_size(n * in / 4, 256), 256, 0, st>>>(w.dS, w.dT, El, w.X[l], n * in / 4, dEl, w.dX);
             else
-                ngcf_mix_bwd_scalar_kernel<<<ngcf_grid(n * in, 256), 256, 0, st>>>(w.dS, w.dT, El, w.X[l], n * in, dEl, w.dX);
+                ngcf_mix_bwd_scalar_kernel<<<grid_size(n * in, 256), 256, 0, st>>>(w.dS, w.dT, El, w.X[l], n * in, dEl, w.dX);
             DRB_CUDA(cudaGetLastError());
             rc = launch_spmm(adj, w.dX, w.AdX, nullptr, in, st);                                       // A_hat symmetric
             if (rc != DRB_OK) return rc;
             if (l > 0) {
-                ngcf_add_kernel<<<ngcf_grid(n * in, 256), 256, 0, st>>>(dEl, w.AdX, nullptr, 0, 0, n, in, dEl);
+                ngcf_add_kernel<<<grid_size(n * in, 256), 256, 0, st>>>(dEl, w.AdX, nullptr, 0, 0, n, in, dEl);
             } else {   // gradient of the ego table: block 0 of G + the chain through layer 0
-                ngcf_add_kernel<<<ngcf_grid(n * in, 256), 256, 0, st>>>(dEl, w.AdX, w.G, C, 0, n, in, w.gE);
+                ngcf_add_kernel<<<grid_size(n * in, 256), 256, 0, st>>>(dEl, w.AdX, w.G, C, 0, n, in, w.gE);
             }
             DRB_CUDA(cudaGetLastError());
             dE = dEl;
@@ -528,13 +462,8 @@ extern "C" int drb_ngcf_bpr_train_steps_dropout(float *d_E0, float *d_W, void *d
         p.step_loss = w.scratch;                           // the real loss was written by ngcf_finalize_kernel
         p.phases = 2;
         rc = launch_steps(p, st, true);
+        if (rc == DRB_OK) rc = dense_update(d_W, w.gW, w.mW, w.vW, q.nW, h, adam_step0 + s, w.hdr, st);
         if (rc != DRB_OK) return rc;
-        const double tt = (double)(adam_step0 + s + 1);
-        const float step_size = (float)((double)h->lr / (1.0 - pow((double)h->beta1, tt)));
-        const float bc2_sqrt = (float)sqrt(1.0 - pow((double)h->beta2, tt));
-        ngcf_update_w_kernel<<<ngcf_grid(q.nW, 256), 256, 0, st>>>(d_W, w.gW, w.mW, w.vW, q.nW, h->lr, h->opt, h->beta1, h->beta2,
-                                                                 h->eps, step_size, bc2_sqrt, w.hdr);
-        DRB_CUDA(cudaGetLastError());
     }
     if (sync_and_check) return check_nan(d_ws, st, nan_step);
     return DRB_OK;

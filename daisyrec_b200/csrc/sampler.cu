@@ -211,13 +211,6 @@ __global__ void explode_pointwise_kernel(const int32_t *__restrict__ coo_u, cons
     }
 }
 
-static int grid_for(long long n, int block)
-{
-    long long b = (n + block - 1) / block, cap = (long long)sm_count() * 16;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
-}
-
 }  // namespace drb
 
 using namespace drb;
@@ -278,7 +271,7 @@ extern "C" int drb_sampler_assemble_mixed(const int64_t *d_row_ptr, const int32_
     DRB_REQUIRE(d_row_ptr && d_js && U > 0 && I > 0 && uniform_num >= 0 && other_num >= 0 && uniform_num + other_num > 0,
                 "sampler_assemble_mixed: bad arguments");
     DRB_REQUIRE((uniform_num == 0 || d_draws) && (other_num == 0 || (d_cdf && d_u01)), "sampler_assemble_mixed: null input");
-    assemble_mixed_kernel<<<grid_for((long long)U * (uniform_num + other_num), 256), 256, 0, (cudaStream_t)stream>>>(
+    assemble_mixed_kernel<<<grid_size((long long)U * (uniform_num + other_num), 256), 256, 0, (cudaStream_t)stream>>>(
         d_row_ptr, d_col, d_draws, d_cdf, d_u01, U, I, uniform_num, other_num, d_js);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
@@ -290,8 +283,8 @@ extern "C" int drb_sampler_explode_pointwise(const int32_t *d_coo_u, const int32
     DRB_REQUIRE(d_coo_u && d_coo_i && d_label && d_rows && nnz >= 0 && G >= 0 && (G == 0 || d_js),
                 "sampler_explode_pointwise: bad arguments");
     if (nnz == 0) return DRB_OK;
-    explode_pointwise_kernel<<<grid_for(nnz * (1 + G), 256), 256, 0, (cudaStream_t)stream>>>(d_coo_u, d_coo_i, d_label,
-                                                                                             nnz, d_js, G, d_rows);
+    explode_pointwise_kernel<<<grid_size(nnz * (1 + G), 256), 256, 0, (cudaStream_t)stream>>>(d_coo_u, d_coo_i, d_label,
+                                                                                              nnz, d_js, G, d_rows);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }
@@ -317,8 +310,8 @@ extern "C" int drb_kth_complement_var(const int64_t *d_row_ptr, const int32_t *d
 {
     DRB_REQUIRE(d_row_ptr && d_offsets && d_draws && d_out && rows >= 0, "kth_complement_var: bad arguments");
     if (rows == 0) return DRB_OK;
-    kth_complement_var_kernel<<<grid_for(rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(d_row_ptr, d_col, d_offsets,
-                                                                                          d_draws, rows, d_out);
+    kth_complement_var_kernel<<<grid_size(rows * 32, 256), 256, 0, (cudaStream_t)stream>>>(d_row_ptr, d_col, d_offsets,
+                                                                                           d_draws, rows, d_out);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }
@@ -329,8 +322,8 @@ extern "C" int drb_sampler_draw_philox(uint64_t seed, uint64_t offset, const int
     DRB_REQUIRE(d_row_ptr && d_draws && d_bad_user && U > 0 && I > 0 && G > 0, "sampler_draw_philox: bad arguments");
     cudaStream_t st = (cudaStream_t)stream;
     DRB_CUDA(cudaMemsetAsync(d_bad_user, 0x7f, sizeof(int32_t), st));
-    draw_philox_kernel<<<grid_for((long long)U * G, 256), 256, 0, st>>>(seed, offset, d_row_ptr, U, I, G, d_draws,
-                                                                       d_bad_user);
+    draw_philox_kernel<<<grid_size((long long)U * G, 256), 256, 0, st>>>(seed, offset, d_row_ptr, U, I, G, d_draws,
+                                                                         d_bad_user);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }
@@ -339,8 +332,8 @@ extern "C" int drb_sampler_kth_complement(const int64_t *d_row_ptr, const int32_
                                           int32_t U, int32_t I, int32_t G, int32_t *d_js, void *stream)
 {
     DRB_REQUIRE(d_row_ptr && d_draws && d_js && U > 0 && I > 0 && G > 0, "sampler_kth_complement: bad arguments");
-    kth_complement_kernel<<<grid_for((long long)U * G, 256), 256, 0, (cudaStream_t)stream>>>(d_row_ptr, d_col, d_draws, U,
-                                                                                             G, d_js);
+    kth_complement_kernel<<<grid_size((long long)U * G, 256), 256, 0, (cudaStream_t)stream>>>(d_row_ptr, d_col, d_draws, U,
+                                                                                              G, d_js);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }
@@ -350,7 +343,7 @@ extern "C" int drb_sampler_explode(const int32_t *d_coo_u, const int32_t *d_coo_
 {
     DRB_REQUIRE(d_coo_u && d_coo_i && d_js && d_triples && nnz >= 0 && G > 0, "sampler_explode: bad arguments");
     if (nnz == 0) return DRB_OK;
-    explode_kernel<<<grid_for(nnz * G, 256), 256, 0, (cudaStream_t)stream>>>(d_coo_u, d_coo_i, nnz, d_js, G, d_triples);
+    explode_kernel<<<grid_size(nnz * G, 256), 256, 0, (cudaStream_t)stream>>>(d_coo_u, d_coo_i, nnz, d_js, G, d_triples);
     DRB_CUDA(cudaGetLastError());
     return DRB_OK;
 }

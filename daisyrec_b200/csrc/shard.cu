@@ -85,13 +85,11 @@ extern "C" int drb_shard_gather_triples(const int32_t *d_triples, const int64_t 
     long long m = (n + batch - 1) / batch;
     DRB_CUDA(cudaMemsetAsync(d_scratch_counts, 0, sizeof(unsigned long long) * (size_t)(m > 0 ? m : 1), st));
     if (n > 0) {
-        long long blocks = (n + 255) / 256, cap = (long long)sm_count() * 16;
-        if (blocks > cap) blocks = cap;
-        shard_count_kernel<<<(int)blocks, 256, 0, st>>>(d_triples, d_perm, n, user_lo, user_hi, batch, d_scratch_counts);
+        const int blocks = grid_size(n, 256);
+        shard_count_kernel<<<blocks, 256, 0, st>>>(d_triples, d_perm, n, user_lo, user_hi, batch, d_scratch_counts);
         shard_scan_kernel<<<1, 1024, 0, st>>>(d_scratch_counts, m, (long long *)d_step_offsets);
-        shard_scatter_kernel<<<(int)blocks, 256, 0, st>>>(d_triples, d_perm, n, user_lo, user_hi, batch,
-                                                          (const long long *)d_step_offsets, d_scratch_counts, d_bu, d_bi,
-                                                          d_bj);
+        shard_scatter_kernel<<<blocks, 256, 0, st>>>(d_triples, d_perm, n, user_lo, user_hi, batch,
+                                                     (const long long *)d_step_offsets, d_scratch_counts, d_bu, d_bi, d_bj);
     } else {
         DRB_CUDA(cudaMemsetAsync(d_step_offsets, 0, sizeof(int64_t), st));
     }

@@ -143,7 +143,7 @@ class NFM(GeneralRecommender):
 
     def _host_keep(self, rows_per_step):
         """The masks nn.Dropout would draw for steps of rows_per_step[k] triples, drawn by torch on the global CPU generator in
-        the reference's order -> uint8 CUDA tensor [step][forward call][site][rows][F] (drb_nfm_bpr_train_steps_dropout)."""
+        the reference's order -> uint8 CUDA tensor [step][forward call][site][rows][F] (drb_nfm_bpr_train_steps)."""
         F, sites, keep = self.factors, 1 + self.num_layers, 1.0 - self.dropout
         parts = []
         for B in rows_per_step:

@@ -304,6 +304,13 @@ def gather_triples(d_triples, d_perm=None):
 
 
 # ------------------------------------------------------------------ training
+def _check_step(rc):
+    """A NaN / infinite loss raises ValueError, as the reference's fit() does; any other failure DrbError."""
+    if rc == L.DRB_ERR_NAN_LOSS:
+        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
+    L.check(rc)
+
+
 class MFWorkspace:
     """Device scratch of the step kernel: gradient accumulators, row counters, optimiser state (Adam m, v; Adagrad /
     RMSprop one table)."""
@@ -334,9 +341,7 @@ def mf_bpr_train_steps(P, Q, ws, bu, bi, bj, batch, first_step, n_steps, hp, ada
     fn = L.lib().drb_mf_bpr_train_steps_det if getattr(ws, "det", False) else L.lib().drb_mf_bpr_train_steps
     rc = fn(_ptr(P), _ptr(Q), _ptr(ws.buf), ws.U, ws.I, ws.F, _ptr(bu), _ptr(bi), _ptr(bj), n, batch, first_step, n_steps,
             C.byref(hp), adam_step0, _ptr(losses), 1 if check else 0, C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return losses[:n_steps]
 
 
@@ -353,9 +358,7 @@ def mf_bpr_train_steps_fused_neg(P, Q, ws, bu, bi, d_row_ptr, d_col, seed, batch
                                                   None if neg_out is None else _ptr(neg_out), bu.numel(), batch, first_step,
                                                   n_steps, C.byref(hp), adam_step0, _ptr(losses), 1 if check else 0,
                                                   C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return losses[:n_steps]
 
 
@@ -380,9 +383,7 @@ def mf_bpr_train_step_host(P, Q, ws, h_bu, h_bi, h_bj, hp, stage, adam_step0=0):
     loss = C.c_double(0.0)
     rc = L.lib().drb_mf_bpr_train_step_host(_ptr(P), _ptr(Q), _ptr(ws.buf), ws.U, ws.I, ws.F, hp_(h_bu), hp_(h_bi),
                                             hp_(h_bj), n, C.byref(hp), adam_step0, _ptr(stage), C.byref(loss), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return loss.value
 
 
@@ -400,9 +401,7 @@ def mf_bpr_train_steps_host(P, Q, ws, h_bu, h_bi, h_bj, batch, n_steps, hp, adam
     rc = L.lib().drb_mf_bpr_train_steps_host(_ptr(P), _ptr(Q), _ptr(ws.buf), ws.U, ws.I, ws.F, h_bu.data_ptr(),
                                              h_bi.data_ptr(), h_bj.data_ptr(), n, batch, n_steps, C.byref(hp), adam_step0,
                                              _ptr(stage), _ptr(d_loss), h_loss.data_ptr(), C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return h_loss[:n_steps]
 
 
@@ -429,9 +428,7 @@ def fm_train_steps(P, Q, bias, ws, bu, bi, bj, batch, first_step, n_steps, hp, a
     rc = L.lib().drb_fm_train_steps(_ptr(P), _ptr(Q), _ptr(bias), _ptr(ws.buf), ws.U, ws.I, ws.F, _ptr(bu), _ptr(bi), _ptr(bj),
                                     bu.numel(), batch, first_step, n_steps, C.byref(hp), adam_step0, 1 if apply else 0,
                                     _ptr(losses), 1 if check else 0, C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return losses[:n_steps]
 
 
@@ -567,9 +564,7 @@ def lgcn_bpr_train_steps(E0, ws, graph, num_layers, bu, bi, bj, batch, first_ste
                                           _ptr(bi), _ptr(bj), bu.numel(), batch, first_step, n_steps, C.byref(hp),
                                           adam_step0, 1 if apply else 0, _ptr(losses), 1 if check else 0,
                                           C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return losses[:n_steps]
 
 
@@ -607,7 +602,7 @@ def ngcf_forward(E0, W, ws, graph, tower_dtype=0, dropout=0.0, keep=None):
         if keep.numel() != ngcf_keep_bytes(ws):
             raise ValueError("keep must hold (user_num + item_num) x sum(hidden widths) bytes")
     out = torch.empty((ws.U + ws.I, sum(ws.dims)), dtype=torch.float32, device=E0.device)
-    L.check(L.lib().drb_ngcf_forward_dropout(_ptr(E0), _ptr(W), _ptr(ws.buf), ws.U, ws.I, _dims_arr(ws.dims), len(ws.dims) - 1,
+    L.check(L.lib().drb_ngcf_forward(_ptr(E0), _ptr(W), _ptr(ws.buf), ws.U, ws.I, _dims_arr(ws.dims), len(ws.dims) - 1,
                                              *graph.args(), tower_dtype, None if keep is None else _ptr(keep),
                                              C.c_float(dropout if keep is not None else 0.0), _ptr(out), _stream()))
     return out
@@ -624,15 +619,13 @@ def ngcf_bpr_train_steps(E0, W, ws, graph, bu, bi, bj, batch, first_step, n_step
             raise ValueError("keep must hold n_steps x (user_num + item_num) x sum(hidden widths) bytes")
     losses = torch.empty(max(1, n_steps), dtype=torch.float64, device=E0.device)
     nan_step = C.c_int64(-1)
-    rc = L.lib().drb_ngcf_bpr_train_steps_dropout(_ptr(E0), _ptr(W), _ptr(ws.buf), ws.U, ws.I, _dims_arr(ws.dims), len(ws.dims) - 1,
+    rc = L.lib().drb_ngcf_bpr_train_steps(_ptr(E0), _ptr(W), _ptr(ws.buf), ws.U, ws.I, _dims_arr(ws.dims), len(ws.dims) - 1,
                                                   *graph.args(), _ptr(bu), _ptr(bi), _ptr(bj), bu.numel(), batch, first_step,
                                                   n_steps, C.byref(hp), adam_step0, 1 if apply else 0, tower_dtype,
                                                   None if keep is None else _ptr(keep),
                                                   C.c_float(dropout if keep is not None else 0.0), _ptr(losses),
                                                   1 if check else 0, C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return losses[:n_steps]
 
 
@@ -659,7 +652,7 @@ class NfmWorkspace:
 def nfm_bpr_train_steps(P, Q, bias, N, Rs, ws, act, bu, bi, bj, batch, first_step, n_steps, hp, adam_step0=0, apply=True,
                         check=True, tower_dtype=0, dropout=0.0, keep=None):
     """keep (with dropout > 0): uint8 CUDA tensor of the masks torch's Dropout modules draw, per step
-    [forward call][site][batch][F] (drb_nfm_bpr_train_steps_dropout)."""
+    [forward call][site][batch][F] (drb_nfm_bpr_train_steps)."""
     for t in (P, Q, bias, N):
         _dev(t, torch.float32, "parameter")
     for t, nm in ((bu, "bu"), (bi, "bi"), (bj, "bj")):
@@ -671,14 +664,12 @@ def nfm_bpr_train_steps(P, Q, bias, N, Rs, ws, act, bu, bi, bj, batch, first_ste
             raise ValueError("keep must hold n_steps x 2 x (1 + num_layers) x batch x factors bytes")
     losses = torch.empty(max(1, n_steps), dtype=torch.float64, device=P.device)
     nan_step = C.c_int64(-1)
-    rc = L.lib().drb_nfm_bpr_train_steps_dropout(
+    rc = L.lib().drb_nfm_bpr_train_steps(
         _ptr(P), _ptr(Q), _ptr(bias), _ptr(N), None if Rs is None or Rs.numel() == 0 else _ptr(Rs), _ptr(ws.buf), ws.U, ws.I, ws.F,
         ws.Ln, ws.bn, act, ws.max_rows, _ptr(bu), _ptr(bi), _ptr(bj), bu.numel(), batch, first_step, n_steps, C.byref(hp), adam_step0,
         1 if apply else 0, tower_dtype, None if keep is None else _ptr(keep), C.c_float(dropout if keep is not None else 0.0),
         _ptr(losses), 1 if check else 0, C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return losses[:n_steps]
 
 
@@ -735,9 +726,7 @@ def neumf_bpr_train_steps(tabs, W, ws, bu, bi, bj, batch, first_step, n_steps, h
                                            tower_dtype, C.c_float(dropout), C.c_uint64(dropout_seed),
                                            None if drop_masks is None else _ptr(drop_masks), mode, _ptr(losses),
                                            1 if check else 0, C.byref(nan_step), _stream())
-    if rc == L.DRB_ERR_NAN_LOSS:
-        raise ValueError("Loss=Nan or Infinity: current settings does not fit the recommender")
-    L.check(rc)
+    _check_step(rc)
     return losses[:n_steps]
 
 

@@ -245,9 +245,9 @@ int drb_fm_predict(const float *d_P, const float *d_Q, const float *d_bias, int3
  * drb_ngcf_forward      NGCF.forward :157-172 -> [(U+I), sum(dims)] = cat(E_0 .. E_L) (what rank / full_rank / predict score
  *                       with: feed its user / item halves to drb_mf_rank, drb_mf_full_rank, drb_mf_predict)
  * drb_ngcf_bpr_train_steps  calc_loss :174-205 + backward + optimizer.step for n_steps batches (apply = 0: loss of one batch).
- * drb_ngcf_forward_dropout / drb_ngcf_bpr_train_steps_dropout  the same with nn.Dropout(mess_dropout) of :164 active (reference
- *    default 0.1; the reference builds the module inside forward(), so it drops at rank() time too): d_keep = the masks torch
- *    draws, one per layer over its [(U+I), width] output, as bytes, layers concatenated (train_steps: steps concatenated).
+ * Both with nn.Dropout(mess_dropout) of :164 active when d_keep != NULL (reference default 0.1; the reference builds the module
+ *    inside forward(), so it drops at rank() time too): d_keep = the masks torch draws, one per layer over its [(U+I), width]
+ *    output, as bytes, layers concatenated (train_steps: steps concatenated).  d_keep = NULL: no dropout.
  * Layer widths: 1..256.  tower_dtype as for NeuMF (0 fp32, 1 bf16 tcgen05 GEMMs). */
 int64_t drb_ngcf_param_count(const int32_t *h_dims, int32_t num_layers);
 size_t drb_ngcf_workspace_bytes(int32_t user_num, int32_t item_num, const int32_t *h_dims, int32_t num_layers, int32_t opt);
@@ -255,25 +255,15 @@ int drb_ngcf_workspace_init(void *d_ws, int32_t user_num, int32_t item_num, cons
                             int32_t opt, void *stream);
 int drb_ngcf_forward(const float *d_E0, const float *d_W, void *d_ws, int32_t user_num, int32_t item_num, const int32_t *h_dims,
                      int32_t num_layers, const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val,
-                     const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg, int32_t tower_dtype, float *d_out,
-                     void *stream);
-int drb_ngcf_forward_dropout(const float *d_E0, const float *d_W, void *d_ws, int32_t user_num, int32_t item_num,
-                             const int32_t *h_dims, int32_t num_layers, const int64_t *d_row_ptr, const int32_t *d_col,
-                             const float *d_val, const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg,
-                             int32_t tower_dtype, const uint8_t *d_keep, float mess_dropout, float *d_out, void *stream);
-int drb_ngcf_bpr_train_steps_dropout(float *d_E0, float *d_W, void *d_ws, int32_t user_num, int32_t item_num,
-                                     const int32_t *h_dims, int32_t num_layers, const int64_t *d_row_ptr, const int32_t *d_col,
-                                     const float *d_val, const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg,
-                                     const int32_t *d_bu, const int32_t *d_bi, const int32_t *d_bj, int64_t n, int64_t batch,
-                                     int64_t first_step, int64_t n_steps, const drb_hyper *hyper, int64_t adam_step0,
-                                     int32_t apply, int32_t tower_dtype, const uint8_t *d_keep, float mess_dropout,
-                                     double *d_step_loss, int32_t sync_and_check, int64_t *nan_step, void *stream);
+                     const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg, int32_t tower_dtype,
+                     const uint8_t *d_keep, float mess_dropout, float *d_out, void *stream);
 int drb_ngcf_bpr_train_steps(float *d_E0, float *d_W, void *d_ws, int32_t user_num, int32_t item_num, const int32_t *h_dims,
                              int32_t num_layers, const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val,
                              const int32_t *d_seg_row, const int64_t *d_seg_ptr, int64_t nseg, const int32_t *d_bu,
                              const int32_t *d_bi, const int32_t *d_bj, int64_t n, int64_t batch, int64_t first_step,
                              int64_t n_steps, const drb_hyper *hyper, int64_t adam_step0, int32_t apply, int32_t tower_dtype,
-                             double *d_step_loss, int32_t sync_and_check, int64_t *nan_step, void *stream);
+                             const uint8_t *d_keep, float mess_dropout, double *d_step_loss, int32_t sync_and_check,
+                             int64_t *nan_step, void *stream);
 
 /* ---- NFM + BPR (daisy/model/NFMRecommender.py:14-209; SURVEY 8(f) rank 4) ------------------------------------------
  * P [U,F], Q [I,F] factor tables; d_bias = packed [u_bias (U), i_bias (I), bias_];
@@ -283,9 +273,9 @@ int drb_ngcf_bpr_train_steps(float *d_E0, float *d_W, void *d_ws, int32_t user_n
  * drb_nfm_bpr_train_steps  calc_loss :125-151 + backward + optimizer.step: the pos and the neg forward are separate calls in the
  *    reference, so every BatchNorm takes the statistics of ITS half of the 2*batch rows and moves its running statistics
  *    twice per step (pos first); apply = 0 evaluates the loss of one batch (the running statistics still move, as under train()).
- * drb_nfm_bpr_train_steps_dropout  the same with the Dropout modules of :67,:88 active (the reference default, assets/nfm.yaml:
- *    dropout 0.5): d_keep holds the masks torch's modules draw, as bytes, per step [forward call: pos, neg][site: FM_layers'
- *    Dropout, then the one behind each activation][batch][factors]; the host draws them on torch's CPU generator in that order
+ *    With d_keep != NULL the Dropout modules of :67,:88 are active (the reference default, assets/nfm.yaml: dropout 0.5):
+ *    d_keep holds the masks torch's modules draw, as bytes, per step [forward call: pos, neg][site: FM_layers' Dropout, then
+ *    the one behind each activation][batch][factors]; the host draws them on torch's CPU generator in that order
  *    (model/NFMRecommender.py), so a step equals the reference's.  d_keep = NULL: no dropout.
  * drb_nfm_scores  forward() under model.eval() (running statistics) for (d_u[k], d_i[k]) pairs: rank / full_rank / predict
  *    (:153-209); feed the scores to drb_topk_from_scores.  max_rows: rows of activation scratch (>= 2 * batch). */
@@ -298,14 +288,8 @@ int drb_nfm_bpr_train_steps(float *d_P, float *d_Q, float *d_bias, float *d_N, f
                             int32_t item_num, int32_t factors, int32_t num_layers, int32_t batch_norm, int32_t act,
                             int64_t max_rows, const int32_t *d_bu, const int32_t *d_bi, const int32_t *d_bj, int64_t n,
                             int64_t batch, int64_t first_step, int64_t n_steps, const drb_hyper *hyper, int64_t adam_step0,
-                            int32_t apply, int32_t tower_dtype, double *d_step_loss, int32_t sync_and_check, int64_t *nan_step,
-                            void *stream);
-int drb_nfm_bpr_train_steps_dropout(float *d_P, float *d_Q, float *d_bias, float *d_N, float *d_Rs, void *d_ws, int32_t user_num,
-                                    int32_t item_num, int32_t factors, int32_t num_layers, int32_t batch_norm, int32_t act,
-                                    int64_t max_rows, const int32_t *d_bu, const int32_t *d_bi, const int32_t *d_bj, int64_t n,
-                                    int64_t batch, int64_t first_step, int64_t n_steps, const drb_hyper *hyper,
-                                    int64_t adam_step0, int32_t apply, int32_t tower_dtype, const uint8_t *d_keep, float dropout,
-                                    double *d_step_loss, int32_t sync_and_check, int64_t *nan_step, void *stream);
+                            int32_t apply, int32_t tower_dtype, const uint8_t *d_keep, float dropout, double *d_step_loss,
+                            int32_t sync_and_check, int64_t *nan_step, void *stream);
 int drb_nfm_scores(const float *d_P, const float *d_Q, const float *d_bias, const float *d_N, const float *d_Rs, void *d_ws,
                    int32_t user_num, int32_t item_num, int32_t factors, int32_t num_layers, int32_t batch_norm, int32_t act,
                    int32_t opt, int64_t max_rows, const int32_t *d_u, const int32_t *d_i, int64_t n, int32_t tower_dtype,
