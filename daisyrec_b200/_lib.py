@@ -143,6 +143,13 @@ SIGNATURES = {
     "drb_sampler_draw_mt19937_mixed": (C.c_int, [vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp, c_i32p]),
     "drb_sampler_assemble_mixed": (C.c_int, [vp, vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, vp, vp]),
     "drb_sampler_explode_pointwise": (C.c_int, [vp, vp, vp, C.c_int64, vp, C.c_int32, vp, vp]),
+    "drb_sgns_positions": (C.c_int, [vp, C.c_int64, vp, C.c_int32, C.c_int32, vp, vp, vp]),
+    "drb_sgns_explode": (C.c_int, [vp, vp, C.c_int64, C.c_int32, vp, vp, vp, vp, vp, vp]),
+    "drb_item2vec_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "drb_item2vec_workspace_init": (C.c_int, [vp, C.c_int32, C.c_int32, C.c_int32, vp]),
+    "drb_item2vec_train_steps": (C.c_int, [vp, vp, C.c_int32, C.c_int32, vp, vp, vp, C.c_int64, C.c_int64, C.c_int64,
+                                           C.c_int64, C.POINTER(Hyper), C.c_int64, C.c_int32, vp, C.c_int32, c_i64p, vp]),
+    "drb_item2vec_user_embed": (C.c_int, [vp, vp, vp, C.c_int32, C.c_int32, vp, vp]),
     "drb_csr_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int64]),
     "drb_csr_build": (C.c_int, [vp, vp, C.c_int64, C.c_int32, C.c_int32, vp, vp, vp, c_i64p, vp]),
     "drb_lgcn_build_adj": (C.c_int, [vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int64, vp, vp, vp, vp]),

@@ -61,7 +61,7 @@ __global__ void index_range_kernel(const T *__restrict__ ids, long long n, int n
 
 }  // namespace drb
 
-extern "C" int drb_version(void) { return 201; }
+extern "C" int drb_version(void) { return 202; }
 
 // nn.Embedding raises IndexError for an id outside its table (torch/nn/functional.py embedding); the kernels index raw
 // tables, so fit() / rank() run this check once per uploaded index array.  h_bad[c] = ids of column c outside [0, h_hi[c]).

@@ -487,10 +487,10 @@ extern "C" int drb_mf_workspace_init(void *d_ws, int32_t U, int32_t I, int32_t F
 namespace drb {
 int fill_params(StepParams &p, float *P, float *Q, void *d_ws, int U, int I, int F, const int32_t *bu, const int32_t *bi,
                 const int32_t *bj, long long n, long long batch, long long first, long long nsteps, const drb_hyper *h,
-                long long adam_step0, double *d_step_loss, int apply, float *d_bias, int det)
+                long long adam_step0, double *d_step_loss, int apply, float *d_bias, int det, int shared)
 {
     DRB_REQUIRE(P && Q && d_ws && bu && bi && bj && h && d_step_loss, "null pointer argument");
-    DRB_REQUIRE(U > 0 && I > 0 && F > 0 && batch > 0 && n >= 0 && first >= 0 && nsteps >= 0, "bad sizes");
+    DRB_REQUIRE((shared ? U == 0 && P == Q && h->loss == DRB_LOSS_CL && !d_bias && !det : U > 0) && I > 0 && F > 0 && batch > 0 && n >= 0 && first >= 0 && nsteps >= 0, "bad sizes");
     DRB_REQUIRE(h->opt >= DRB_OPT_SGD && h->opt <= DRB_OPT_RMSPROP, "unknown optimizer id %d", h->opt);
     DRB_REQUIRE(h->loss >= DRB_LOSS_BPR && h->loss <= DRB_LOSS_SL, "unknown loss id %d", h->loss);
     DRB_REQUIRE((first + nsteps - 1) * batch < n || nsteps == 0 || n == 0, "steps [%lld,%lld) exceed %lld triples", first,
@@ -507,6 +507,10 @@ int fill_params(StepParams &p, float *P, float *Q, void *d_ws, int U, int I, int
     p.step_loss = d_step_loss;
     p.apply = apply;
     p.bias = d_bias;
+    if (shared) {   // both gradient contributions of a triple accumulate into the one table's accumulator
+        p.shared = 1;
+        p.ws.gP = p.ws.gQ;
+    }
     return DRB_OK;
 }
 }  // namespace drb
@@ -742,4 +746,68 @@ extern "C" int drb_mf_bpr_phase(float *d_P, float *d_Q, void *d_ws, int32_t U, i
     p.phases = phase;
     p.dense_hint = 1;
     return launch_steps(p, (cudaStream_t)stream);
+}
+
+// ---- Item2Vec (daisy/model/Item2VecRecommender.py): the point-wise CL step on ONE shared item table, and the user rows
+namespace drb {
+// P[u] = sum of Q[i] over the user's sorted train row, for every user with a train item (:56-60); one warp per user,
+// the row's items summed in order, lanes over the factors
+__global__ void item2vec_user_embed_kernel(const int64_t *__restrict__ row_ptr, const int32_t *__restrict__ col,
+                                           const float *__restrict__ Q, int U, int F, float *__restrict__ P)
+{
+    const int lane = threadIdx.x & 31;
+    const long long nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long u = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; u < U; u += nw) {
+        const long long b = row_ptr[u], e = row_ptr[u + 1];
+        if (b == e) continue;           // not a key of train_ur: the row keeps its initial values
+        for (int f = lane; f < F; f += 32) {
+            float acc = 0.f;
+            for (long long s = b; s < e; ++s) acc += __ldg(Q + (size_t)__ldg(col + s) * F + f);
+            P[(size_t)u * F + f] = acc;
+        }
+    }
+}
+}  // namespace drb
+
+extern "C" size_t drb_item2vec_workspace_bytes(int32_t I, int32_t F, int32_t opt)
+{
+    return carve(nullptr, 0, I, F, opt, nullptr);
+}
+
+extern "C" int drb_item2vec_workspace_init(void *d_ws, int32_t I, int32_t F, int32_t opt, void *stream)
+{
+    DRB_REQUIRE(d_ws != nullptr && I > 0 && F > 0, "item2vec_workspace_init: bad arguments");
+    DRB_CUDA(cudaMemsetAsync(d_ws, 0, carve(nullptr, 0, I, F, opt, nullptr), (cudaStream_t)stream));
+    return DRB_OK;
+}
+
+extern "C" int drb_item2vec_train_steps(float *d_Q, void *d_ws, int32_t I, int32_t F, const int32_t *d_bt, const int32_t *d_bc,
+                                        const int32_t *d_blabel, int64_t n, int64_t batch, int64_t first_step, int64_t n_steps,
+                                        const drb_hyper *hyper, int64_t adam_step0, int32_t apply, double *d_step_loss,
+                                        int32_t sync_and_check, int64_t *nan_step, void *stream)
+{
+    DRB_REQUIRE(hyper && hyper->loss == DRB_LOSS_CL, "item2vec_train_steps: the loss is BCEWithLogitsLoss (DRB_LOSS_CL)");
+    DRB_REQUIRE(hyper->reg_1 == 0.f && hyper->reg_2 == 0.f, "item2vec_train_steps: Item2Vec has no regulariser");
+    StepParams p;
+    int rc = fill_params(p, d_Q, d_Q, d_ws, 0, I, F, d_bt, d_bc, d_blabel, n, batch, first_step, n_steps, hyper, adam_step0,
+                         d_step_loss, apply ? 1 : 0, nullptr, 0, 1);
+    if (rc != DRB_OK) return rc;
+    if (n_steps == 0) return DRB_OK;
+    DRB_REQUIRE(apply || n_steps == 1, "item2vec_train_steps: apply=0 evaluates the loss of ONE batch");
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = launch_steps(p, st);
+    if (rc != DRB_OK) return rc;
+    if (sync_and_check) return check_nan(d_ws, st, nan_step);
+    return DRB_OK;
+}
+
+extern "C" int drb_item2vec_user_embed(const int64_t *d_row_ptr, const int32_t *d_col, const float *d_Q, int32_t U, int32_t F,
+                                       float *d_P, void *stream)
+{
+    DRB_REQUIRE(d_row_ptr && d_col && d_Q && d_P && U >= 0 && F > 0, "item2vec_user_embed: bad arguments");
+    if (U == 0) return DRB_OK;
+    item2vec_user_embed_kernel<<<grid_size((long long)U * 32, 256), 256, 0, (cudaStream_t)stream>>>(d_row_ptr, d_col, d_Q, U,
+                                                                                                   F, d_P);
+    DRB_CUDA(cudaGetLastError());
+    return DRB_OK;
 }

@@ -97,6 +97,18 @@ __global__ void draw_philox_kernel(uint64_t seed, uint64_t offset, const int64_t
     }
 }
 
+// the k-th smallest item missing from the sorted row col[b, e): k + #{s : col[s] - s <= k} (col[s] - s is non-decreasing,
+// so one binary search)
+__device__ __forceinline__ int kth_complement(const int32_t *__restrict__ col, long long b, long long e, int k)
+{
+    long long lo = 0, hi = e - b;  // first s with col[s]-s > k
+    while (lo < hi) {
+        long long mid = (lo + hi) >> 1;
+        if ((long long)__ldg(col + b + mid) - mid <= (long long)k) lo = mid + 1; else hi = mid;
+    }
+    return k + (int)lo;
+}
+
 // js[u,g] = k-th smallest item not in the user's sorted row (k = draws[u,g])
 __global__ void kth_complement_kernel(const int64_t *__restrict__ row_ptr, const int32_t *__restrict__ col,
                                       const int32_t *__restrict__ draws, int U, int G, int32_t *__restrict__ js)
@@ -105,14 +117,7 @@ __global__ void kth_complement_kernel(const int64_t *__restrict__ row_ptr, const
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
          idx += (long long)gridDim.x * blockDim.x) {
         int u = (int)(idx / G);
-        long long b = row_ptr[u], e = row_ptr[u + 1];
-        int k = draws[idx];
-        long long lo = 0, hi = e - b;  // first s with col[s]-s > k
-        while (lo < hi) {
-            long long mid = (lo + hi) >> 1;
-            if ((long long)__ldg(col + b + mid) - mid <= (long long)k) lo = mid + 1; else hi = mid;
-        }
-        js[idx] = k + (int)lo;
+        js[idx] = kth_complement(col, row_ptr[u], row_ptr[u + 1], draws[idx]);
     }
 }
 
@@ -126,15 +131,7 @@ __global__ void kth_complement_var_kernel(const int64_t *__restrict__ row_ptr, c
     long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
     for (long long m = warp; m < rows; m += nwarps) {          // one warp per row
         long long b = row_ptr[m], e = row_ptr[m + 1];
-        for (long long d = offsets[m] + lane; d < offsets[m + 1]; d += 32) {
-            int k = draws[d];
-            long long lo = 0, hi = e - b;
-            while (lo < hi) {
-                long long mid = (lo + hi) >> 1;
-                if ((long long)__ldg(col + b + mid) - mid <= (long long)k) lo = mid + 1; else hi = mid;
-            }
-            out[d] = k + (int)lo;
-        }
+        for (long long d = offsets[m] + lane; d < offsets[m + 1]; d += 32) out[d] = kth_complement(col, b, e, draws[d]);
     }
 }
 
@@ -167,14 +164,7 @@ __global__ void assemble_mixed_kernel(const int64_t *__restrict__ row_ptr, const
          idx += (long long)gridDim.x * blockDim.x) {
         int u = (int)(idx / G), g = (int)(idx - (long long)u * G);
         if (g < un) {
-            long long b = row_ptr[u], e = row_ptr[u + 1];
-            int k = draws[(long long)u * un + g];
-            long long lo = 0, hi = e - b;
-            while (lo < hi) {
-                long long mid = (lo + hi) >> 1;
-                if ((long long)__ldg(col + b + mid) - mid <= (long long)k) lo = mid + 1; else hi = mid;
-            }
-            js[idx] = k + (int)lo;
+            js[idx] = kth_complement(col, row_ptr[u], row_ptr[u + 1], draws[(long long)u * un + g]);
         } else {
             double x = u01[(long long)u * on + (g - un)];
             int lo = 0, hi = I;  // first index with cdf[index] > x
@@ -211,9 +201,99 @@ __global__ void explode_pointwise_kernel(const int32_t *__restrict__ coo_u, cons
     }
 }
 
+// ---------------------------------------------------------------- skip-gram negative sampling (sampler.py:105-160)
+// Positions are the df rows grouped stably by user (users ascending, df order inside a user): su / si [n].  Position p sits
+// at index i of its user's sequence [s, e); its context window is j in [max(i-w, 0), min(i+w, L-1)] without i.
+__device__ __forceinline__ void sgns_segment(const int32_t *__restrict__ su, long long n, long long p, long long &s,
+                                             long long &e)
+{
+    const int u = __ldg(su + p);
+    long long lo = 0, hi = p;           // first position of user u
+    while (lo < hi) {
+        long long mid = (lo + hi) >> 1;
+        if (__ldg(su + mid) < u) lo = mid + 1; else hi = mid;
+    }
+    s = lo;
+    lo = p + 1; hi = n;                 // one past its last position
+    while (lo < hi) {
+        long long mid = (lo + hi) >> 1;
+        if (__ldg(su + mid) <= u) lo = mid + 1; else hi = mid;
+    }
+    e = lo;
+}
+
+// count[p] = number of context items of position p (= its number of negatives); bound[p] = I - deg(user), the size of the
+// complement its negatives are drawn from
+__global__ void sgns_positions_kernel(const int32_t *__restrict__ su, long long n, const int64_t *__restrict__ row_ptr, int I,
+                                      int w, int64_t *__restrict__ count, int64_t *__restrict__ bound)
+{
+    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (long long)gridDim.x * blockDim.x) {
+        long long s, e;
+        sgns_segment(su, n, p, s, e);
+        const long long i = p - s, L = e - s;
+        const long long lo = i - w > 0 ? i - w : 0, hi = i + w < L - 1 ? i + w : L - 1;
+        count[p] = hi - lo;             // hi - lo + 1 window slots minus the target itself
+        const int u = __ldg(su + p);
+        bound[p] = (int64_t)I - (row_ptr[u + 1] - row_ptr[u]);
+    }
+}
+
+// rows[2*off[p] ..] of position p: its c positives [t, seq[j], 1] in ascending j, then its c negatives [t, neg, 0] with
+// neg = the draws[off[p] + k]-th item missing from the user's sorted train row
+__global__ void sgns_explode_kernel(const int32_t *__restrict__ su, const int32_t *__restrict__ si, long long n, int w,
+                                    const int64_t *__restrict__ off, const int64_t *__restrict__ row_ptr,
+                                    const int32_t *__restrict__ col, const int32_t *__restrict__ draws,
+                                    int32_t *__restrict__ rows)
+{
+    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (long long)gridDim.x * blockDim.x) {
+        long long s, e;
+        sgns_segment(su, n, p, s, e);
+        const long long i = p - s, L = e - s;
+        const long long lo = i - w > 0 ? i - w : 0, hi = i + w < L - 1 ? i + w : L - 1;
+        const long long d0 = off[p], c = off[p + 1] - d0;
+        const int t = __ldg(si + p), u = __ldg(su + p);
+        int32_t *r = rows + 6 * d0;
+        for (long long j = lo; j <= hi; ++j) {
+            if (j == i) continue;
+            r[0] = t; r[1] = __ldg(si + s + j); r[2] = 1;
+            r += 3;
+        }
+        const long long rb = row_ptr[u], re = row_ptr[u + 1];
+        for (long long k = 0; k < c; ++k) {
+            r[0] = t; r[1] = kth_complement(col, rb, re, __ldg(draws + d0 + k)); r[2] = 0;
+            r += 3;
+        }
+    }
+}
+
 }  // namespace drb
 
 using namespace drb;
+
+extern "C" int drb_sgns_positions(const int32_t *d_su, int64_t n, const int64_t *d_row_ptr, int32_t item_num,
+                                  int32_t window, int64_t *d_count, int64_t *d_bound, void *stream)
+{
+    DRB_REQUIRE(d_su && d_row_ptr && d_count && d_bound && n >= 0 && item_num > 0 && window >= 0,
+                "sgns_positions: bad arguments");
+    if (n == 0) return DRB_OK;
+    sgns_positions_kernel<<<grid_size(n, 256), 256, 0, (cudaStream_t)stream>>>(d_su, n, d_row_ptr, item_num, window, d_count,
+                                                                               d_bound);
+    DRB_CUDA(cudaGetLastError());
+    return DRB_OK;
+}
+
+extern "C" int drb_sgns_explode(const int32_t *d_su, const int32_t *d_si, int64_t n, int32_t window, const int64_t *d_offsets,
+                                const int64_t *d_row_ptr, const int32_t *d_col, const int32_t *d_draws, int32_t *d_rows,
+                                void *stream)
+{
+    DRB_REQUIRE(d_su && d_si && d_offsets && d_row_ptr && d_col && d_draws && d_rows && n >= 0 && window >= 0,
+                "sgns_explode: bad arguments");
+    if (n == 0) return DRB_OK;
+    sgns_explode_kernel<<<grid_size(n, 256), 256, 0, (cudaStream_t)stream>>>(d_su, d_si, n, window, d_offsets, d_row_ptr,
+                                                                             d_col, d_draws, d_rows);
+    DRB_CUDA(cudaGetLastError());
+    return DRB_OK;
+}
 
 extern "C" int drb_mt19937_seed(uint32_t *st, uint32_t seed)
 {

@@ -100,6 +100,9 @@ struct StepParams {
     // deterministic accumulation: run-to-run bitwise reproducible steps (fixed-point int64 atomics, see Workspace); single GPU,
     // fused persistent launch only
     int det = 0;
+    // Item2Vec (Item2VecRecommender.py:48-52): both rows of a triple come from ONE table.  The launcher passes U = 0, P = Q and
+    // ws.gP = ws.gQ; the kernel then counts the target row in cntI and claims it as an item row.  GEN instantiation only.
+    int shared = 0;
     // multi-GPU persistent mode: step s trains local triples [step_offsets[s], step_offsets[s+1]) (device array; the union
     // of the ranks' ranges is the global batch s).  nullptr = uniform batches of `batch` triples.
     const long long *step_offsets = nullptr;
@@ -130,7 +133,8 @@ inline StepParams split_step(const drb_hyper *h, int U, int I, const int32_t *bu
 
 int fill_params(StepParams &p, float *P, float *Q, void *d_ws, int U, int I, int F, const int32_t *bu, const int32_t *bi,
                 const int32_t *bj, long long n, long long batch, long long first, long long nsteps, const drb_hyper *h,
-                long long adam_step0, double *d_step_loss, int apply, float *d_bias = nullptr, int det = 0);
+                long long adam_step0, double *d_step_loss, int apply, float *d_bias = nullptr, int det = 0,
+                int shared = 0);
 int launch_steps(StepParams &p, cudaStream_t st, bool keep_status = false);
 int check_nan(void *d_ws, cudaStream_t st, int64_t *nan_step);
 

@@ -479,7 +479,8 @@ __device__ __forceinline__ void bpr_steps_body(StepParams &p, XCH &xch)
                             }
                         }
                         if (gl == 0) {
-                            red_add_u32(p.ws.cntU + iu[r], 1u);
+                            if (GEN && p.shared) red_add_u64(p.ws.cntI + iu[r], 1ull);   // the target is an item row too
+                            else red_add_u32(p.ws.cntU + iu[r], 1u);
                             red_add_u64(p.ws.cntI + ii[r], 1ull);
                             if (!pw) red_add_u64(p.ws.cntI + ij[r], 1ull << 32);
                             if (GEN && p.bias != nullptr) {   // d loss / d (u_bias, i_bias, bias_): no regulariser (:76-95)
@@ -613,11 +614,12 @@ __device__ __forceinline__ void bpr_steps_body(StepParams &p, XCH &xch)
                             u = __ldg(p.bu + base + t0 + t);
                             i = __ldg(p.bi + base + t0 + t);
                             j = pw ? i : __ldg(p.bj + base + t0 + t);   // point-wise: that plane holds labels
+                            if (GEN && p.shared) j = u;                  // shared table: the target is claimed as an item row
                         }
                         unsigned cu = 0;
                         unsigned long long ci = 0, cj = 0;
                         if (ok && gl == 0) {
-                            cu = atomicExch(p.ws.cntU + u, 0u);
+                            if (!(GEN && p.shared)) cu = atomicExch(p.ws.cntU + u, 0u);
                             ci = atomicExch(p.ws.cntI + i, 0ull);
                             cj = atomicExch(p.ws.cntI + j, 0ull);
                         }

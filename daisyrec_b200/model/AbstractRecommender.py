@@ -276,11 +276,15 @@ class GeneralRecommender(AbstractRecommender):
             d_triples = self._triples_dev
         if d_triples.is_cuda and getattr(self, '_range_ok', None) != (id(data), stamp):
             # nn.Embedding's IndexError (the kernels index raw tables): one pass over the ids per uploaded array
-            pointwise = str(self.loss_type).upper() in ('CL', 'SL')
-            ops.check_index_range(d_triples, (self.user_num, self.item_num, (1 << 62) if pointwise else self.item_num),
-                                  ('user', 'item', 'label' if pointwise else 'negative item'))
+            ops.check_index_range(d_triples, *self._triple_columns())
             self._range_ok = (id(data), stamp)
         return d_triples
+
+    def _triple_columns(self):
+        """(upper bounds, names) of the loader rows' three columns, for the range check of _device_triples."""
+        pointwise = str(self.loss_type).upper() in ('CL', 'SL')
+        return ((self.user_num, self.item_num, (1 << 62) if pointwise else self.item_num),
+                ('user', 'item', 'label' if pointwise else 'negative item'))
 
     def _fit_epoch_sharded(self, plan, epoch):
         """N > 1: same global batches as the single-GPU run; this rank trains the triples of its users."""

@@ -205,6 +205,28 @@ def sampler_explode_pointwise(d_coo_u, d_coo_i, d_label, d_js):
     return rows
 
 
+def sgns_positions(d_su, d_row_ptr, item_num, window):
+    """Skip-gram positions (users ascending): -> (context counts int64 [n], complement sizes int64 [n]) on the device."""
+    _dev(d_su, torch.int32, "su"); _dev(d_row_ptr, torch.int64, "row_ptr")
+    n = d_su.numel()
+    count = torch.empty(max(n, 1), dtype=torch.int64, device=d_su.device)
+    bound = torch.empty(max(n, 1), dtype=torch.int64, device=d_su.device)
+    L.check(L.lib().drb_sgns_positions(_ptr(d_su), n, _ptr(d_row_ptr), item_num, window, _ptr(count), _ptr(bound), _stream()))
+    return count[:n], bound[:n]
+
+
+def sgns_explode(d_su, d_si, window, d_offsets, d_row_ptr, d_col, d_draws):
+    """-> int32 [2 * offsets[-1], 3] skip-gram rows on the device (positives then negatives of every position)."""
+    _dev(d_su, torch.int32, "su"); _dev(d_si, torch.int32, "si"); _dev(d_offsets, torch.int64, "offsets")
+    _dev(d_row_ptr, torch.int64, "row_ptr"); _dev(d_col, torch.int32, "col"); _dev(d_draws, torch.int32, "draws")
+    n = d_su.numel()
+    T = 2 * int(d_offsets[-1].item())
+    rows = torch.empty((max(T, 1), 3), dtype=torch.int32, device=d_su.device)
+    L.check(L.lib().drb_sgns_explode(_ptr(d_su), _ptr(d_si), n, window, _ptr(d_offsets), _ptr(d_row_ptr), _ptr(d_col),
+                                     _ptr(d_draws), _ptr(rows), _stream()))
+    return rows[:T]
+
+
 # ------------------------------------------------------------------ CSR / adjacency builders
 def csr_build(d_row, d_col, n_rows, n_cols):
     """COO int32 pairs on the device -> (row_ptr int64[n_rows+1], col int32[nnz_unique]) sorted + duplicate-free."""
@@ -455,6 +477,41 @@ def fm_predict(P, Q, bias, u, i):
     L.check(L.lib().drb_fm_predict(_ptr(P), _ptr(Q), _ptr(bias), P.shape[0], Q.shape[0], P.shape[1], _ptr(u), _ptr(i),
                                    u.numel(), _ptr(out), _stream()))
     return out
+
+
+# ------------------------------------------------------------------ Item2Vec
+class Item2VecWorkspace:
+    """Step-kernel scratch of the shared item table: accumulator, row counters and optimiser state of the item rows."""
+
+    def __init__(self, item_num, factors, opt, device):
+        self.I, self.F = item_num, factors
+        self.opt = L.OPT_KIND[opt]
+        self.buf = torch.empty(L.lib().drb_item2vec_workspace_bytes(item_num, factors, self.opt), dtype=torch.uint8,
+                               device=device)
+        L.check(L.lib().drb_item2vec_workspace_init(_ptr(self.buf), item_num, factors, self.opt, _stream()))
+
+
+def item2vec_train_steps(Q, ws, bt, bc, blabel, batch, first_step, n_steps, hp, adam_step0=0, apply=True, check=True):
+    """Steps of BCEWithLogitsLoss(sum) on (target, context, label) planes, both rows from the one table Q -> float64 losses."""
+    _dev(Q, torch.float32, "Q")
+    for t, nm in ((bt, "target"), (bc, "context"), (blabel, "label")):
+        _dev(t, torch.int32, nm)
+    losses = torch.empty(max(n_steps, 1), dtype=torch.float64, device=Q.device)
+    nan_step = C.c_int64(-1)
+    rc = L.lib().drb_item2vec_train_steps(_ptr(Q), _ptr(ws.buf), ws.I, ws.F, _ptr(bt), _ptr(bc), _ptr(blabel), bt.numel(),
+                                          batch, first_step, n_steps, C.byref(hp), adam_step0, 1 if apply else 0,
+                                          _ptr(losses), 1 if check else 0, C.byref(nan_step), _stream())
+    _check_step(rc)
+    return losses[:n_steps]
+
+
+def item2vec_user_embed(d_row_ptr, d_col, Q, P):
+    """P[u] = sum of Q over user u's train CSR row, for every user whose row is not empty (in place)."""
+    _dev(d_row_ptr, torch.int64, "row_ptr"); _dev(d_col, torch.int32, "col")
+    _dev(Q, torch.float32, "Q"); _dev(P, torch.float32, "P")
+    L.check(L.lib().drb_item2vec_user_embed(_ptr(d_row_ptr), _ptr(d_col), _ptr(Q), P.shape[0], P.shape[1], _ptr(P),
+                                            _stream()))
+    return P
 
 
 # ------------------------------------------------------------------ inference

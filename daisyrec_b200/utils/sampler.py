@@ -147,3 +147,52 @@ class BasicNegtiveSampler(AbstractSampler):
             return self._pointwise(torch.from_numpy(coo_u).cuda(), torch.from_numpy(coo_i).cuda(), d_js)
         d_tr = ops.sampler_explode(torch.from_numpy(coo_u).cuda(), torch.from_numpy(coo_i).cuda(), d_js)
         return TripleArray.attach(d_tr.cpu().numpy(), d_tr)
+
+
+class SkipGramNegativeSampler(AbstractSampler):
+    """Skip-gram rows <target, context, label> for Item2Vec (daisy/utils/sampler.py:105-160), built on the device.
+
+    Every df row is a position of its user's sequence (users ascending, df row order inside a user, duplicates kept).  A
+    position contributes its window's context items as positives [target, context, 1] in ascending position, then as many
+    negatives [target, item, 0] drawn uniformly with replacement from the items outside config['train_ur'][user] -- the same
+    numpy MT19937 words np.random.choice would consume, so numpy's global state moves on exactly as in the reference.
+    ``sampling()`` returns the int64 [T, 3] host array with its int32 device twin attached (fit() does not upload it again).
+    """
+
+    def __init__(self, df, config, discard=False):
+        super().__init__(config)
+        self.context_window = int(config['context_window'])
+        self.csr = config.get('train_csr', None)                   # (row_ptr int64, col int32) to skip the dict walk
+        freq = df[self.iid_name].value_counts()
+        prob_discard = 1 - np.sqrt(config['rho'] / freq)           # computed (and 'rho' required) with or without discard
+        if discard:                                                # one uniform per df row, before any negative is drawn
+            rnd_p = np.random.uniform(low=0., high=1., size=len(df))
+            df = df[rnd_p >= df[self.iid_name].map(prob_discard).values]
+        self.users = np.array(df[self.uid_name].values, dtype=np.int32)
+        self.items = np.array(df[self.iid_name].values, dtype=np.int32)
+
+    def sampling(self):
+        ops.require_cuda()
+        n, I, w = len(self.users), self.item_num, self.context_window
+        if self.csr is not None:
+            row_ptr, col = self.csr
+        else:
+            row_ptr, col = csr_from_ur(self.ur, int(self.users.max()) + 1 if n else 0)
+        col = np.ascontiguousarray(col, np.int32)
+        d_row_ptr = torch.from_numpy(np.ascontiguousarray(row_ptr, np.int64)).cuda()
+        d_col = torch.from_numpy(col if len(col) else np.zeros(1, np.int32)).cuda()
+        d_su, order = torch.sort(torch.from_numpy(self.users).cuda(), stable=True)     # groupby(uid): stable, users ascending
+        d_si = torch.from_numpy(self.items).cuda()[order].contiguous()
+        count, bound = ops.sgns_positions(d_su, d_row_ptr, I, w)
+        d_off = torch.zeros(n + 1, dtype=torch.int64, device=d_su.device)
+        torch.cumsum(count, 0, out=d_off[1:])
+        state = ops.mt19937_from_numpy()
+        try:                                                       # host: one np.random.choice(cands, size=c) per position
+            draws = ops.bounded_draws_mt19937(state, bound.cpu().numpy(), d_off.cpu().numpy())
+        finally:
+            ops.mt19937_to_numpy(state)                            # numpy's stream moves on as in the reference
+        d_draws = torch.from_numpy(draws if len(draws) else np.zeros(1, np.int32)).cuda()
+        d_rows = ops.sgns_explode(d_su, d_si, w, d_off, d_row_ptr, d_col, d_draws)
+        if d_rows.shape[0] == 0:
+            return np.array([])                                    # np.array of no rows: float64 (0,)
+        return TripleArray.attach(d_rows.cpu().numpy().astype(np.int64), d_rows)

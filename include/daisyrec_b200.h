@@ -238,6 +238,37 @@ int drb_fm_full_rank(const float *d_P, const float *d_Q, const float *d_bias, in
 int drb_fm_predict(const float *d_P, const float *d_Q, const float *d_bias, int32_t user_num, int32_t item_num,
                    int32_t factors, const int32_t *d_u, const int32_t *d_i, int64_t n, float *d_out, void *stream);
 
+/* ---- Item2Vec (daisy/model/Item2VecRecommender.py; skip-gram sampler daisy/utils/sampler.py:105-160) --------------------
+ * SkipGramNegativeSampler.sampling(): the df rows grouped stably by user (groupby(uid)[iid].agg(list), :158-159) are the
+ * positions; d_su / d_si [n] = their users (ascending) and items.  drb_sgns_positions writes, per position, the number c of
+ * context items of the window (:136-146, = its number of negatives) and the size I - deg(user) of the complement of
+ * config['train_ur'][user] (:132-133) its negatives come from.  The negatives are numpy's np.random.choice(cands, size=c)
+ * (:148): drb_bounded_draws_mt19937 with one row per position replays them on the host.  drb_sgns_explode then writes the
+ * int32 [2 * sum c, 3] rows in the reference's order: per position its c positives [target, seq[j], 1] in ascending j, then
+ * its c negatives [target, k-th item outside the user's sorted CSR row, 0].  d_offsets [n+1] = exclusive scan of the counts
+ * (row block of position p starts at 2 * d_offsets[p]; its draws at d_offsets[p]). */
+int drb_sgns_positions(const int32_t *d_su, int64_t n, const int64_t *d_row_ptr, int32_t item_num, int32_t window,
+                       int64_t *d_count, int64_t *d_bound, void *stream);
+int drb_sgns_explode(const int32_t *d_su, const int32_t *d_si, int64_t n, int32_t window, const int64_t *d_offsets,
+                     const int64_t *d_row_ptr, const int32_t *d_col, const int32_t *d_draws, int32_t *d_rows, void *stream);
+/* Item2Vec.fit's step loop (AbstractRecommender.py:112-128 with Item2Vec.calc_loss :62-69): BCEWithLogitsLoss(sum) of
+ * <shared[target], shared[context]> against the label, both rows read from and both gradients applied to ONE table d_Q
+ * [item_num, factors] (== shared_embedding.weight, dense: every DRB_OPT_* kind moves every row).  The MF step kernel (GEN
+ * instantiation) in shared-table mode: one persistent launch for n_steps steps; a triple whose target equals its context
+ * contributes both gradients to that row.  hyper->loss must be DRB_LOSS_CL and reg_1 = reg_2 = 0; apply=0 evaluates the loss
+ * of one batch (n_steps must be 1).  The workspace covers the item rows only. */
+size_t drb_item2vec_workspace_bytes(int32_t item_num, int32_t factors, int32_t opt);
+int drb_item2vec_workspace_init(void *d_ws, int32_t item_num, int32_t factors, int32_t opt, void *stream);
+int drb_item2vec_train_steps(float *d_Q, void *d_ws, int32_t item_num, int32_t factors, const int32_t *d_bt,
+                             const int32_t *d_bc, const int32_t *d_blabel, int64_t n, int64_t batch, int64_t first_step,
+                             int64_t n_steps, const drb_hyper *hyper, int64_t adam_step0, int32_t apply, double *d_step_loss,
+                             int32_t sync_and_check, int64_t *nan_step, void *stream);
+/* The user rows after training (Item2VecRecommender.py:56-60): d_P[u] = sum of d_Q[i] over the user's sorted train CSR row
+ * (= config['train_ur'][u]); users with an empty row keep their values.  rank / full_rank / predict are drb_mf_* on
+ * (d_P, d_Q). */
+int drb_item2vec_user_embed(const int64_t *d_row_ptr, const int32_t *d_col, const float *d_Q, int32_t user_num,
+                            int32_t factors, float *d_P, void *stream);
+
 /* ---- NGCF + BPR (daisy/model/NGCFRecommender.py:38-252; SURVEY 8(f) rank 4; node_dropout = 0) -------------------------
  * E0: the ego table cat(embed_user, embed_item) [(U+I), dims[0]];  dims[0..L]: embedding size then hidden_size_list;
  * W: flat fp32 block, per BiGNN layer W1 [out,in], b1 [out], W2 [out,in], b2 [out] (linear, interact_transform; :46-47);

@@ -1,6 +1,6 @@
 """Secondary measurements (not the driver's bench): BASELINE configs 3, 4, 5 on one GPU.
 
-    python scripts/bench_models.py lightgcn|neumf|mf-netflix [--batch B] [--steps K]
+    python scripts/bench_models.py lightgcn|neumf|mf-netflix|item2vec [--batch B] [--steps K]
 Prints one JSON line per run: triples/s with CUDA events around K steps after warm-up.
 """
 import argparse
@@ -39,14 +39,110 @@ def batches(U, I, n, dev, d=None):
     return bu, bi, bj
 
 
+def card():
+    """Name and power limit of the card the numbers below come from (read in the same process as the measurement)."""
+    import subprocess
+    try:
+        watts = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i",
+                                str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        watts = "unknown"
+    return {"gpu": torch.cuda.get_device_name(), "power_limit": watts}
+
+
+def bench_item2vec(dev, steps):
+    """Item2Vec at the ml-20m shape: the skip-gram sampler (window 2) stage by stage and end to end, then the shared-table
+    Adam step (F = 100) at B = 1 048 576 and B = 256, and a check of both against the C oracle at a small seeded size."""
+    import time
+    import numpy as np
+    import pandas as pd
+    from daisyrec_b200.utils.sampler import SkipGramNegativeSampler
+    from oracle import item2vec_oracle as orc
+    out = card()
+    U, I, nnz = SHAPES["ml-20m"]
+    F, w = 100, 2
+    d = make_interactions(U, I, nnz, device=dev)
+    df = pd.DataFrame({"user": d["coo_u"].cpu().numpy(), "item": d["coo_i"].cpu().numpy()})
+    cfg = dict(UID_NAME="user", IID_NAME="item", item_num=I, train_ur=None, context_window=w, rho=1e-5,
+               train_csr=(d["row_ptr"].cpu().numpy(), d["col"].cpu().numpy()))
+    sampler = SkipGramNegativeSampler(df, cfg)
+    # stages: device positions + scan, host MT19937 draws, device explode (the rows stay on the device)
+    np.random.seed(1)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    d_su, order = torch.sort(torch.from_numpy(sampler.users).to(dev), stable=True)
+    d_si = torch.from_numpy(sampler.items).to(dev)[order].contiguous()
+    count, bound = ops.sgns_positions(d_su, d["row_ptr"], I, w)
+    d_off = torch.zeros(len(sampler.users) + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(count, 0, out=d_off[1:])
+    h_off, h_bound = d_off.cpu().numpy(), bound.cpu().numpy()
+    t1 = time.perf_counter()
+    st = ops.mt19937_from_numpy()
+    draws = ops.bounded_draws_mt19937(st, h_bound, h_off)
+    t2 = time.perf_counter()
+    d_draws = torch.from_numpy(draws).to(dev)
+    rows = ops.sgns_explode(d_su, d_si, w, d_off, d["row_ptr"], d["col"], d_draws)
+    torch.cuda.synchronize()
+    t3 = time.perf_counter()
+    T = rows.shape[0]
+    del rows, d_draws, draws
+    np.random.seed(1)
+    t4 = time.perf_counter()
+    host_rows = sampler.sampling()                      # the class end to end, int64 host array included
+    t5 = time.perf_counter()
+    assert host_rows.shape[0] == T
+    out["sampler"] = {"shape": "ml-20m", "window": w, "positions": len(sampler.users), "T": T,
+                      "device_ms": round(1e3 * ((t1 - t0) + (t3 - t2)), 2), "host_draw_ms": round(1e3 * (t2 - t1), 2),
+                      "wall_ms": round(1e3 * (t5 - t4), 2)}
+    d_rows = host_rows._drb_device
+    del host_rows
+    # steps: Adam, F = 100; the item table (10.7 MB) and its state stay L2-resident, the index planes stream
+    g = torch.Generator(device=dev); g.manual_seed(5)
+    Q0 = (torch.randn(I, F, device=dev, generator=g) * 0.01).contiguous()
+    hp = ops.hyper(0.001, 0.0, 0.0, "adam", loss="CL")
+    out["step"] = []
+    for B in (1 << 20, 256):
+        k = max(2, steps)
+        n = B * k
+        perm = torch.randint(0, T, (n,), device=dev, generator=g)
+        bt, bc, bl = (d_rows[perm, c].contiguous() for c in range(3))
+        Q = Q0.clone()
+        ws = ops.Item2VecWorkspace(I, F, "adam", dev)
+        ms = timed(lambda: ops.item2vec_train_steps(Q, ws, bt, bc, bl, B, 0, k, hp, check=False), 1, 3) / k
+        bytes_step = (16 * F + 12) * B + 2 * 4 * 4 * I * F      # rows + indices, and theta, g, m, v of every item row in + out
+        out["step"].append({"B": B, "F": F, "opt": "adam", "steps_per_launch": k, "ms_per_step": round(ms, 4),
+                            "samples_per_s": round(B / ms * 1e3), "achieved_GBps": round(bytes_step / ms / 1e6, 1)})
+    # outputs against the C oracle at a small seeded size (3 Adam steps)
+    Is, B = 500, 4096
+    gs = torch.Generator(device=dev); gs.manual_seed(7)
+    trip = torch.stack([torch.randint(0, Is, (3 * B,), device=dev, generator=gs),
+                        torch.randint(0, Is, (3 * B,), device=dev, generator=gs),
+                        torch.randint(0, 2, (3 * B,), device=dev, generator=gs)], 1).to(torch.int32)
+    Qs = (torch.randn(Is, F, device=dev, generator=gs) * 0.1).contiguous()
+    Qo = Qs.cpu().numpy().copy()
+    ws = ops.Item2VecWorkspace(Is, F, "adam", dev)
+    losses = ops.item2vec_train_steps(Qs, ws, *(trip[:, c].contiguous() for c in range(3)), B, 0, 3, hp).cpu().numpy()
+    state, lo = {}, []
+    h = trip.cpu().numpy()
+    for s in range(3):
+        lo.append(orc.item2vec_step(Qo, h[s * B:(s + 1) * B], "adam", 0.001, state, step_count=s + 1))
+    out["oracle_check"] = {"I": Is, "F": F, "B": B, "steps": 3,
+                           "max_rel_loss_diff": float(np.max(np.abs(losses - lo) / np.abs(lo))),
+                           "max_abs_table_diff": float(np.abs(Qs.cpu().numpy() - Qo).max())}
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("what", choices=["lightgcn", "neumf", "mf-netflix", "mf-fit", "mf-fused"])
+    ap.add_argument("what", choices=["lightgcn", "neumf", "mf-netflix", "mf-fit", "mf-fused", "item2vec"])
     ap.add_argument("--batch", type=int, default=0)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--tower", default="fp32", choices=["fp32", "bf16"])
     a = ap.parse_args()
     dev = torch.device("cuda")
+    if a.what == "item2vec":
+        print(json.dumps(bench_item2vec(dev, a.steps)))
+        return
     if a.what == "lightgcn":
         U, I, nnz = SHAPES["amazon-book"]
         F, L = 64, 3
