@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 SO = os.path.join(LIBDIR, "libdaisyrec_b200.so")
-SOURCES = ["capi.cu", "mf_bpr.cu", "sampler.cu", "rank.cu", "shard.cu", "lightgcn.cu", "neumf.cu", "comm.cu", "metrics.cu", "csr.cu", "randperm.cu", "p2p.cu", "ngcf.cu", "nfm.cu"]
+SOURCES = ["capi.cu", "mf_bpr.cu", "sampler.cu", "rank.cu", "shard.cu", "lightgcn.cu", "neumf.cu", "comm.cu", "metrics.cu", "csr.cu", "randperm.cu", "p2p.cu", "ngcf.cu", "nfm.cu", "vae.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--threads", "4"]
 

@@ -150,6 +150,16 @@ SIGNATURES = {
     "drb_item2vec_train_steps": (C.c_int, [vp, vp, C.c_int32, C.c_int32, vp, vp, vp, C.c_int64, C.c_int64, C.c_int64,
                                            C.c_int64, C.POINTER(Hyper), C.c_int64, C.c_int32, vp, C.c_int32, c_i64p, vp]),
     "drb_item2vec_user_embed": (C.c_int, [vp, vp, vp, C.c_int32, C.c_int32, vp, vp]),
+    "drb_vae_param_count": (C.c_int64, [C.c_int32, vp, C.c_int32, C.c_int32]),
+    "drb_vae_workspace_bytes": (C.c_size_t, [C.c_int32, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int64]),
+    "drb_vae_workspace_init": (C.c_int, [vp, C.c_int32, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int64, vp]),
+    "drb_vae_train_steps": (C.c_int, [vp, vp, C.c_int32, vp, C.c_int32, C.c_int32, C.c_int64, vp, vp, vp, C.c_int32, vp,
+                                      C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.POINTER(Hyper), C.c_int64, C.c_int32,
+                                      C.c_int32, C.c_int32, C.c_float, vp, vp, C.c_uint64, C.c_double, C.c_int64, C.c_int64,
+                                      vp, C.c_int32, c_i64p, vp]),
+    "drb_vae_forward": (C.c_int, [vp, vp, C.c_int32, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int64, vp, vp, vp, C.c_int32,
+                                  vp, C.c_int64, C.c_int32, C.c_int32, vp, vp]),
+    "drb_vae_candidate_scores": (C.c_int, [vp, C.c_int32, vp, C.c_int32, C.c_int32, vp, C.c_int64, vp, C.c_int32, vp, vp]),
     "drb_csr_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int64]),
     "drb_csr_build": (C.c_int, [vp, vp, C.c_int64, C.c_int32, C.c_int32, vp, vp, vp, c_i64p, vp]),
     "drb_lgcn_build_adj": (C.c_int, [vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int64, vp, vp, vp, vp]),

@@ -5,3 +5,4 @@ from .LightGCNRecommender import LightGCN  # noqa: F401
 from .NGCFRecommender import NGCF  # noqa: F401
 from .NFMRecommender import NFM  # noqa: F401
 from .Item2VecRecommender import Item2Vec  # noqa: F401
+from .VAECFRecommender import VAECF  # noqa: F401

@@ -740,6 +740,93 @@ def nfm_scores(P, Q, bias, N, Rs, ws, act, u, i, tower_dtype=0):
     return out
 
 
+# ------------------------------------------------------------------ Multi-VAE
+def _hidden_arr(hidden):
+    arr = (C.c_int32 * max(1, len(hidden)))(*[int(h) for h in hidden])
+    return arr, len(hidden)
+
+
+def vae_param_count(item_num, hidden, latent_dim):
+    arr, n = _hidden_arr(hidden)
+    return int(L.lib().drb_vae_param_count(item_num, arr, n, latent_dim))
+
+
+class VaeWorkspace:
+    def __init__(self, item_num, hidden, latent_dim, opt, max_rows, device):
+        self.I, self.hidden, self.lat, self.max_rows = item_num, [int(h) for h in hidden], int(latent_dim), int(max_rows)
+        self.opt = L.OPT_SGD if opt == "sgd" else L.OPT_ADAM
+        self._arr, self.Ln = _hidden_arr(self.hidden)
+        nbytes = L.lib().drb_vae_workspace_bytes(item_num, self._arr, self.Ln, self.lat, self.opt, self.max_rows)
+        if nbytes == 0:
+            raise ValueError("VAECF: item_num > 0, at most 8 positive hidden sizes, latent_dim >= 2 and max_rows >= 1")
+        self.buf = torch.empty(nbytes, dtype=torch.uint8, device=device)
+        L.check(L.lib().drb_vae_workspace_init(_ptr(self.buf), item_num, self._arr, self.Ln, self.lat, self.opt, self.max_rows,
+                                               _stream()))
+
+
+class VaeRatings:
+    """The rating rows as a device CSR: row_ptr int64 [U+1], col int32, val float32 (duplicate-free, no zeros)."""
+
+    def __init__(self, row_ptr, col, val):
+        self.row_ptr = _dev(row_ptr, torch.int64, "row_ptr")
+        self.col = _dev(col, torch.int32, "col") if col.numel() else torch.zeros(1, dtype=torch.int32, device=row_ptr.device)
+        self.val = _dev(val, torch.float32, "val") if val.numel() else torch.zeros(1, dtype=torch.float32, device=row_ptr.device)
+        self.U = row_ptr.numel() - 1
+
+    def args(self):
+        return _ptr(self.row_ptr), _ptr(self.col), _ptr(self.val), self.U
+
+
+def vae_train_steps(N, ws, R, users, batch, first_step, n_steps, hp, adam_step0=0, apply=True, training=True, tower_dtype=0,
+                    dropout=0.0, keep=None, eps=None, seed=0, anneal_cap=0.2, total_anneal_steps=0, update0=0, check=True):
+    """keep: int32 CUDA tensor of bit-packed torch keep-masks (ceil(batch * item_num / 32) words per step) or None (Philox);
+    eps: float32 CUDA tensor [n_steps, batch, latent_dim // 2] or None (Philox).  -> float64 losses [n_steps]."""
+    _dev(N, torch.float32, "N"); _dev(users, torch.int32, "users")
+    if keep is not None:
+        _dev(keep, torch.int32, "keep")
+        if keep.numel() < n_steps * ((batch * ws.I + 31) // 32):
+            raise ValueError("keep too short for n_steps batches")
+    if eps is not None:
+        _dev(eps, torch.float32, "eps")
+        last = min(batch, users.numel() - (first_step + n_steps - 1) * batch)
+        if eps.numel() < ((n_steps - 1) * batch + last) * (ws.lat // 2):
+            raise ValueError("eps too short for n_steps batches")
+    losses = torch.empty(max(1, n_steps), dtype=torch.float64, device=N.device)
+    nan_step = C.c_int64(-1)
+    rc = L.lib().drb_vae_train_steps(_ptr(N), _ptr(ws.buf), ws.I, ws._arr, ws.Ln, ws.lat, ws.max_rows, *R.args(), _ptr(users),
+                                     users.numel(), batch, first_step, n_steps, C.byref(hp), adam_step0, 1 if apply else 0,
+                                     1 if training else 0, tower_dtype, C.c_float(dropout),
+                                     None if keep is None else _ptr(keep), None if eps is None else _ptr(eps),
+                                     C.c_uint64(seed), C.c_double(anneal_cap), int(total_anneal_steps), int(update0),
+                                     _ptr(losses), 1 if check else 0, C.byref(nan_step), _stream())
+    _check_step(rc)
+    return losses[:n_steps]
+
+
+VAE_OUT = {"scores": 0, "hidden": 1, "latent": 2}
+
+
+def vae_forward(N, ws, R, users, what="scores", tower_dtype=0):
+    """eval-mode forward for int32 CUDA user ids: 'scores' [n, item_num], 'hidden' (last decoder hidden) or 'latent'
+    (encoder output: mu, logvar)."""
+    _dev(N, torch.float32, "N"); _dev(users, torch.int32, "users")
+    width = {"scores": ws.I, "hidden": ws.hidden[0] if ws.hidden else ws.lat // 2, "latent": ws.lat}[what]
+    out = torch.empty((users.numel(), width), dtype=torch.float32, device=N.device)
+    L.check(L.lib().drb_vae_forward(_ptr(N), _ptr(ws.buf), ws.I, ws._arr, ws.Ln, ws.lat, ws.opt, ws.max_rows, *R.args(),
+                                    _ptr(users), users.numel(), VAE_OUT[what], tower_dtype, _ptr(out), _stream()))
+    return out
+
+
+def vae_candidate_scores(N, ws, hidden_rows, cands):
+    """decoder output at the candidates only: hidden_rows [n, K] from vae_forward(.., 'hidden'), cands int64 [n, C]."""
+    _dev(hidden_rows, torch.float32, "hidden_rows"); _dev(cands, torch.int64, "cands")
+    n, Cn = cands.shape
+    out = torch.empty((n, Cn), dtype=torch.float32, device=N.device)
+    L.check(L.lib().drb_vae_candidate_scores(_ptr(N), ws.I, ws._arr, ws.Ln, ws.lat, _ptr(hidden_rows), n, _ptr(cands), Cn,
+                                             _ptr(out), _stream()))
+    return out
+
+
 # ------------------------------------------------------------------ NeuMF
 NEUMF_MODE = {"NeuMF": 0, "NeuMF-pre": 0, "GMF": 1, "MLP": 2}       # config['model_name'] (NeuMFRecommender.py:48-50)
 

@@ -15,7 +15,7 @@ def get_dataloader(ds, batch_size, shuffle, num_workers=4):
 
 
 def _bulk(ds):
-    return isinstance(ds, (BasicDataset, CandidatesDataset))
+    return isinstance(ds, (BasicDataset, CandidatesDataset, AEDataset))
 
 
 class BasicDataset(Dataset):
@@ -46,3 +46,18 @@ class CandidatesDataset(Dataset):
     def __getitem__(self, index):
         u, c = self.data[index]
         return torch.tensor(u), torch.tensor(c)
+
+
+class AEDataset(Dataset):
+    """The users (or items) of the train set for the auto-encoder models (daisy/utils/dataset.py:40-58): ``data`` is the
+    1-D array of ``train_set[yield_col].unique()``, in order of first appearance."""
+
+    def __init__(self, train_set, yield_col='user'):
+        super().__init__()
+        self.data = train_set[yield_col].unique()
+
+    def __len__(self):
+        return len(self.data)
+
+    def __getitem__(self, index):
+        return self.data[index]

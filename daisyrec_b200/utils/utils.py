@@ -107,3 +107,38 @@ def build_candidates_set(test_ur, train_ur, config, drop_past_inter=True):
             samples = np.concatenate((picked[lo:hi].astype(np.int64), gts[k]), axis=None)
         test_ucands.append([u, samples])
     return test_u, test_ucands
+
+
+def get_history_matrix(df, config, row='user', use_config_value_name=False):
+    """daisy/utils/utils.py:87-123, vectorised: (history_matrix int64 [row_num, max_len], history_value float32 [row_num,
+    max_len], history_len int64 [row_num]).  A row's entries keep their df order and are padded with (0, 0.0)."""
+    logger = config['logger']
+    assert row in df.columns, f'invalid name {row}: not in columns of history dataframe'
+    uid_name, iid_name = config['UID_NAME'], config['IID_NAME']
+    user_ids, item_ids = df[uid_name].values, df[iid_name].values
+    value_name = config['INTER_NAME'] if use_config_value_name else None
+    user_num, item_num = config['user_num'], config['item_num']
+    values = np.ones(len(df)) if value_name is None else df[value_name].values
+    if row == 'user':
+        row_num, max_col_num = user_num, item_num
+        row_ids, col_ids = user_ids, item_ids
+    else:
+        row_num, max_col_num = item_num, user_num
+        row_ids, col_ids = item_ids, user_ids
+    row_ids = np.asarray(row_ids, dtype=np.int64)
+    history_len = np.bincount(row_ids, minlength=row_num).astype(np.int64) if len(row_ids) else np.zeros(row_num, np.int64)
+    if len(history_len) > row_num:
+        raise IndexError(f'index {len(history_len) - 1} is out of bounds for axis 0 with size {row_num}')
+    col_num = np.max(history_len)
+    if col_num > max_col_num * 0.2:
+        logger.info(f'Max value of {row}\'s history interaction records has reached: {col_num / max_col_num * 100:.4f}% of the total.')
+    order = np.argsort(row_ids, kind='stable')
+    starts = np.zeros(row_num + 1, np.int64)
+    np.cumsum(history_len, out=starts[1:])
+    pos = np.empty(len(row_ids), np.int64)
+    pos[order] = np.arange(len(row_ids), dtype=np.int64) - starts[row_ids[order]]      # rank of each entry inside its row
+    history_matrix = np.zeros((row_num, col_num), dtype=np.int64)
+    history_value = np.zeros((row_num, col_num))
+    history_matrix[row_ids, pos] = np.asarray(col_ids, dtype=np.int64)
+    history_value[row_ids, pos] = values
+    return torch.LongTensor(history_matrix), torch.FloatTensor(history_value), torch.LongTensor(history_len)

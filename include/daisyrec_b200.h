@@ -326,6 +326,42 @@ int drb_nfm_scores(const float *d_P, const float *d_Q, const float *d_bias, cons
                    int32_t opt, int64_t max_rows, const int32_t *d_u, const int32_t *d_i, int64_t n, int32_t tower_dtype,
                    float *d_scores, void *stream);
 
+/* ---- Multi-VAE (daisy/model/VAECFRecommender.py) ------------------------------------------------------------------
+ * Dims: item_num, hidden[L] (mlp_hidden_size, L <= 8), latent_dim (>= 2).  Encoder item_num -> hidden[0..L-1] -> latent_dim,
+ * decoder latent_dim/2 -> hidden[L-1..0] -> item_num, Tanh between the Linears of each side.
+ * d_N: flat fp32 block in module-registration order: encoder.0 weight stored TRANSPOSED [item_num, hidden[0]], its bias, then
+ *    every other Linear as torch lays it out (weight [out, in], bias [out]); each weight and bias is zero-padded to a multiple
+ *    of 4 floats, so all of them start 16-byte aligned (drb_vae_param_count includes the padding).
+ * Ratings: CSR over users (d_row_ptr i64[U+1], d_col i32, d_val f32), duplicate-free, zeros dropped.
+ * drb_vae_train_steps  calc_loss + backward + optimizer.step (SGD / Adam over the whole block) for n_steps batches of d_users
+ *    (a ragged last batch takes the rest); apply = 0 evaluates the loss of one batch.  training != 0: dropout on the normalised
+ *    input and z = eps * exp(0.5 logvar) + mu.  Keep bits: d_keep = torch's keep-mask of each step ([batch, item_num] row-major,
+ *    bit-packed little-endian into 32-bit words, ceil(batch * item_num / 32) words per step), NULL = Philox4x32-10(seed).
+ *    eps: d_eps [n_steps][batch][latent_dim/2], NULL = Philox + Box-Muller.  Step s is update number update0 + s + 1 of the
+ *    KL anneal, min(anneal_cap, update / total_anneal_steps) (anneal_cap when total_anneal_steps <= 0).
+ *    tower_dtype 1 runs the GEMMs with bf16 operands on tcgen05 where their N fits one MMA.
+ * drb_vae_forward  eval mode (no dropout, z = mu) for d_users[0, n): what 0 -> decoder output rows [n, item_num],
+ *    1 -> last decoder hidden rows [n, hidden[0]] (latent_dim/2 when L = 0), 2 -> encoder output rows [n, latent_dim].
+ * drb_vae_candidate_scores  decoder output at candidate ids only: scores[r, c] = <hidden rows[r], W_out[cands[r, c]]> + b_out. */
+int64_t drb_vae_param_count(int32_t item_num, const int32_t *hidden, int32_t num_hidden, int32_t latent_dim);
+size_t drb_vae_workspace_bytes(int32_t item_num, const int32_t *hidden, int32_t num_hidden, int32_t latent_dim, int32_t opt,
+                               int64_t max_rows);
+int drb_vae_workspace_init(void *d_ws, int32_t item_num, const int32_t *hidden, int32_t num_hidden, int32_t latent_dim, int32_t opt,
+                           int64_t max_rows, void *stream);
+int drb_vae_train_steps(float *d_N, void *d_ws, int32_t item_num, const int32_t *hidden, int32_t num_hidden, int32_t latent_dim,
+                        int64_t max_rows, const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val, int32_t user_num,
+                        const int32_t *d_users, int64_t n, int64_t batch, int64_t first_step, int64_t n_steps, const drb_hyper *h,
+                        int64_t adam_step0, int32_t apply, int32_t training, int32_t tower_dtype, float dropout,
+                        const uint32_t *d_keep, const float *d_eps, uint64_t seed, double anneal_cap, int64_t total_anneal_steps,
+                        int64_t update0, double *d_step_loss, int32_t sync_and_check, int64_t *nan_step, void *stream);
+int drb_vae_forward(const float *d_N, void *d_ws, int32_t item_num, const int32_t *hidden, int32_t num_hidden, int32_t latent_dim,
+                    int32_t opt, int64_t max_rows, const int64_t *d_row_ptr, const int32_t *d_col, const float *d_val,
+                    int32_t user_num, const int32_t *d_users, int64_t n, int32_t what, int32_t tower_dtype, float *d_out,
+                    void *stream);
+int drb_vae_candidate_scores(const float *d_N, int32_t item_num, const int32_t *hidden, int32_t num_hidden, int32_t latent_dim,
+                             const float *d_hidden, int64_t n, const int64_t *d_cands, int32_t num_cands, float *d_scores,
+                             void *stream);
+
 /* ---- multi-GPU (one process per GPU; user-sharded P, replicated Q; SURVEY 8(e)) ---------------
  * There is no multi-device path in the reference (single process, AbstractRecommender.py:99-100);
  * these entry points split the synchronous step where the exchange has to happen:

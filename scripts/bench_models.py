@@ -1,6 +1,6 @@
 """Secondary measurements (not the driver's bench): BASELINE configs 3, 4, 5 on one GPU.
 
-    python scripts/bench_models.py lightgcn|neumf|mf-netflix|item2vec [--batch B] [--steps K]
+    python scripts/bench_models.py lightgcn|neumf|mf-netflix|item2vec|vae [--batch B] [--steps K]
 Prints one JSON line per run: triples/s with CUDA events around K steps after warm-up.
 """
 import argparse
@@ -132,9 +132,143 @@ def bench_item2vec(dev, steps):
     return out
 
 
+def _vae_model(U, I, row_ptr, col, dev, **kw):
+    import logging
+    from daisyrec_b200.model.VAECFRecommender import VAECF
+    cfg = dict(gpu="", logger=logging.getLogger("b"), user_num=U, item_num=I, mlp_hidden_size=None, latent_dim=128, dropout=0.5,
+               lr=1e-3, epochs=1, total_anneal_steps=100000, anneal_cap=0.2, optimizer="adam", init_method="default",
+               early_stop=False, topk=50, train_csr=(row_ptr, col), progress=False)
+    cfg.update(kw)
+    return VAECF(cfg)
+
+
+def bench_vae(dev, steps, batch):
+    """Multi-VAE at the ml-20m shape (defaults: mlp_hidden_size [600], latent_dim 128, dropout 0.5, Adam): ms/step and users/s
+    for fp32 / bf16 x torch / philox at B = 256 and one larger B, the per-kernel split (torch.profiler), FLOP and byte counts
+    from shapes, the reference VAECF on CUDA (oracle/_ref) at B = 256, and an fp64-oracle parity check at a small shape."""
+    import time
+    import numpy as np
+    from oracle import vae_oracle as vo
+    out = [dict(card())]
+    U, I, nnz = SHAPES["ml-20m"]
+    d = make_interactions(U, I, nnz, device=dev)
+    row_ptr, col = d["row_ptr"].cpu().numpy(), d["col"].cpu().numpy()
+    deg = np.diff(row_ptr)
+    H, lat = 600, 128
+    nN = ops.vae_param_count(I, [H], lat)
+    g = torch.Generator(); g.manual_seed(11)
+    for B in (256, batch or 2048):
+        K = max(2, steps)
+        users = torch.randperm(U, generator=g)[:B * K].to(torch.int32).to(dev)
+        nnz_b = float(deg[users.cpu().numpy()].mean()) * B
+        wide = 3 * 2.0 * B * I * H                                                     # decoder out, dW_out, d hidden
+        small = 3 * 2.0 * B * (H * lat + (lat // 2) * H)
+        sparse = 2 * 2.0 * nnz_b * H
+        adam_bytes = 32.0 * nN                                                         # W, g, m, v read + written
+        logit_bytes = 4.0 * B * I * 5                                                  # GEMM write, 2 softmax reads, 1 write, 1 GEMM read
+        for td in ("fp32", "bf16"):
+            for eng in ("torch", "philox"):
+                torch.manual_seed(1)
+                m = _vae_model(U, I, row_ptr, col, dev, tower_dtype=td, dropout_engine=eng)
+                m.train()
+                m._begin_fit("adam", B)
+                m._steps(users[:B], B, 1)                                              # warm-up
+                torch.cuda.synchronize()
+                t0 = time.time()
+                losses = m._steps(users, B, K)
+                torch.cuda.synchronize()
+                ms = (time.time() - t0) * 1e3 / K
+                out.append(dict(model="VAECF", shape="ml-20m", batch=B, tower_dtype=td, dropout_engine=eng, ms_per_step=ms,
+                                users_per_s=B / ms * 1e3, loss_last=float(losses[-1]), flop_per_step=wide + small + sparse,
+                                TFLOPs=(wide + small + sparse) / ms / 1e9, adam_and_logit_bytes=adam_bytes + logit_bytes,
+                                GBps=(adam_bytes + logit_bytes) / ms / 1e6, params=nN, nnz_per_step=nnz_b))
+                del m
+                torch.cuda.empty_cache()
+    # per-kernel split of one Philox step at B = 256 per dtype
+    from torch.profiler import profile, ProfilerActivity
+    for td in ("fp32", "bf16"):
+        torch.manual_seed(1)
+        m = _vae_model(U, I, row_ptr, col, dev, tower_dtype=td, dropout_engine="philox")
+        m.train()
+        m._begin_fit("adam", 256)
+        us = torch.randperm(U, generator=g)[:256 * 8].to(torch.int32).to(dev)
+        m._steps(us, 256, 2)
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            m._steps(us, 256, 8)
+            torch.cuda.synchronize()
+        split = {}
+        for e in prof.key_averages():
+            if e.device_type.name == "CUDA" and getattr(e, "device_time_total", 0) > 0:
+                split[e.key[:60]] = round(e.device_time_total / 8 / 1e3, 4)
+        out.append(dict(model="VAECF", batch=256, tower_dtype=td, kernel_ms_per_step=dict(sorted(split.items(), key=lambda kv: -kv[1])[:14])))
+        del m
+    # the reference VAECF on CUDA (installed copy), on the first 4096 users (its padded history lives on the device)
+    try:
+        from oracle import ref_harness as rh
+        rh.use_root(rh.INSTALLED_ROOT)
+        rh.import_reference()
+        from daisy.model.VAECFRecommender import VAECF as RefVAE
+        Ur = 4096
+        L = int(deg[:Ur].max())
+        hid = np.zeros((Ur, L), np.int64)
+        for u in range(Ur):
+            hid[u, :deg[u]] = col[row_ptr[u]:row_ptr[u + 1]]
+        hval = (np.arange(L)[None, :] < deg[:Ur, None]).astype(np.float32)
+        cfg = rh.make_config("multi-vae", user_num=Ur, item_num=I, history_item_id=torch.from_numpy(hid),
+                             history_item_value=torch.from_numpy(hval))
+        cfg["gpu"] = "0"
+        ref = RefVAE(cfg).cuda()
+        opt = ref._build_optimizer(optimizer="adam", lr=1e-3)
+        ref.train()
+
+        def ref_step(b):
+            ref.zero_grad()
+            loss = ref.calc_loss(b)
+            loss.backward()
+            opt.step()
+        ub = [torch.randint(0, Ur, (256,), generator=g) for _ in range(steps + 2)]
+        ref_step(ub[0]); ref_step(ub[1])
+        torch.cuda.synchronize()
+        t0 = time.time()
+        for b in ub[2:]:
+            ref_step(b)
+        torch.cuda.synchronize()
+        ms = (time.time() - t0) * 1e3 / steps
+        out.append(dict(model="reference VAECF (torch, CUDA)", batch=256, ms_per_step=ms, users_per_s=256 / ms * 1e3))
+    except Exception as e:                                  # the installed reference copy is optional
+        out.append(dict(model="reference VAECF (torch, CUDA)", error=repr(e)[:200]))
+    # parity against the fp64 oracle at a small shape (host masks and eps, one Adam step)
+    Us, Is = 64, 500
+    rng = np.random.default_rng(0)
+    hid = rng.integers(0, Is, size=(Us, 30))
+    hval = (rng.random((Us, 30)) < 0.8).astype(np.float32)
+    from daisyrec_b200.model.VAECFRecommender import VAECF
+    import logging
+    torch.manual_seed(3)
+    m = VAECF(dict(gpu="", logger=logging.getLogger("b"), user_num=Us, item_num=Is, mlp_hidden_size=[64], latent_dim=32,
+                   dropout=0.5, lr=1e-3, epochs=1, total_anneal_steps=100, anneal_cap=0.2, optimizer="adam", init_method="default",
+                   early_stop=False, topk=10, history_item_id=torch.from_numpy(hid), history_item_value=torch.from_numpy(hval),
+                   dropout_engine="torch"))
+    N0 = vo.from_device(m.net.cpu().numpy(), Is, [64], 32).astype(np.float64)
+    b = np.arange(32)
+    st = torch.get_rng_state()
+    loss = m.train_step(torch.from_numpy(b))
+    torch.set_rng_state(st)
+    mask = torch.empty(32, Is).bernoulli_(0.5).numpy().astype(np.float64)
+    eps = torch.randn(32, 16).numpy().astype(np.float64)
+    R = vo.rating_matrix(hid, hval, Is)
+    lo, grad = vo.loss_grad(N0, R[b], Is, [64], 32, 0.5, mask, eps, vo.anneal(1, 0.2, 100))
+    Nn = vo.step(N0, grad, "adam", 1e-3, {}, 1)
+    dN = np.abs(vo.from_device(m.net.cpu().numpy(), Is, [64], 32) - Nn)
+    out.append(dict(check="oracle parity, 64 users x 500 items, one Adam step", loss=loss, oracle_loss=lo,
+                    loss_rel=abs(loss - lo) / abs(lo), params_max_abs=float(dN.max()), params_over_1e5=int((dN > 1e-5).sum())))
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("what", choices=["lightgcn", "neumf", "mf-netflix", "mf-fit", "mf-fused", "item2vec"])
+    ap.add_argument("what", choices=["lightgcn", "neumf", "mf-netflix", "mf-fit", "mf-fused", "item2vec", "vae"])
     ap.add_argument("--batch", type=int, default=0)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--tower", default="fp32", choices=["fp32", "bf16"])
@@ -142,6 +276,10 @@ def main():
     dev = torch.device("cuda")
     if a.what == "item2vec":
         print(json.dumps(bench_item2vec(dev, a.steps)))
+        return
+    if a.what == "vae":
+        for line in bench_vae(dev, a.steps, a.batch):
+            print(json.dumps(line))
         return
     if a.what == "lightgcn":
         U, I, nnz = SHAPES["amazon-book"]
