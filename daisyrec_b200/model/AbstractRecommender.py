@@ -80,14 +80,14 @@ def epoch_permutation(n, shuffle, generator=None, seed=None):
     return torch.randperm(n, generator=g)
 
 
-def loader_plan(train_loader):
-    """Decode a DataLoader into (triples ndarray, batch_size, shuffle, drop_last, generator), or None when it is not the
-    plain ``DataLoader(BasicDataset(int[T,3]), batch_size, shuffle)`` of run_examples/test.py:93-94 (then fit() falls back
-    to iterating it batch by batch)."""
+def loader_plan(train_loader, shape_ok=lambda data: data.ndim == 2 and data.shape[1] == 3):
+    """Decode a DataLoader into (rows ndarray, batch_size, shuffle, drop_last, generator), or None when it is not a plain
+    ``DataLoader(dataset, batch_size, shuffle)`` over a dataset whose ``.data`` ndarray passes ``shape_ok`` -- by default
+    the ``BasicDataset(int[T,3])`` of run_examples/test.py:93-94 (then fit() falls back to iterating it batch by batch)."""
     ds = getattr(train_loader, 'dataset', None)
     data = getattr(ds, 'data', None)
     bs = getattr(train_loader, 'batch_size', None)
-    if not isinstance(data, np.ndarray) or data.ndim != 2 or data.shape[1] != 3 or bs is None:
+    if not isinstance(data, np.ndarray) or not shape_ok(data) or bs is None:
         return None
     sampler = getattr(train_loader, 'sampler', None)
     if not isinstance(getattr(train_loader, 'batch_sampler', None), BatchSampler):
@@ -101,6 +101,63 @@ def loader_plan(train_loader):
     if gen is not None:
         return None
     return data, int(bs), shuffle, bool(train_loader.drop_last), train_loader.generator
+
+
+def candidate_rows(test_loader):
+    """Decode a test loader into (users int64 ndarray [n], candidates int64 ndarray [n, C]): the (user, candidates) rows of
+    a CandidatesDataset are read directly, any other iterable of (users, candidates) batches is iterated."""
+    data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
+    if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
+        users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
+        return users, np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
+    us, cs = [], []
+    for b_us, b_c in test_loader:
+        us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
+        cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
+    if not us:
+        return np.zeros(0, np.int64), np.zeros((0, 0), np.int64)
+    return torch.cat(us).numpy(), torch.cat(cs).numpy()
+
+
+def mask_segments(n_rows, batch, first, n_steps, bytes_per_step, cap=64 << 20):
+    """Split steps first .. first+n_steps-1 over n_rows index rows (``batch`` rows a step, the last step may hold fewer)
+    into calls whose host-drawn dropout masks take at most ``cap`` bytes -> (first_step, count, rows) in step order: count
+    steps of ``rows = batch`` rows, or the ragged last step alone (count 1, rows < batch), which gets its own draws."""
+    chunk = max(1, cap // max(1, bytes_per_step))
+    s, end = first, first + n_steps
+    while s < end:
+        k = min(chunk, end - s)
+        full = k if (s + k) * batch <= n_rows else k - 1
+        if full > 0:
+            yield s, full, batch
+        if full < k:
+            yield s + full, 1, n_rows - (s + full) * batch
+        s += k
+
+
+def tower_dtype(config, allowed=('fp32', 'bf16')):
+    """config['tower_dtype'] -> its kernel code: the index in ``allowed`` (0 fp32, 1 bf16, 2 fused)."""
+    td = str(config.get('tower_dtype', 'fp32')).lower()
+    if td not in allowed:
+        names = [f"'{a}'" for a in allowed]
+        raise ValueError(f"tower_dtype must be {', '.join(names[:-1])} or {names[-1]}, got {td!r}")
+    return allowed.index(td)
+
+
+def dropout_engine(config):
+    """config['dropout_engine']: 'auto' | 'torch' (host masks from the global CPU generator) | 'philox' (device masks)."""
+    engine = str(config.get('dropout_engine', 'auto')).lower()
+    if engine not in ('auto', 'torch', 'philox'):
+        raise ValueError(f"dropout_engine must be 'auto', 'torch' or 'philox', got {engine!r}")
+    return engine
+
+
+def dropout_rate(p):
+    """A dropout probability as nn.Dropout takes it (None -> 0.0)."""
+    p = float(p or 0.0)
+    if not 0.0 <= p < 1.0:
+        raise ValueError(f"dropout probability has to be in [0, 1), but got {p}")
+    return p
 
 
 class AbstractRecommender(object):
@@ -184,6 +241,119 @@ class GeneralRecommender(AbstractRecommender):
         import torch.distributed as dist
         self.world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
         self.rank_id = dist.get_rank() if self.world > 1 else 0
+        self._ws, self._hp, self._opt_steps = None, None, 0
+
+    # ------------------------------------------------------------------ state
+    _BUFFERS = ()                               # state_dict() keys that hold statistics, not trained parameters
+
+    def parameters(self):
+        return [t for k, t in self.state_dict().items() if k not in self._BUFFERS]
+
+    def load_state_dict(self, sd):
+        """Copy every state_dict() key from sd (reshaped to the parameter's shape)."""
+        for k, t in self.state_dict().items():
+            t.copy_(torch.as_tensor(sd[k]).reshape(t.shape))
+        self._tables_changed()
+
+    def to(self, device):
+        """The parameters live on self.device from construction on; kept for drivers that call model.to(device)."""
+        return self
+
+    def _tables_changed(self):
+        """Called when the parameters changed: drop whatever was computed from them."""
+
+    # ------------------------------------------------------------------ set-up
+    def _hyper(self, opt):
+        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt)
+
+    def _begin_fit(self, opt):
+        """fit() builds a fresh optimizer (AbstractRecommender.py:105): fresh optimiser state and step count.  Classes whose
+        scratch grows with the batch allocate it in _ensure."""
+        self._hp = self._hyper(opt)
+        self._opt_steps = 0
+        self._fit_opt = opt
+        self._ws = None
+
+    def _ensure(self, rows):
+        """Optimiser state and scratch for a call outside fit() that will hold up to ``rows`` index rows (classes without
+        scratch ignore it): a fresh fit's state the first time."""
+        if self._ws is None:
+            self._begin_fit(self._optimizer_name())
+
+    # ------------------------------------------------------------------ ids (nn.Embedding's IndexError: kernels index raw tables)
+    def _users(self, ids):
+        """Host-checked user ids -> int64 device tensor."""
+        u = torch.as_tensor(ids).reshape(-1).to(torch.int64)
+        if u.numel() and (int(u.min()) < 0 or int(u.max()) >= self.user_num):
+            raise IndexError(f'index out of range in self: user id outside [0, {self.user_num})')
+        return u.to(self.device)
+
+    def _planes(self, cols, dtype=torch.int32):
+        """A batch's id columns -> contiguous device planes of ``dtype``, checked against the bounds of _triple_columns()
+        before any kernel sees them."""
+        planes = [torch.as_tensor(c).to(self.device, dtype).reshape(-1).contiguous() for c in cols]
+        bounds, names = self._triple_columns()
+        ops.check_index_range(torch.stack(planes, 1), bounds[:len(planes)], names[:len(planes)])
+        return planes
+
+    # ------------------------------------------------------------------ reference surface
+    def forward(self, user, item):
+        """Scores of the (user[k], item[k]) pairs for index tensors."""
+        return self._score_pairs(*self._planes((user, item)))
+
+    def __call__(self, *args):
+        return self.forward(*args)
+
+    def train_step(self, batch):
+        """zero_grad + calc_loss + backward + optimizer.step on one batch in train mode (AbstractRecommender.py:119-128)
+        -> loss.item()."""
+        self._check_loss_type()
+        bu, bi, bj = self._planes(batch[:3])
+        self._ensure(2 * bu.numel())
+        was = self.training
+        self.train()
+        try:
+            return float(self._train_steps(bu, bi, bj, max(1, bu.numel()), 0, 1).item())
+        finally:
+            self.train(was)
+
+    def rank(self, test_loader):
+        """-> float32 ndarray [n_test_users, topk] of candidate ids, best first, rows in loader order."""
+        users, cands = candidate_rows(test_loader)
+        if len(users) == 0:
+            return np.zeros((0,), np.float32)
+        users = self._users(users)
+        d_cands = torch.from_numpy(np.ascontiguousarray(cands)).to(self.device)
+        ops.check_index_range(d_cands.reshape(-1, 1), (self.item_num,), ('candidate item',))
+        return self._rank_rows(users, d_cands, min(self.topk, cands.shape[1])).cpu().numpy()
+
+    def full_rank(self, u):
+        """-> int64 ndarray [topk] over every item; no masking of train items."""
+        return self._full_rank_rows(self._users([int(u)]), min(self.topk, self.item_num))[0].cpu().numpy()
+
+    def predict(self, u, i):
+        """-> python float."""
+        users = self._users([int(u)])
+        if not 0 <= int(i) < self.item_num:
+            raise IndexError(f'index out of range in self: item id outside [0, {self.item_num})')
+        return float(self._score_pairs(users, torch.tensor([int(i)], dtype=torch.int32, device=self.device)).item())
+
+    # per-class scoring on checked device ids; the defaults run the MF kernels on _score_tables()
+    def _score_tables(self):
+        """(user table, item table) the MF scoring kernels read."""
+        return self.embed_user.weight, self.embed_item.weight
+
+    def _rank_rows(self, users, cands, k):
+        """users int64 [n], cands int64 [n, C] -> float32 [n, k] candidate ids, best first."""
+        return ops.mf_rank(*self._score_tables(), users, cands, k)
+
+    def _full_rank_rows(self, users, k):
+        """users int64 [n] -> int64 [n, k] item ids, best first."""
+        return ops.mf_full_rank(*self._score_tables(), users, k)
+
+    def _score_pairs(self, u, i):
+        """-> float32 [n] scores of the (u[k], i[k]) pairs."""
+        return ops.mf_predict(*self._score_tables(), u.to(torch.int32), i.to(torch.int32))
 
     def _loader_plan(self, train_loader):
         return loader_plan(train_loader)

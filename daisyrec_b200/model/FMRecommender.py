@@ -10,7 +10,6 @@ and a sweep over the ``U + I + 1`` bias scalars in phase 2.  The biases live in 
     fit -> drb_gather_triples + drb_fm_train_steps     calc_loss -> drb_fm_train_steps(apply=0)
     rank -> drb_fm_rank     full_rank -> drb_fm_full_rank     predict / forward -> drb_fm_predict
 """
-import numpy as np
 import torch
 
 from .. import ops
@@ -51,36 +50,18 @@ class FM(GeneralRecommender):
         self.u_bias = _Table(self.bias[:U].view(U, 1))
         self.i_bias = _Table(self.bias[U:U + I].view(I, 1))
         self.bias_ = self.bias[U + I:]
-        self._ws = None
-        self._opt_steps = 0
 
     # ------------------------------------------------------------------ plumbing
-    def parameters(self):
-        return [self.embed_user.weight, self.embed_item.weight, self.u_bias.weight, self.i_bias.weight, self.bias_]
-
     def state_dict(self):
         return {'embed_user.weight': self.embed_user.weight, 'embed_item.weight': self.embed_item.weight,
                 'u_bias.weight': self.u_bias.weight, 'i_bias.weight': self.i_bias.weight, 'bias_': self.bias_}
 
-    def load_state_dict(self, sd):
-        for k, t in self.state_dict().items():
-            t.copy_(torch.as_tensor(sd[k]).reshape(t.shape))
-
-    def to(self, device):
-        return self
-
-    def _hyper(self, opt=None):
-        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt or self._optimizer_name(), loss=str(self.loss_type).upper())
+    def _hyper(self, opt):
+        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt, loss=str(self.loss_type).upper())
 
     def _begin_fit(self, opt):
-        """fit() builds a fresh optimizer (AbstractRecommender.py:105): fresh optimiser state / step count."""
-        self._hp = self._hyper(opt)
-        self._opt_steps = 0
+        super()._begin_fit(opt)
         self._ws = ops.FMWorkspace(self.user_num, self.item_num, self.factors, opt, self.device)
-
-    def _ensure_ws(self):
-        if self._ws is None:
-            self._begin_fit(self._optimizer_name())
 
     def _train_steps(self, bu, bi, bj, batch, first, n_steps):
         losses = ops.fm_train_steps(self.embed_user.weight, self.embed_item.weight, self.bias, self._ws, bu, bi, bj, batch,
@@ -88,62 +69,21 @@ class FM(GeneralRecommender):
         self._opt_steps += n_steps
         return losses
 
-    # ------------------------------------------------------------------ reference surface
-    def forward(self, user, item):
-        """FMRecommender.py:61-68 for index tensors."""
-        u = torch.as_tensor(user).to(self.device, torch.int32).reshape(-1).contiguous()
-        i = torch.as_tensor(item).to(self.device, torch.int32).reshape(-1).contiguous()
-        return ops.fm_predict(self.embed_user.weight, self.embed_item.weight, self.bias, u, i)
-
-    __call__ = forward
-
+    # ------------------------------------------------------------------ reference surface (FMRecommender.py:61-131)
     def calc_loss(self, batch):
         """FMRecommender.py:70-97: 0-d fp32 loss of one (user, pos, neg) / (user, item, label) batch; no update."""
         self._check_loss_type()
-        self._ensure_ws()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
+        bu, bi, bj = self._planes(batch[:3])
+        self._ensure(0)
         loss = ops.fm_train_steps(self.embed_user.weight, self.embed_item.weight, self.bias, self._ws, bu, bi, bj,
                                   max(1, bu.numel()), 0, 1, self._hp, adam_step0=self._opt_steps, apply=False)
         return loss.to(torch.float32).reshape(())
 
-    def train_step(self, batch):
-        """zero_grad + calc_loss + backward + optimizer.step on one batch (AbstractRecommender.py:119-128) -> loss.item()."""
-        self._check_loss_type()
-        self._ensure_ws()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
-        return float(self._train_steps(bu, bi, bj, max(1, bu.numel()), 0, 1).item())
+    def _rank_rows(self, users, cands, k):
+        return ops.fm_rank(self.embed_user.weight, self.embed_item.weight, self.bias, users, cands, k)
 
-    def predict(self, u, i):
-        """FMRecommender.py:97-101 -> python float."""
-        return float(self.forward([u], [i]).item())
+    def _full_rank_rows(self, users, k):
+        return ops.fm_full_rank(self.embed_user.weight, self.embed_item.weight, self.bias, users, k)
 
-    def rank(self, test_loader):
-        """FMRecommender.py:103-121 -> float32 ndarray [n_test_users, topk], rows in loader order."""
-        data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
-        if len(users) == 0:
-            return np.zeros((0,), np.float32)
-        if users.min() < 0 or users.max() >= self.user_num:
-            raise IndexError('index out of range in self: test user id outside [0, user_num)')
-        d_cands = torch.from_numpy(np.ascontiguousarray(cands)).to(self.device)
-        ops.check_index_range(d_cands.reshape(-1, 1), (self.item_num,), ('candidate item',))
-        k = min(self.topk, cands.shape[1])
-        out = ops.fm_rank(self.embed_user.weight, self.embed_item.weight, self.bias, torch.from_numpy(users).to(self.device),
-                          d_cands, k)
-        return out.cpu().numpy()
-
-    def full_rank(self, u):
-        """FMRecommender.py:123-131 -> int64 ndarray [topk]."""
-        users = torch.tensor([int(u)], dtype=torch.int64, device=self.device)
-        k = min(self.topk, self.item_num)
-        return ops.fm_full_rank(self.embed_user.weight, self.embed_item.weight, self.bias, users, k)[0].cpu().numpy()
+    def _score_pairs(self, u, i):
+        return ops.fm_predict(self.embed_user.weight, self.embed_item.weight, self.bias, u.to(torch.int32), i.to(torch.int32))

@@ -47,35 +47,17 @@ class Item2Vec(GeneralRecommender):
         _INIT[self.initializer](wi)
         self.user_embedding = _Table(wu.to(self.device))
         self.shared_embedding = _Table(wi.to(self.device))
-        self._ws = None
-        self._opt_steps = 0
 
     # ------------------------------------------------------------------ plumbing
-    def parameters(self):
-        return [self.user_embedding.weight, self.shared_embedding.weight]
-
     def state_dict(self):
         return {'user_embedding.weight': self.user_embedding.weight, 'shared_embedding.weight': self.shared_embedding.weight}
 
-    def load_state_dict(self, sd):
-        for k, t in self.state_dict().items():
-            t.copy_(torch.as_tensor(sd[k]).reshape(t.shape))
-
-    def to(self, device):
-        return self
-
-    def _hyper(self, opt=None):
-        return ops.hyper(self.lr, 0.0, 0.0, opt or self._optimizer_name(), loss='CL')
+    def _hyper(self, opt):
+        return ops.hyper(self.lr, 0.0, 0.0, opt, loss='CL')
 
     def _begin_fit(self, opt):
-        """fit() builds a fresh optimizer (AbstractRecommender.py:105): fresh optimiser state / step count."""
-        self._hp = self._hyper(opt)
-        self._opt_steps = 0
+        super()._begin_fit(opt)
         self._ws = ops.Item2VecWorkspace(self.item_num, self.factors, opt, self.device)
-
-    def _ensure_ws(self):
-        if self._ws is None:
-            self._begin_fit(self._optimizer_name())
 
     def _train_steps(self, bu, bi, bj, batch, first, n_steps):
         losses = ops.item2vec_train_steps(self.shared_embedding.weight, self._ws, bu, bi, bj, batch, first, n_steps, self._hp,
@@ -86,11 +68,8 @@ class Item2Vec(GeneralRecommender):
     def _triple_columns(self):
         return (self.item_num, self.item_num, 1 << 62), ('target item', 'context item', 'label')
 
-    def _batch(self, batch):
-        planes = [torch.as_tensor(b).to(self.device, torch.int32).reshape(-1).contiguous() for b in batch[:3]]
-        ops.check_index_range(torch.stack(planes[:2], 1).contiguous(), (self.item_num, self.item_num),
-                              ('target item', 'context item'))
-        return planes
+    def _score_tables(self):
+        return self.user_embedding.weight, self.shared_embedding.weight
 
     # ------------------------------------------------------------------ reference surface
     def fit(self, train_loader):
@@ -109,59 +88,12 @@ class Item2Vec(GeneralRecommender):
 
     def forward(self, target_i, context_j):
         """<shared[target], shared[context]> for index tensors."""
-        t = torch.as_tensor(target_i).to(self.device, torch.int32).reshape(-1).contiguous()
-        c = torch.as_tensor(context_j).to(self.device, torch.int32).reshape(-1).contiguous()
-        return ops.mf_predict(self.shared_embedding.weight, self.shared_embedding.weight, t, c)
-
-    __call__ = forward
+        return ops.mf_predict(self.shared_embedding.weight, self.shared_embedding.weight, *self._planes((target_i, context_j)))
 
     def calc_loss(self, batch):
         """0-d fp32 BCEWithLogitsLoss(sum) of one (target, context, label) batch; no update."""
-        self._ensure_ws()
-        bt, bc, bl = self._batch(batch)
+        bt, bc, bl = self._planes(batch[:3])
+        self._ensure(0)
         loss = ops.item2vec_train_steps(self.shared_embedding.weight, self._ws, bt, bc, bl, max(1, bt.numel()), 0, 1, self._hp,
                                         adam_step0=self._opt_steps, apply=False)
         return loss.to(torch.float32).reshape(())
-
-    def train_step(self, batch):
-        """zero_grad + calc_loss + backward + optimizer.step on one batch (AbstractRecommender.py:119-128) -> loss.item()."""
-        self._ensure_ws()
-        bt, bc, bl = self._batch(batch)
-        return float(self._train_steps(bt, bc, bl, max(1, bt.numel()), 0, 1).item())
-
-    def predict(self, u, i):
-        """(user_embedding[u] * shared_embedding[i]).sum() -> python float."""
-        d_u = torch.tensor([int(u)], dtype=torch.int32, device=self.device)
-        d_i = torch.tensor([int(i)], dtype=torch.int32, device=self.device)
-        return float(ops.mf_predict(self.user_embedding.weight, self.shared_embedding.weight, d_u, d_i).item())
-
-    def rank(self, test_loader):
-        """float32 ndarray [n_test_users, topk], rows in loader order (MF's ranking on (user_embedding, shared_embedding))."""
-        data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
-        if len(users) == 0:
-            return np.zeros((0,), np.float32)
-        if users.min() < 0 or users.max() >= self.user_num:
-            raise IndexError('index out of range in self: test user id outside [0, user_num)')
-        d_cands = torch.from_numpy(np.ascontiguousarray(cands)).to(self.device)
-        ops.check_index_range(d_cands.reshape(-1, 1), (self.item_num,), ('candidate item',))
-        k = min(self.topk, cands.shape[1])
-        out = ops.mf_rank(self.user_embedding.weight, self.shared_embedding.weight, torch.from_numpy(users).to(self.device),
-                          d_cands, k)
-        return out.cpu().numpy()
-
-    def full_rank(self, u):
-        """int64 ndarray [topk] over every item; no masking of train items."""
-        users = torch.tensor([int(u)], dtype=torch.int64, device=self.device)
-        k = min(self.topk, self.item_num)
-        return ops.mf_full_rank(self.user_embedding.weight, self.shared_embedding.weight, users, k)[0].cpu().numpy()

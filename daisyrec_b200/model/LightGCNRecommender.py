@@ -57,35 +57,20 @@ class LightGCN(GeneralRecommender):
         else:
             row_ptr, col, val = ops.lgcn_norm_adj(np.asarray(m.row), np.asarray(m.col), self.user_num, self.item_num)
         self.graph = ops.LgcnGraph(row_ptr, col, val, self.device)
-        self._ws = None
-        self._opt_steps = 0
 
     # ------------------------------------------------------------------ plumbing
-    def parameters(self):
-        return [self.embed_user.weight, self.embed_item.weight]
-
     def state_dict(self):
         return {'embed_user.weight': self.embed_user.weight, 'embed_item.weight': self.embed_item.weight}
 
-    def load_state_dict(self, sd):
-        self.embed_user.weight.copy_(sd['embed_user.weight'])
-        self.embed_item.weight.copy_(sd['embed_item.weight'])
-        self.restore_user_e = self.restore_item_e = None
-
-    def _hyper(self, opt=None):
-        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt or self._optimizer_name())
+    def _tables_changed(self):
+        self.restore_user_e = self.restore_item_e = None             # LightGCNRecommender.py:133-134
 
     def _begin_fit(self, opt):
+        super()._begin_fit(opt)
         self._ws = ops.LgcnWorkspace(self.user_num, self.item_num, self.factors, opt, self.device)
-        self._opt_steps = 0
-        self._hp = self._hyper(opt)
-
-    def _ensure_ws(self):
-        if self._ws is None:
-            self._begin_fit(self._optimizer_name())
 
     def _train_steps(self, bu, bi, bj, batch, first, n_steps):
-        self.restore_user_e = self.restore_item_e = None             # LightGCNRecommender.py:133-134
+        self._tables_changed()
         losses = ops.lgcn_bpr_train_steps(self.E0, self._ws, self.graph, self.num_layers, bu, bi, bj, batch, first,
                                           n_steps, self._hp, adam_step0=self._opt_steps)
         self._opt_steps += n_steps
@@ -94,56 +79,21 @@ class LightGCN(GeneralRecommender):
     # ------------------------------------------------------------------ reference surface
     def forward(self):
         """LightGCNRecommender.py:117-129 -> (user_embedding, item_embedding) after propagation + layer mean."""
-        self._ensure_ws()
+        self._ensure(0)
         Em = ops.lgcn_propagate(self.E0, self._ws, self.graph, self.num_layers)
         return Em[:self.user_num], Em[self.user_num:]
 
     def calc_loss(self, batch):
         self._check_loss_type()
-        self._ensure_ws()
-        self.restore_user_e = self.restore_item_e = None
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
+        bu, bi, bj = self._planes(batch[:3])
+        self._ensure(0)
+        self._tables_changed()
         loss = ops.lgcn_bpr_train_steps(self.E0, self._ws, self.graph, self.num_layers, bu, bi, bj, bu.numel(), 0, 1,
                                         self._hp, apply=False)
         return loss.to(torch.float32).reshape(())
 
-    def train_step(self, batch):
-        self._check_loss_type()
-        self._ensure_ws()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
-        return float(self._train_steps(bu, bi, bj, bu.numel(), 0, 1).item())
-
-    def _cached(self):
+    def _score_tables(self):
+        """The propagated tables (restore_user_e / restore_item_e), recomputed after a step or a load."""
         if self.restore_user_e is None or self.restore_item_e is None:
             self.restore_user_e, self.restore_item_e = self.forward()
         return self.restore_user_e, self.restore_item_e
-
-    def predict(self, u, i):
-        eu, ei = self._cached()
-        uu = torch.tensor([int(u)], dtype=torch.int32, device=self.device)
-        ii = torch.tensor([int(i)], dtype=torch.int32, device=self.device)
-        return float(ops.mf_predict(eu, ei, uu, ii).item())
-
-    def rank(self, test_loader):
-        eu, ei = self._cached()
-        data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
-        k = min(self.topk, cands.shape[1])
-        out = ops.mf_rank(eu, ei, torch.from_numpy(users).to(self.device),
-                          torch.from_numpy(np.ascontiguousarray(cands)).to(self.device), k)
-        return out.cpu().numpy()
-
-    def full_rank(self, u):
-        eu, ei = self._cached()
-        users = torch.tensor([int(u)], dtype=torch.int64, device=self.device)
-        return ops.mf_full_rank(eu, ei, users, min(self.topk, self.item_num))[0].cpu().numpy()

@@ -56,8 +56,6 @@ class MF(GeneralRecommender):
             self._P_full_cpu, self.embed_user, self._bounds, self._trainer = wu, None, None, None
         else:
             self.embed_user = _Table(wu.to(self.device))
-        self._ws = None
-        self._opt_steps = 0
         self._stage = None
         self.step_variant = ops.mf_step_variant(self.factors, self.user_num + self.item_num)   # runs the one-off on-device selection
         # optional B200 key: True = every cross-thread sum of a step in fixed point (bitwise reproducible runs); single GPU
@@ -82,9 +80,6 @@ class MF(GeneralRecommender):
             self._neg_seed = int(torch.empty((), dtype=torch.int64).random_().item()) & ((1 << 63) - 1)
 
     # ------------------------------------------------------------------ plumbing
-    def parameters(self):
-        return [self._full_user_table(), self.embed_item.weight]
-
     def state_dict(self):
         return {'embed_user.weight': self._full_user_table(), 'embed_item.weight': self.embed_item.weight}
 
@@ -97,9 +92,6 @@ class MF(GeneralRecommender):
             pu = pu[lo:hi]
         self.embed_user.weight.copy_(pu)
         self.embed_item.weight.copy_(sd['embed_item.weight'])
-
-    def to(self, device):
-        return self
 
     # ------------------------------------------------------------------ multi-GPU (user-sharded P)
     def _shard(self, bounds):
@@ -141,16 +133,15 @@ class MF(GeneralRecommender):
         pos = torch.arange(lo, hi, device=self.device)
         return allgather_rows(self.embed_user.weight, pos, self.user_num)
 
-    def _hyper(self, opt=None):
-        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt or self._optimizer_name(), loss=str(self.loss_type).upper())
+    def _hyper(self, opt):
+        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt, loss=str(self.loss_type).upper())
 
     def _begin_fit(self, opt):
         """fit() builds a fresh optimizer (AbstractRecommender.py:105): fresh Adam moments / step count."""
         if str(self.loss_type).upper() in ('CL', 'SL') and (self.world > 1 or self.neg_sampling == 'fused'):
             raise NotImplementedError('the point-wise losses (CL / SL) run on one GPU with sampler-made rows; the sharded '
                                       'step and the fused negative sampler cover the pair-wise losses')
-        self._hp = self._hyper(opt)
-        self._opt_steps = 0
+        super()._begin_fit(opt)
         if self.world > 1:
             if self._trainer is not None:
                 self._trainer.close()                              # keeps a private copy of Q; frees the peer buffers
@@ -158,10 +149,6 @@ class MF(GeneralRecommender):
             self._trainer = None                                   # fresh optimiser state per fit()
             return
         self._ws = ops.MFWorkspace(self.user_num, self.item_num, self.factors, opt, self.device, deterministic=self.deterministic)
-
-    def _ensure_ws(self):
-        if self._ws is None:
-            self._begin_fit(self._optimizer_name())
 
     def _train_steps(self, bu, bi, bj, batch, first, n_steps):
         if self.neg_sampling == 'fused':
@@ -191,13 +178,8 @@ class MF(GeneralRecommender):
             self._shard(self._default_bounds())
         return self.gather_user_table()
 
-    def forward(self, user, item):
-        """MFRecommender.py:63-68: pred = (P[user] * Q[item]).sum(-1) for index tensors."""
-        u = torch.as_tensor(user).to(self.device, torch.int32).reshape(-1).contiguous()
-        i = torch.as_tensor(item).to(self.device, torch.int32).reshape(-1).contiguous()
-        return ops.mf_predict(self._full_user_table(), self.embed_item.weight, u, i)
-
-    __call__ = forward
+    def _score_tables(self):
+        return self._full_user_table(), self.embed_item.weight
 
     def calc_loss(self, batch):
         """MFRecommender.py:70-97: 0-d fp32 loss of one (user, pos, neg) -- or, for CL / SL, (user, item, label) --
@@ -206,19 +188,23 @@ class MF(GeneralRecommender):
         if self.world > 1:
             raise NotImplementedError('calc_loss / train_step on single batches are single-GPU entry points; under torchrun '
                                       'use fit(train_loader) (user-sharded global steps)')
-        self._ensure_ws()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
+        bu, bi, bj = self._planes(batch[:3])
+        self._ensure(0)
         loss = ops.mf_bpr_loss(self.embed_user.weight, self.embed_item.weight, self._ws, bu, bi, bj, self._hp)
         return loss.to(torch.float32).reshape(())
 
     def train_step(self, batch):
         """zero_grad + calc_loss + backward + optimizer.step on one HOST batch
-        (AbstractRecommender.py:119-128); returns loss.item()."""
+        (AbstractRecommender.py:119-128); returns loss.item().  The ids are range-checked on the host: the kernel reads
+        them from there."""
         self._check_loss_type()
         if self.world > 1:
             raise NotImplementedError('train_step is a single-GPU entry point; under torchrun use fit(train_loader)')
-        self._ensure_ws()
         hb = [self._host_i32(b) for b in batch[:3]]
+        for h, hi, name in zip(hb, *self._triple_columns()):
+            if len(h) and (int(h.min()) < 0 or int(h.max()) >= hi):
+                raise IndexError(f'index out of range in self: {name} id(s) outside [0, {hi})')
+        self._ensure(0)
         n = len(hb[0])
         if self._stage is None or self._stage.numel() < 3 * ((n + 3) // 4 * 4) + 4:
             self._stage = ops.stage_buffer(n, self.device)
@@ -233,7 +219,7 @@ class MF(GeneralRecommender):
         ``.to(device)`` copies and ``loss.item()`` reads kept, but pipelined (copy of batch s+1 under the
         kernel of batch s).  Returns the per-step losses (CPU float64 tensor)."""
         self._check_loss_type()
-        self._ensure_ws()
+        self._ensure(0)
         n = h_bu.numel()
         if n_steps is None:
             n_steps = (n + batch_size - 1) // batch_size
@@ -242,61 +228,25 @@ class MF(GeneralRecommender):
         self._opt_steps += n_steps
         return losses
 
-    def predict(self, u, i):
-        """MFRecommender.py:99-104 -> python float."""
-        return float(self.forward([u], [i]).item())
-
-    def rank(self, test_loader):
-        """MFRecommender.py:106-123 -> float32 ndarray [n_test_users, topk], rows in loader order."""
-        ds = getattr(test_loader, 'dataset', None)
-        data = getattr(ds, 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:                                                   # any iterable of (us, cands_ids) batches
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
-        if len(users) == 0:
-            return np.zeros((0,), np.float32)
-        k = min(self.topk, cands.shape[1])
-        if users.min() < 0 or users.max() >= self.user_num:
-            raise IndexError('index out of range in self: test user id outside [0, user_num)')
+    def _rank_rows(self, users, cands, k):
         if self.world > 1:
             return self._rank_sharded(users, cands, k)
-        d_cands = torch.from_numpy(np.ascontiguousarray(cands)).to(self.device)
-        ops.check_index_range(d_cands.reshape(-1, 1), (self.item_num,), ('candidate item',))
-        out = ops.mf_rank(self.embed_user.weight, self.embed_item.weight, torch.from_numpy(users).to(self.device), d_cands, k)
-        return out.cpu().numpy()
+        return super()._rank_rows(users, cands, k)
 
     def _rank_sharded(self, users, cands, k):
         """Each rank scores the test users it owns; one all-gather assembles [n_users, k] in loader order."""
         from ..parallel import allgather_rows, owner_of
         if self._bounds is None:
             self._shard(self._default_bounds())
-        mine = np.flatnonzero(owner_of(users, self._bounds) == self.rank_id)
-        lo = int(self._bounds[self.rank_id])
+        mine = torch.from_numpy(np.flatnonzero(owner_of(users.cpu().numpy(), self._bounds) == self.rank_id)).to(self.device)
         if len(mine):
-            loc = ops.mf_rank(self.embed_user.weight, self.embed_item.weight,
-                              torch.from_numpy(users[mine] - lo).to(self.device),
-                              torch.from_numpy(np.ascontiguousarray(cands[mine])).to(self.device), k)
+            loc = ops.mf_rank(self.embed_user.weight, self.embed_item.weight, users[mine] - int(self._bounds[self.rank_id]),
+                              cands[mine], k)
         else:
             loc = torch.zeros((0, k), dtype=torch.float32, device=self.device)
-        out = allgather_rows(loc, torch.from_numpy(mine).to(self.device), len(users))
-        return out.cpu().numpy()
-
-    def full_rank(self, u):
-        """MFRecommender.py:126-133 -> int64 ndarray [topk]; no masking of train items."""
-        users = torch.tensor([int(u)], dtype=torch.int64, device=self.device)
-        k = min(self.topk, self.item_num)
-        return ops.mf_full_rank(self._full_user_table(), self.embed_item.weight, users, k)[0].cpu().numpy()
+        return allgather_rows(loc, mine, len(users))
 
     def full_rank_users(self, users):
         """Batched full_rank (B200 extension): int64 ndarray [len(users), topk]."""
-        users = torch.as_tensor(np.asarray(users, dtype=np.int64)).to(self.device)
-        k = min(self.topk, self.item_num)
-        return ops.mf_full_rank(self._full_user_table(), self.embed_item.weight, users, k).cpu().numpy()
+        users = self._users(np.asarray(users, dtype=np.int64))
+        return self._full_rank_rows(users, min(self.topk, self.item_num)).cpu().numpy()

@@ -17,11 +17,10 @@ Two reference behaviours are NOT mirrored because they are failures, not results
 the reference's own ``backward()`` raise (the in-place ``fm += ...`` of :120 aliases the activation output), and
 ``predict()`` with ``batch_norm`` feeds a 1-D row to BatchNorm1d, which rejects it.  Both work here.
 """
-import numpy as np
 import torch
 
 from .. import ops
-from .AbstractRecommender import GeneralRecommender, _Table, _init_table, _INIT
+from .AbstractRecommender import GeneralRecommender, _Table, _init_table, _INIT, dropout_rate, mask_segments, tower_dtype
 
 
 class NFM(GeneralRecommender):
@@ -33,9 +32,7 @@ class NFM(GeneralRecommender):
         self.act_function = config['act_function']
         self.num_layers = config['num_layers']
         self.batch_norm = bool(config['batch_norm'])
-        self.dropout = float(config['dropout'] or 0.0)
-        if not 0.0 <= self.dropout < 1.0:
-            raise ValueError(f"dropout probability has to be in [0, 1), but got {self.dropout}")
+        self.dropout = dropout_rate(config['dropout'])
         if self.act_function not in ops.NFM_ACT:
             raise NotImplementedError(f"act_function={self.act_function!r}: expected one of {sorted(ops.NFM_ACT)}")
         self.lr = config['lr']
@@ -89,18 +86,12 @@ class NFM(GeneralRecommender):
         for k in range(n_bn):
             run[k * 2 * F + F:(k + 1) * 2 * F] = 1.0                     # running_var starts at 1
         self.running = run.to(self.device)
-        td = str(config.get('tower_dtype', 'fp32')).lower()
-        if td not in ('fp32', 'bf16'):
-            raise ValueError(f"tower_dtype must be 'fp32' or 'bf16', got {td!r}")
-        self._tower_dtype = 1 if td == 'bf16' else 0
+        self._tower_dtype = tower_dtype(config)
         self._act = ops.NFM_ACT[self.act_function]
         self._rows = int(config.get('nfm_scratch_rows', 1 << 16))
-        self._ws = None
-        self._opt_steps = 0
 
     # ------------------------------------------------------------------ plumbing
-    def parameters(self):
-        return [self.embed_user.weight, self.embed_item.weight, self.u_bias.weight, self.i_bias.weight, self.bias_, self.net]
+    _BUFFERS = ('running',)
 
     def state_dict(self):
         return {'embed_user.weight': self.embed_user.weight, 'embed_item.weight': self.embed_item.weight,
@@ -108,38 +99,20 @@ class NFM(GeneralRecommender):
                 'net': self.net, 'running': self.running}
 
     def load_state_dict(self, sd):
+        """Copies the keys present: the other parameters keep their values."""
         for k, t in self.state_dict().items():
             if k in sd:
                 t.copy_(torch.as_tensor(sd[k]).reshape(t.shape))
 
-    def to(self, device):
-        return self
-
-    def _hyper(self, opt=None):
-        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt or self._optimizer_name())
-
-    def _workspace(self, rows, opt, fresh=False):
-        rows = max(int(rows), self._rows, 2)
-        if fresh or self._ws is None or self._ws.max_rows < rows:
-            if not fresh and self._ws is not None:
-                raise RuntimeError('NFM scratch too small; set config["nfm_scratch_rows"] >= 2 * batch_size')
-            self._ws = ops.NfmWorkspace(self.user_num, self.item_num, self.factors, self.num_layers, self.batch_norm, opt, rows,
-                                        self.device)
-        return self._ws
-
-    def _begin_fit(self, opt):
-        self._hp = self._hyper(opt)
-        self._opt_steps = 0
-        self._fit_opt = opt
-        self._ws = None                                              # fresh optimiser state per fit()
-
     def _ensure(self, rows):
-        if getattr(self, '_hp', None) is None or self._ws is None:
-            if getattr(self, '_hp', None) is None:
-                self._begin_fit(self._optimizer_name())
-            self._workspace(rows, self._fit_opt, fresh=True)
+        if self._hp is None:
+            self._begin_fit(self._optimizer_name())
+        rows = max(int(rows), self._rows, 2)
+        if self._ws is None:
+            self._ws = ops.NfmWorkspace(self.user_num, self.item_num, self.factors, self.num_layers, self.batch_norm,
+                                        self._fit_opt, rows, self.device)
         elif self._ws.max_rows < rows:
-            self._workspace(rows, self._fit_opt)
+            raise RuntimeError('NFM scratch too small; set config["nfm_scratch_rows"] >= 2 * batch_size')
 
     def _host_keep(self, rows_per_step):
         """The masks nn.Dropout would draw for steps of rows_per_step[k] triples, drawn by torch on the global CPU generator in
@@ -161,90 +134,40 @@ class NFM(GeneralRecommender):
         args = (self.embed_user.weight, self.embed_item.weight, self.bias, self.net, self.running, self._ws, self._act)
         if not self._dropping():
             return ops.nfm_bpr_train_steps(*args, bu, bi, bj, batch, first, n_steps, self._hp, **kw)
-        n = bu.numel()
-        per_step = 2 * (1 + self.num_layers) * batch * self.factors
-        chunk = max(1, (64 << 20) // per_step)                           # at most 64 MB of masks per call
-        out, s = [], first
-        while s < first + n_steps:
-            k = min(chunk, first + n_steps - s)
-            full = k if (s + k) * batch <= n else k - 1                   # a ragged last batch gets its own masks + call
-            if full > 0:
-                out.append(ops.nfm_bpr_train_steps(*args, bu, bi, bj, batch, s, full, self._hp, dropout=self.dropout,
-                                                   keep=self._host_keep([batch] * full),
-                                                   **dict(kw, adam_step0=self._opt_steps + (s - first))))
-            if full < k:
-                base = (s + full) * batch
-                last = n - base
-                out.append(ops.nfm_bpr_train_steps(*args, bu[base:], bi[base:], bj[base:], last, 0, 1, self._hp, dropout=self.dropout,
-                                                   keep=self._host_keep([last]),
-                                                   **dict(kw, adam_step0=self._opt_steps + (s + full - first))))
-            s += k
+        out = []
+        for s, k, rows in mask_segments(bu.numel(), batch, first, n_steps, 2 * (1 + self.num_layers) * batch * self.factors):
+            lo, s0 = (s * batch, 0) if rows < batch else (0, s)       # a ragged last step runs as a batch of its own
+            out.append(ops.nfm_bpr_train_steps(*args, bu[lo:], bi[lo:], bj[lo:], rows, s0, k, self._hp, dropout=self.dropout,
+                                               keep=self._host_keep([rows] * k),
+                                               **dict(kw, adam_step0=self._opt_steps + (s - first))))
         return torch.cat(out)
 
     def _train_steps(self, bu, bi, bj, batch, first, n_steps):
-        if self._ws is None:
-            self._workspace(2 * batch, self._fit_opt, fresh=True)
+        self._ensure(2 * batch)
         losses = self._steps(bu, bi, bj, batch, first, n_steps)
         self._opt_steps += n_steps
         return losses
 
-    # ------------------------------------------------------------------ reference surface
-    def _scores(self, u, i):
-        self._ensure(2)
-        return ops.nfm_scores(self.embed_user.weight, self.embed_item.weight, self.bias, self.net, self.running, self._ws,
-                              self._act, u, i, self._tower_dtype)
-
-    def forward(self, user, item):
-        """NFMRecommender.py:110-123 in eval mode (running statistics) for index tensors."""
-        u = torch.as_tensor(user).to(self.device, torch.int32).reshape(-1).contiguous()
-        i = torch.as_tensor(item).to(self.device, torch.int32).reshape(-1).contiguous()
-        return self._scores(u, i)
-
-    __call__ = forward
-
+    # ------------------------------------------------------------------ reference surface (eval mode: running statistics)
     def calc_loss(self, batch):
         """NFMRecommender.py:125-151 under train(): 0-d fp32 loss; the BatchNorm running statistics move as they do there."""
         self._check_loss_type()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
+        bu, bi, bj = self._planes(batch[:3])
         self._ensure(2 * bu.numel())
         loss = self._steps(bu, bi, bj, bu.numel(), 0, 1, apply=False)
         return loss.to(torch.float32).reshape(())
 
-    def train_step(self, batch):
-        self._check_loss_type()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
-        self._ensure(2 * bu.numel())
-        was = self.training
-        self.train()                                                 # a training step runs in train mode (dropout on)
-        try:
-            return float(self._train_steps(bu, bi, bj, bu.numel(), 0, 1).item())
-        finally:
-            self.train(was)
+    def _score_pairs(self, u, i):
+        self._ensure(2)
+        return ops.nfm_scores(self.embed_user.weight, self.embed_item.weight, self.bias, self.net, self.running, self._ws,
+                              self._act, u.to(torch.int32), i.to(torch.int32), self._tower_dtype)
 
-    def predict(self, u, i):
-        return float(self.forward([int(u)], [int(i)]).item())
-
-    def rank(self, test_loader):
-        data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
+    def _rank_rows(self, users, cands, k):
         n, C = cands.shape
-        d_cands = torch.from_numpy(np.ascontiguousarray(cands)).to(self.device)
-        u_rep = torch.from_numpy(np.repeat(users, C).astype(np.int32)).to(self.device)
-        scores = self._scores(u_rep, d_cands.reshape(-1).to(torch.int32).contiguous()).view(n, C).contiguous()
-        return ops.topk_from_scores(scores, d_cands, min(self.topk, C)).cpu().numpy()
+        scores = self._score_pairs(users.repeat_interleave(C), cands.reshape(-1)).view(n, C).contiguous()
+        return ops.topk_from_scores(scores, cands, k)
 
-    def full_rank(self, u):
-        items = torch.arange(self.item_num, dtype=torch.int32, device=self.device)
-        users = torch.full((self.item_num,), int(u), dtype=torch.int32, device=self.device)
-        scores = self._scores(users, items).view(1, -1).contiguous()
-        return ops.topk_from_scores(scores, None, min(self.topk, self.item_num))[0].cpu().numpy()
+    def _full_rank_rows(self, users, k):
+        items = torch.arange(self.item_num, dtype=torch.int32, device=self.device).repeat(users.numel())
+        scores = self._score_pairs(users.repeat_interleave(self.item_num), items).view(users.numel(), -1).contiguous()
+        return ops.topk_from_scores(scores, None, k)

@@ -19,7 +19,7 @@ import numpy as np
 import torch
 
 from .. import ops
-from .AbstractRecommender import GeneralRecommender, _Table, _init_table, _INIT
+from .AbstractRecommender import GeneralRecommender, _Table, _init_table, _INIT, dropout_rate, tower_dtype
 
 
 class NGCF(GeneralRecommender):
@@ -41,9 +41,7 @@ class NGCF(GeneralRecommender):
         if float(self.node_dropout or 0.0) != 0.0:
             raise NotImplementedError('NGCF on the B200 path runs with node_dropout = 0 (the reference default; a sparse dropout '
                                       'of the adjacency drawn from the torch RNG)')
-        self.message_dropout = float(self.message_dropout or 0.0)
-        if not 0.0 <= self.message_dropout < 1.0:
-            raise ValueError(f"dropout probability has to be in [0, 1), but got {self.message_dropout}")
+        self.message_dropout = dropout_rate(self.message_dropout)
         self.reg_1 = config['reg_1']
         self.reg_2 = config['reg_2']
         self.loss_type = config['loss_type']
@@ -81,36 +79,18 @@ class NGCF(GeneralRecommender):
         m = self.interaction_matrix
         row_ptr, col, val = ops.lgcn_norm_adj(np.asarray(m.row), np.asarray(m.col), self.user_num, self.item_num)
         self.graph = ops.LgcnGraph(row_ptr, col, val, self.device)
-        td = str(config.get('tower_dtype', 'fp32')).lower()
-        if td not in ('fp32', 'bf16'):
-            raise ValueError(f"tower_dtype must be 'fp32' or 'bf16', got {td!r}")
-        self._tower_dtype = 1 if td == 'bf16' else 0
-        self._ws = None
-        self._opt_steps = 0
+        self._tower_dtype = tower_dtype(config)
 
     # ------------------------------------------------------------------ plumbing
-    def parameters(self):
-        return [self.embed_user.weight, self.embed_item.weight, self.gnn]
-
     def state_dict(self):
         return {'embed_user.weight': self.embed_user.weight, 'embed_item.weight': self.embed_item.weight, 'gnn': self.gnn}
 
-    def load_state_dict(self, sd):
-        for k, t in self.state_dict().items():
-            t.copy_(torch.as_tensor(sd[k]).reshape(t.shape))
-        self.restore_user_e = self.restore_item_e = None
-
-    def _hyper(self, opt=None):
-        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt or self._optimizer_name())
+    def _tables_changed(self):
+        self.restore_user_e = self.restore_item_e = None             # NGCFRecommender.py:175-176
 
     def _begin_fit(self, opt):
+        super()._begin_fit(opt)
         self._ws = ops.NgcfWorkspace(self.user_num, self.item_num, self.hidden_size_list, opt, self.device)
-        self._opt_steps = 0
-        self._hp = self._hyper(opt)
-
-    def _ensure_ws(self):
-        if self._ws is None:
-            self._begin_fit(self._optimizer_name())
 
     def _host_keep(self, n_forwards):
         """The masks nn.Dropout(mess_dropout) draws for n_forwards forward() calls: per call one bernoulli_ per layer over its
@@ -125,7 +105,7 @@ class NGCF(GeneralRecommender):
         return torch.cat(parts).to(self.device)
 
     def _train_steps(self, bu, bi, bj, batch, first, n_steps):
-        self.restore_user_e = self.restore_item_e = None             # NGCFRecommender.py:175-176
+        self._tables_changed()
         kw = dict(tower_dtype=self._tower_dtype, dropout=self.message_dropout)
         if self.message_dropout <= 0.0:
             losses = ops.ngcf_bpr_train_steps(self.E0, self.gnn, self._ws, self.graph, bu, bi, bj, batch, first, n_steps, self._hp,
@@ -144,58 +124,23 @@ class NGCF(GeneralRecommender):
     # ------------------------------------------------------------------ reference surface
     def forward(self):
         """NGCFRecommender.py:157-172 -> (user_all_embeddings, item_all_embeddings): the concatenated layer outputs."""
-        self._ensure_ws()
+        self._ensure(0)
         rep = ops.ngcf_forward(self.E0, self.gnn, self._ws, self.graph, self._tower_dtype, dropout=self.message_dropout,
                                keep=self._host_keep(1))              # the reference's forward() always drops (:164)
         return rep[:self.user_num], rep[self.user_num:]
 
     def calc_loss(self, batch):
         self._check_loss_type()
-        self._ensure_ws()
-        self.restore_user_e = self.restore_item_e = None
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
+        bu, bi, bj = self._planes(batch[:3])
+        self._ensure(0)
+        self._tables_changed()
         loss = ops.ngcf_bpr_train_steps(self.E0, self.gnn, self._ws, self.graph, bu, bi, bj, bu.numel(), 0, 1, self._hp,
                                         apply=False, tower_dtype=self._tower_dtype, dropout=self.message_dropout,
                                         keep=self._host_keep(1))
         return loss.to(torch.float32).reshape(())
 
-    def train_step(self, batch):
-        self._check_loss_type()
-        self._ensure_ws()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
-        return float(self._train_steps(bu, bi, bj, bu.numel(), 0, 1).item())
-
-    def _cached(self):
+    def _score_tables(self):
+        """The propagated tables (restore_user_e / restore_item_e), recomputed after a step or a load."""
         if self.restore_user_e is None or self.restore_item_e is None:
             self.restore_user_e, self.restore_item_e = self.forward()
         return self.restore_user_e, self.restore_item_e
-
-    def predict(self, u, i):
-        eu, ei = self._cached()
-        uu = torch.tensor([int(u)], dtype=torch.int32, device=self.device)
-        ii = torch.tensor([int(i)], dtype=torch.int32, device=self.device)
-        return float(ops.mf_predict(eu, ei, uu, ii).item())
-
-    def rank(self, test_loader):
-        eu, ei = self._cached()
-        data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
-        k = min(self.topk, cands.shape[1])
-        out = ops.mf_rank(eu, ei, torch.from_numpy(users).to(self.device),
-                          torch.from_numpy(np.ascontiguousarray(cands)).to(self.device), k)
-        return out.cpu().numpy()
-
-    def full_rank(self, u):
-        eu, ei = self._cached()
-        users = torch.tensor([int(u)], dtype=torch.int64, device=self.device)
-        return ops.mf_full_rank(eu, ei, users, min(self.topk, self.item_num))[0].cpu().numpy()

@@ -11,7 +11,7 @@ import numpy as np
 import torch
 
 from .. import ops
-from .AbstractRecommender import GeneralRecommender, _Table, _INIT
+from .AbstractRecommender import GeneralRecommender, _Table, _INIT, dropout_engine, dropout_rate, mask_segments, tower_dtype
 
 
 class NeuMF(GeneralRecommender):
@@ -23,7 +23,6 @@ class NeuMF(GeneralRecommender):
         self.epochs = config['epochs']
         self.reg_1 = config['reg_1']
         self.reg_2 = config['reg_2']
-        self.dropout = config['dropout']
         self.model = config['model_name']
         self.user_num, self.item_num = config['user_num'], config['item_num']
         self.factors, self.num_layers = config['factors'], config['num_layers']
@@ -37,9 +36,7 @@ class NeuMF(GeneralRecommender):
         self._mode = ops.NEUMF_MODE[self.model]                       # 0 NeuMF / NeuMF-pre, 1 GMF, 2 MLP
         self.GMF_model = config.get('GMF_model', None)
         self.MLP_model = config.get('MLP_model', None)
-        self.dropout = float(self.dropout or 0.0)
-        if not (0.0 <= self.dropout < 1.0):
-            raise ValueError(f'dropout must be in [0, 1), got {self.dropout}')
+        self.dropout = dropout_rate(config['dropout'])
         if self.factors % 4 != 0:
             raise NotImplementedError('NeuMF on the B200 path needs factors to be a multiple of 4 (128-bit rows)')
         F, Ln = self.factors, self.num_layers
@@ -77,16 +74,11 @@ class NeuMF(GeneralRecommender):
         self.embed_user_MLP = _Table(embs[2].weight.detach().to(self.device).contiguous())
         self.embed_item_MLP = _Table(embs[3].weight.detach().to(self.device).contiguous())
         self.tower = tower.to(self.device)
-        self._ws = None
-        self._opt_steps = 0
         self._rows = int(config.get('neumf_scratch_rows', 1 << 16))
         # optional B200 key: 'fp32' (CUDA cores, parity path, default) | 'bf16' (tcgen05 tensor cores, BASELINE config 3)
         #                   | 'fused' (bf16 tcgen05, the whole tower step of a 64-triple tile inside one CTA: activations stay in
         #                     shared / tensor memory; factors = 32, num_layers = 2, dropout 0 -- other shapes run as 'bf16')
-        td = str(config.get('tower_dtype', 'fp32')).lower()
-        if td not in ('fp32', 'bf16', 'fused'):
-            raise ValueError(f"tower_dtype must be 'fp32', 'bf16' or 'fused', got {td!r}")
-        self._tower_dtype = {'fp32': 0, 'bf16': 1, 'fused': 2}[td]
+        self._tower_dtype = tower_dtype(config, ('fp32', 'bf16', 'fused'))
         # optional B200 key: how nn.Dropout's masks (:61) are produced in train mode.
         #   'torch'  : torch itself draws them on the host, in the reference's order (per step: the pos forward's L masks, then
         #              the neg forward's), from the global CPU generator; they are bit-packed and uploaded -- the reference's
@@ -94,9 +86,7 @@ class NeuMF(GeneralRecommender):
         #   'philox' : counter-based masks generated inside the kernels (same distribution, another stream).
         #   'auto'   : 'torch' while a step's masks stay under 4 M elements (the reference's default batch of 256 is 74 K),
         #              'philox' above (throughput).
-        self.dropout_engine = str(config.get('dropout_engine', 'auto')).lower()
-        if self.dropout_engine not in ('auto', 'torch', 'philox'):
-            raise ValueError(f"dropout_engine must be 'auto', 'torch' or 'philox', got {self.dropout_engine!r}")
+        self.dropout_engine = dropout_engine(config)
 
     def _load_pretrained(self, embs, linears, predict):
         """'NeuMF-pre' (NeuMFRecommender.py:97-116): tables and tower copied from config['GMF_model'] / config['MLP_model'];
@@ -139,40 +129,25 @@ class NeuMF(GeneralRecommender):
         return (self.embed_user_GMF.weight, self.embed_item_GMF.weight, self.embed_user_MLP.weight,
                 self.embed_item_MLP.weight)
 
-    def parameters(self):
-        return list(self._tabs()) + [self.tower]
-
     def state_dict(self):
         return {'embed_user_GMF.weight': self.embed_user_GMF.weight, 'embed_item_GMF.weight': self.embed_item_GMF.weight,
                 'embed_user_MLP.weight': self.embed_user_MLP.weight, 'embed_item_MLP.weight': self.embed_item_MLP.weight,
                 'tower': self.tower}
 
-    def load_state_dict(self, sd):
-        for k, t in self.state_dict().items():
-            t.copy_(torch.as_tensor(sd[k]).reshape(t.shape))
-
-    def _hyper(self, opt=None):
-        return ops.hyper(self.lr, self.reg_1, self.reg_2, opt or self._optimizer_name())
-
-    def _workspace(self, rows, opt=None, fresh=False):
+    def _ensure(self, rows):
+        if self._hp is None:
+            self._begin_fit(self._optimizer_name())
         rows = max(int(rows), self._rows)
-        if fresh or self._ws is None or self._ws.max_rows < rows:
-            keep = None if fresh or self._ws is None else self._ws
-            if keep is not None and opt is None:
-                # growing the scratch would drop the optimiser state: size it up front instead
-                raise RuntimeError('NeuMF scratch too small; set config["neumf_scratch_rows"] >= 2 * batch_size')
-            self._ws = ops.NeumfWorkspace(self.user_num, self.item_num, self.factors, self.num_layers,
-                                          opt or self._optimizer_name(), rows, self.device)
-        return self._ws
+        if self._ws is None:
+            self._ws = ops.NeumfWorkspace(self.user_num, self.item_num, self.factors, self.num_layers, self._fit_opt, rows,
+                                          self.device)
+        elif self._ws.max_rows < rows:
+            # growing the scratch would drop the optimiser state: size it up front instead
+            raise RuntimeError('NeuMF scratch too small; set config["neumf_scratch_rows"] >= 2 * batch_size')
 
     def _begin_fit(self, opt):
-        # dropout masks are counter-based (Philox) on the device; the key is drawn from torch's global RNG so that
-        # torch.manual_seed makes runs reproducible (the masks themselves are NOT torch's: parity holds at dropout=0)
+        super()._begin_fit(opt)
         self._philox_seed = None                                     # drawn lazily: the host-mask engine must not move the RNG here
-        self._hp = self._hyper(opt)
-        self._opt_steps = 0
-        self._fit_opt = opt
-        self._ws = None                                              # fresh optimiser state per fit()
 
     def _host_masks(self, rows_per_step):
         """Parity dropout: the keep-masks nn.Dropout would draw for steps of rows_per_step[k] triples, drawn by torch on the CPU
@@ -200,32 +175,28 @@ class NeuMF(GeneralRecommender):
             self._philox_seed = int(torch.empty((), dtype=torch.int64).random_().item())
         return self._philox_seed
 
+    def _mask_bits(self, batch):
+        """Dropout mask elements of one step: both forward calls over every tower layer."""
+        return 2 * batch * (4 * self.mlp_dim - 2 * self.factors)
+
     def _use_host_masks(self, batch):
         if not self.training or self.dropout <= 0.0 or self._mode == 1:
             return False                                                  # 'GMF' never runs the tower: no Dropout is called
         if self.dropout_engine == 'auto':
-            return 2 * batch * (4 * self.mlp_dim - 2 * self.factors) <= (1 << 22)
+            return self._mask_bits(batch) <= (1 << 22)
         return self.dropout_engine == 'torch'
 
     def _train_steps(self, bu, bi, bj, batch, first, n_steps):
-        if self._ws is None:
-            self._workspace(2 * batch, self._fit_opt, fresh=True)
+        self._ensure(2 * batch)
         p = self.dropout if self.training else 0.0
         kw = dict(tower_dtype=self._tower_dtype, dropout=p, mode=self._mode)
-        n = bu.numel()
         if self._use_host_masks(batch):
-            full = n_steps if (first + n_steps) * batch <= n else n_steps - 1   # a ragged last batch gets its own masks + call
             out = []
-            if full > 0:
-                masks = self._host_masks([batch] * full)
-                out.append(ops.neumf_bpr_train_steps(self._tabs(), self.tower, self._ws, bu, bi, bj, batch, first, full, self._hp,
-                                                     adam_step0=self._opt_steps, drop_masks=masks, **kw))
-            if full < n_steps:
-                base = (first + full) * batch
-                last = n - base
-                masks = self._host_masks([last])
-                out.append(ops.neumf_bpr_train_steps(self._tabs(), self.tower, self._ws, bu[base:], bi[base:], bj[base:], last, 0,
-                                                     1, self._hp, adam_step0=self._opt_steps + full, drop_masks=masks, **kw))
+            for s, k, rows in mask_segments(bu.numel(), batch, first, n_steps, self._mask_bits(batch) // 8):
+                lo, s0 = (s * batch, 0) if rows < batch else (0, s)   # a ragged last step runs as a batch of its own
+                out.append(ops.neumf_bpr_train_steps(self._tabs(), self.tower, self._ws, bu[lo:], bi[lo:], bj[lo:], rows, s0, k,
+                                                     self._hp, adam_step0=self._opt_steps + (s - first),
+                                                     drop_masks=self._host_masks([rows] * k), **kw))
             losses = torch.cat(out)
         else:
             losses = ops.neumf_bpr_train_steps(self._tabs(), self.tower, self._ws, bu, bi, bj, batch, first, n_steps, self._hp,
@@ -233,25 +204,10 @@ class NeuMF(GeneralRecommender):
         self._opt_steps += n_steps
         return losses
 
-    def _ensure(self, rows):
-        if self._ws is None:
-            self._begin_fit(self._optimizer_name())
-            self._workspace(rows, self._fit_opt, fresh=True)
-        elif self._ws.max_rows < rows:
-            self._workspace(rows)
-
     # ------------------------------------------------------------------ reference surface
-    def forward(self, user, item):
-        u = torch.as_tensor(user).to(self.device, torch.int64).reshape(-1).contiguous()
-        i = torch.as_tensor(item).to(self.device, torch.int64).reshape(-1, 1).contiguous()
-        self._ensure(1)
-        return ops.neumf_scores(self._tabs(), self.tower, self._ws, u, i, 1, self._tower_dtype, self._mode).reshape(-1)
-
-    __call__ = forward
-
     def calc_loss(self, batch):
         self._check_loss_type()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
+        bu, bi, bj = self._planes(batch[:3])
         self._ensure(2 * bu.numel())
         masks = self._host_masks([bu.numel()]) if self._use_host_masks(bu.numel()) else None
         loss = ops.neumf_bpr_train_steps(self._tabs(), self.tower, self._ws, bu, bi, bj, bu.numel(), 0, 1, self._hp,
@@ -261,42 +217,15 @@ class NeuMF(GeneralRecommender):
                                          mode=self._mode)
         return loss.to(torch.float32).reshape(())
 
-    def train_step(self, batch):
-        self._check_loss_type()
-        bu, bi, bj = (torch.as_tensor(b).to(self.device, torch.int32).contiguous() for b in batch[:3])
-        self._ensure(2 * bu.numel())
-        was = self.training
-        self.train()                                                 # a training step runs in train mode (dropout on)
-        try:
-            return float(self._train_steps(bu, bi, bj, bu.numel(), 0, 1).item())
-        finally:
-            self.train(was)
-
-    def predict(self, u, i):
-        return float(self.forward([int(u)], [int(i)]).item())
-
-    def rank(self, test_loader):
-        data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
+    def _scores(self, users, items, per_user):
         self._ensure(1)
-        d_users = torch.from_numpy(users).to(self.device)
-        d_cands = torch.from_numpy(np.ascontiguousarray(cands)).to(self.device)
-        scores = ops.neumf_scores(self._tabs(), self.tower, self._ws, d_users, d_cands, cands.shape[1], self._tower_dtype, self._mode)
-        k = min(self.topk, cands.shape[1])
-        return ops.topk_from_scores(scores, d_cands, k).cpu().numpy()
+        return ops.neumf_scores(self._tabs(), self.tower, self._ws, users, items, per_user, self._tower_dtype, self._mode)
 
-    def full_rank(self, u):
-        self._ensure(1)
-        users = torch.tensor([int(u)], dtype=torch.int64, device=self.device)
-        scores = ops.neumf_scores(self._tabs(), self.tower, self._ws, users, None, self.item_num, self._tower_dtype, self._mode)
-        return ops.topk_from_scores(scores, None, min(self.topk, self.item_num))[0].cpu().numpy()
+    def _score_pairs(self, u, i):
+        return self._scores(u.to(torch.int64), i.to(torch.int64).reshape(-1, 1), 1).reshape(-1)
+
+    def _rank_rows(self, users, cands, k):
+        return ops.topk_from_scores(self._scores(users, cands, cands.shape[1]), cands, k)
+
+    def _full_rank_rows(self, users, k):
+        return ops.topk_from_scores(self._scores(users, None, self.item_num), None, k)

@@ -22,10 +22,10 @@ import math
 
 import numpy as np
 import torch
+from tqdm import tqdm
 
 from .. import ops
-from .AbstractRecommender import GeneralRecommender, _INIT, epoch_seed  # noqa: F401
-from torch.utils.data import BatchSampler, RandomSampler, SequentialSampler
+from .AbstractRecommender import GeneralRecommender, _INIT, dropout_engine, dropout_rate, loader_plan, mask_segments, tower_dtype
 
 
 def rating_csr(history_item_id, history_item_value, item_num, device):
@@ -59,25 +59,6 @@ def _pad4(t):
     return torch.cat([t, t.new_zeros((-t.numel()) % 4)])
 
 
-def _ae_plan(train_loader):
-    """(users ndarray, batch_size, shuffle, drop_last, generator) of a plain DataLoader(AEDataset) -- a 1-D array of ids read
-    in DataLoader order -- or None (fit() then iterates the loader batch by batch)."""
-    data = getattr(getattr(train_loader, 'dataset', None), 'data', None)
-    bs = getattr(train_loader, 'batch_size', None)
-    if not isinstance(data, np.ndarray) or data.ndim != 1 or bs is None:
-        return None
-    if not isinstance(getattr(train_loader, 'batch_sampler', None), BatchSampler):
-        return None
-    sampler = getattr(train_loader, 'sampler', None)
-    if isinstance(sampler, RandomSampler) and not sampler.replacement and sampler._num_samples is None and sampler.generator is None:
-        shuffle = True
-    elif isinstance(sampler, SequentialSampler):
-        shuffle = False
-    else:
-        return None
-    return data, int(bs), shuffle, bool(train_loader.drop_last), train_loader.generator
-
-
 class VAECF(GeneralRecommender):
     def __init__(self, config):
         """Same keys as the reference: user_num, item_num, history_item_id, history_item_value, mlp_hidden_size (None ->
@@ -90,9 +71,7 @@ class VAECF(GeneralRecommender):
             raise NotImplementedError('VAECF runs as independent replicas only (DESIGN.md, multi-GPU section)')
         self.epochs = config['epochs']
         self.lr = config['lr']
-        self.dropout = float(config['dropout'] or 0.0)
-        if not 0.0 <= self.dropout < 1.0:
-            raise ValueError(f"dropout probability has to be in [0, 1), but got {self.dropout}")
+        self.dropout = dropout_rate(config['dropout'])
         self.layers = list(config['mlp_hidden_size']) if config['mlp_hidden_size'] is not None else [600]
         self.lat_dim = int(config['latent_dim'])
         self.anneal_cap = config['anneal_cap']
@@ -135,18 +114,10 @@ class VAECF(GeneralRecommender):
         else:
             self.R = rating_csr(config['history_item_id'], config['history_item_value'], self.item_num, self.device)
 
-        td = str(config.get('tower_dtype', 'fp32')).lower()
-        if td not in ('fp32', 'bf16'):
-            raise ValueError(f"tower_dtype must be 'fp32' or 'bf16', got {td!r}")
-        self._tower_dtype = 1 if td == 'bf16' else 0
-        self.dropout_engine = str(config.get('dropout_engine', 'auto')).lower()
-        if self.dropout_engine not in ('auto', 'torch', 'philox'):
-            raise ValueError(f"dropout_engine must be 'auto', 'torch' or 'philox', got {self.dropout_engine!r}")
+        self._tower_dtype = tower_dtype(config)
+        self.dropout_engine = dropout_engine(config)
         self._rows = int(config.get('vae_scratch_rows', 256))
         self._philox_seed = None
-        self._ws = None
-        self._hp = None
-        self._opt_steps = 0
 
     # ------------------------------------------------------------------ plumbing
     def _param_views(self):
@@ -161,38 +132,23 @@ class VAECF(GeneralRecommender):
                 o += -(-b // 4) * 4
         return views
 
-    def parameters(self):
-        return list(self._views.values())
-
     def state_dict(self):
         return dict(self._views)
 
-    def load_state_dict(self, sd):
-        for k, t in self._views.items():
-            t.copy_(torch.as_tensor(sd[k]).to(t.device, t.dtype).reshape(t.shape))
+    def _check_loss_type(self):
+        """The ELBO is VAECF's only loss: its config has no loss_type."""
 
-    def to(self, device):
-        return self
-
-    def _workspace(self, rows, opt=None, fresh=False):
-        rows = max(int(rows), self._rows, 1)
-        if fresh or self._ws is None or self._ws.max_rows < rows:
-            if not fresh and self._ws is not None and self._opt_steps > 0:
-                raise RuntimeError('VAECF scratch too small; set config["vae_scratch_rows"] >= batch_size')
-            self._ws = ops.VaeWorkspace(self.item_num, self.layers, self.lat_dim, opt or self._optimizer_name(), rows, self.device)
-        return self._ws
-
-    def _begin_fit(self, opt, rows=1):
-        """fit() builds a fresh optimizer (AbstractRecommender.py:105): fresh optimiser state and step count."""
-        self._hp = ops.hyper(self.lr, 0.0, 0.0, opt)
-        self._opt_steps = 0
-        self._workspace(rows, opt, fresh=True)
+    def _hyper(self, opt):
+        return ops.hyper(self.lr, 0.0, 0.0, opt)
 
     def _ensure(self, rows):
         if self._hp is None:
-            self._begin_fit(self._optimizer_name(), rows)
-        else:
-            self._workspace(rows)
+            self._begin_fit(self._optimizer_name())
+        rows = max(int(rows), self._rows, 1)
+        if self._ws is None or self._ws.max_rows < rows:
+            if self._ws is not None and self._opt_steps > 0:
+                raise RuntimeError('VAECF scratch too small; set config["vae_scratch_rows"] >= batch_size')
+            self._ws = ops.VaeWorkspace(self.item_num, self.layers, self.lat_dim, self._fit_opt, rows, self.device)
 
     def _host_rng(self, batch):
         """True when the step's dropout mask and eps come from torch's global CPU generator (the reference's stream)."""
@@ -225,7 +181,6 @@ class VAECF(GeneralRecommender):
 
     def _steps(self, users, batch, n_steps, apply=True):
         """n_steps steps over the int32 device ids `users` (a ragged last batch holds the rest) -> float64 losses [n_steps]."""
-        n = users.numel()
         kw = dict(apply=apply, training=self.training, tower_dtype=self._tower_dtype, dropout=self.dropout,
                   anneal_cap=float(self.anneal_cap), total_anneal_steps=int(self.total_anneal_steps))
         args = (self.net, self._ws, self.R)
@@ -237,31 +192,18 @@ class VAECF(GeneralRecommender):
             if apply:
                 self._opt_steps += n_steps
             return out
-        mask_bytes = max(1, batch * self.item_num // 8)
-        chunk = max(1, (64 << 20) // mask_bytes)                       # at most 64 MB of masks per call
-        out, s = [], 0
-        while s < n_steps:
-            k = min(chunk, n_steps - s)
-            full = k if (s + k) * batch <= n else k - 1                  # a ragged last batch gets its own draws and call
-            if full > 0:
-                keep, eps = self._host_draws([batch] * full)
-                out.append(ops.vae_train_steps(*args, users[s * batch:(s + full) * batch], batch, 0, full, self._hp,
-                                               adam_step0=self._opt_steps, keep=keep, eps=eps, update0=self.update, **kw))
-                self.update += full
-                if apply:
-                    self._opt_steps += full
-            if full < k:
-                last = users[(s + full) * batch:]
-                keep, eps = self._host_draws([last.numel()])
-                out.append(ops.vae_train_steps(*args, last, last.numel(), 0, 1, self._hp, adam_step0=self._opt_steps, keep=keep,
-                                               eps=eps, update0=self.update, **kw))
-                self.update += 1
-                if apply:
-                    self._opt_steps += 1
-            s += k
+        out = []
+        for s, k, rows in mask_segments(users.numel(), batch, 0, n_steps, batch * self.item_num // 8):
+            keep, eps = self._host_draws([rows] * k)
+            out.append(ops.vae_train_steps(*args, users[s * batch:s * batch + k * rows], rows, 0, k, self._hp,
+                                           adam_step0=self._opt_steps, keep=keep, eps=eps, update0=self.update, **kw))
+            self.update += k
+            if apply:
+                self._opt_steps += k
         return torch.cat(out)
 
     def _users(self, batch):
+        """Host-checked user ids -> int32 device ids; ids in [-user_num, 0) wrap as history_item_id[user] does."""
         u = torch.as_tensor(batch).reshape(-1).to(torch.int64)
         if u.numel() and (int(u.min()) < -self.user_num or int(u.max()) >= self.user_num):
             raise IndexError(f'index out of range: user id outside [0, {self.user_num})')
@@ -269,30 +211,12 @@ class VAECF(GeneralRecommender):
         return u.to(self.device, torch.int32).contiguous()
 
     # ------------------------------------------------------------------ training
-    def fit(self, train_loader):
-        """The epoch loop (AbstractRecommender.py:103-137) over a DataLoader(AEDataset): each epoch's order is the loader's own
-        permutation, so the batches are the reference's."""
-        opt = self._optimizer_name()
-        plan = _ae_plan(train_loader)
-        self._begin_fit(opt, plan[1] if plan is not None else getattr(train_loader, 'batch_size', None) or 1)
-        last_loss = 0.
-        for epoch in range(1, self.epochs + 1):
-            self.train()
-            if plan is not None:
-                current_loss = self._fit_epoch_users(plan)
-            else:
-                current_loss = 0.
-                for batch in train_loader:
-                    current_loss += self.train_step(batch)
-            self.eval()
-            delta_loss = float(current_loss - last_loss)
-            if (abs(delta_loss) < 1e-5) and self.early_stop:
-                self.logger.info('Satisfy early stop mechanism')
-                break
-            else:
-                last_loss = current_loss
+    def _loader_plan(self, train_loader):
+        """A plain DataLoader(AEDataset): a 1-D array of user ids read in DataLoader order."""
+        return loader_plan(train_loader, lambda data: data.ndim == 1)
 
-    def _fit_epoch_users(self, plan):
+    def _fit_epoch_bulk(self, plan, epoch):
+        """One epoch over the loader's own permutation of the user ids, so the batches are the reference's."""
         data, bs, shuffle, drop_last, gen = plan
         T = len(data)
         key = (id(data), data.ctypes.data, T)
@@ -303,10 +227,16 @@ class VAECF(GeneralRecommender):
         users = self._users_dev if d_perm is None else self._users_dev.index_select(0, d_perm).contiguous()
         n_use = (T // bs) * bs if drop_last else T
         nsteps = (n_use + bs - 1) // bs
-        if nsteps == 0:
-            return 0.
-        self._workspace(bs)
-        return float(self._steps(users[:n_use], bs, nsteps).sum().item())   # raises ValueError on NaN
+        pbar = tqdm(total=nsteps, disable=not self.show_progress)
+        pbar.set_description(f'[Epoch {epoch:03d}]')
+        current_loss = 0.
+        if nsteps:
+            self._ensure(bs)
+            current_loss = float(self._steps(users[:n_use], bs, nsteps).sum().item())   # raises ValueError on NaN
+        pbar.update(nsteps)
+        pbar.set_postfix(loss=current_loss)
+        pbar.close()
+        return current_loss
 
     def calc_loss(self, batch):
         """VAECFRecommender.py:92-110 in the current mode: 0-d fp32 loss; counts one update of the KL anneal; no parameter
@@ -336,42 +266,22 @@ class VAECF(GeneralRecommender):
             raise TypeError('VAECF.forward takes user ids (an integer scalar or 1-d array), not a dense rating matrix; '
                             f'got a {t.dim()}-d {t.dtype} tensor')
         u = self._users(t)
-        self._ensure(1)
-        scores = ops.vae_forward(self.net, self._ws, self.R, u, 'scores', self._tower_dtype)
+        scores = self._scores(u)
         h = ops.vae_forward(self.net, self._ws, self.R, u, 'latent', self._tower_dtype)
         return scores, h[:, :int(self.lat_dim / 2)], h[:, math.ceil(self.lat_dim / 2):]
 
-    __call__ = forward
-
-    def predict(self, u, i):
+    def _scores(self, users):
         self._ensure(1)
-        scores = ops.vae_forward(self.net, self._ws, self.R, self._users([int(u)]), 'scores', self._tower_dtype)
-        return float(scores[0, int(i)].item())
+        return ops.vae_forward(self.net, self._ws, self.R, users, 'scores', self._tower_dtype)
 
-    def rank(self, test_loader):
-        """float32 ndarray [n_test_users, topk] of candidate ids, best first: the decoder output at the candidates only."""
-        data = getattr(getattr(test_loader, 'dataset', None), 'data', None)
-        if isinstance(data, (list, tuple)) and len(data) and len(data[0]) == 2:
-            users = np.fromiter((int(r[0]) for r in data), np.int64, len(data))
-            cands = np.stack([np.asarray(r[1], dtype=np.int64) for r in data])
-        else:
-            us, cs = [], []
-            for b_us, b_c in test_loader:
-                us.append(torch.as_tensor(b_us).reshape(-1).to(torch.int64))
-                cs.append(torch.as_tensor(b_c).to(torch.int64).reshape(us[-1].numel(), -1))
-            if not us:
-                return np.zeros((0,), np.float32)
-            users, cands = torch.cat(us).numpy(), torch.cat(cs).numpy()
-        if len(users) == 0:
-            return np.zeros((0,), np.float32)
-        self._ensure(1)
-        d_cands = torch.from_numpy(np.ascontiguousarray(cands)).to(self.device)
-        ops.check_index_range(d_cands.reshape(-1, 1), (self.item_num,), ('candidate item',))
-        hidden = ops.vae_forward(self.net, self._ws, self.R, self._users(users), 'hidden', self._tower_dtype)
-        scores = ops.vae_candidate_scores(self.net, self._ws, hidden, d_cands)
-        return ops.topk_from_scores(scores, d_cands, min(self.topk, cands.shape[1])).cpu().numpy()
+    def _score_pairs(self, u, i):
+        return self._scores(u).gather(1, i.to(torch.int64).reshape(-1, 1)).reshape(-1)
 
-    def full_rank(self, u):
+    def _rank_rows(self, users, cands, k):
+        """The decoder output at the candidates only."""
         self._ensure(1)
-        scores = ops.vae_forward(self.net, self._ws, self.R, self._users([int(u)]), 'scores', self._tower_dtype)
-        return ops.topk_from_scores(scores, None, min(self.topk, self.item_num))[0].cpu().numpy()
+        hidden = ops.vae_forward(self.net, self._ws, self.R, users, 'hidden', self._tower_dtype)
+        return ops.topk_from_scores(ops.vae_candidate_scores(self.net, self._ws, hidden, cands), cands, k)
+
+    def _full_rank_rows(self, users, k):
+        return ops.topk_from_scores(self._scores(users), None, k)

@@ -171,7 +171,8 @@ def bench_vae(dev, steps, batch):
                 torch.manual_seed(1)
                 m = _vae_model(U, I, row_ptr, col, dev, tower_dtype=td, dropout_engine=eng)
                 m.train()
-                m._begin_fit("adam", B)
+                m._begin_fit("adam")
+                m._ensure(B)
                 m._steps(users[:B], B, 1)                                              # warm-up
                 torch.cuda.synchronize()
                 t0 = time.time()
@@ -190,7 +191,8 @@ def bench_vae(dev, steps, batch):
         torch.manual_seed(1)
         m = _vae_model(U, I, row_ptr, col, dev, tower_dtype=td, dropout_engine="philox")
         m.train()
-        m._begin_fit("adam", 256)
+        m._begin_fit("adam")
+        m._ensure(256)
         us = torch.randperm(U, generator=g)[:256 * 8].to(torch.int32).to(dev)
         m._steps(us, 256, 2)
         torch.cuda.synchronize()
